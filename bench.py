@@ -289,6 +289,7 @@ class Shape:
         self.gather_stream = torch.cuda.Stream(device=dev) if ctx.world > 1 else None
         self.pending = None
         self.defer = self.pipelined and ctx.world > 1 and not args.inline_gather
+        self.last_out = None   # this rank's [B,T,512] output of the latest device_step
 
     def make_plan(self, **kw):
         from sbl_for_multilingual_lip_reading_b200.runner import PipelinedVisualEncoderPlan, VisualEncoderPlan
@@ -336,6 +337,7 @@ class Shape:
                 with torch.cuda.stream(self.gather_stream):
                     self.gather_outputs(self.pending)
             out = plan.forward_device(s)
+            self.last_out = out
             if defer and self.pending is not None and not gather_first:
                 # issued BEHIND the replay: the step's first kernels (encoder clusters, gated stem) get their SMs before
                 # the gather's small CTAs look for room beside them
@@ -400,6 +402,24 @@ class Ctx:
     pass
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_output(out_dir, name, t, seed=0):
+    """--dump-outputs: write `t` as <out_dir>/<name>.npy in float32.  Above the 64 MiB budget it is cut to a fixed, seeded
+    sample of its rows along dim 0 (sorted indices, the same for the same shape)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    t = t.detach().float()
+    row_bytes = t[0].numel() * 4
+    if t.numel() * 4 > DUMP_BUDGET_BYTES:
+        keep = max(1, DUMP_BUDGET_BYTES // row_bytes)
+        idx = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+        t = t[idx.to(t.device)]
+    np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def run_b200_arm(args):
     import torch
     import torch.distributed as dist
@@ -454,6 +474,14 @@ def run_b200_arm(args):
     # ---- device-timed run (the metric) -----------------------------------------------------
     dev_ms = main.time_device(args.steps, args.warmup, sampler=sampler)
     value = world * B / (dev_ms * 1e-3)
+    if args.dump_outputs:
+        out = main.last_out
+        if world > 1:   # what the caller receives: every rank's block, gathered in rank order
+            full = torch.empty((world * B, T, 512), dtype=torch.float32, device=dev)
+            dist.all_gather_into_tensor(full, out.contiguous())
+            out = full
+        if rank == 0:
+            dump_output(args.dump_outputs, "encoder_output", out)
 
     # ---- end-to-end run (host buffers, H2D + D2H inside the timed region).  Measured right after the device-timed run:
     # both are K-step bursts on a GPU that has not yet been driven into its power cap by the seconds-long `sustained`
@@ -866,7 +894,7 @@ def run_config4_sweep(args):
                 torch.cuda.synchronize(dev)
                 return sharding.max_over_ranks((time.perf_counter() - t0) / reps, dev)
 
-        reps = max(2, min(args.steps, 10))
+        reps = args.steps
         t_full, o0 = timed(full, reps)
         t_ours, o1 = timed(ours, reps)
         t_ref, o2 = timed(ref, reps)
@@ -961,7 +989,7 @@ def run_config3(args):
         ms = sharding.max_over_ranks(sum(a.elapsed_time(b) for a, b in evs), dev) / steps
         return ms, float(loss.detach()), launches
 
-    steps, warmup = max(3, min(args.steps, 10)), max(2, min(args.warmup, 3))
+    steps, warmup = args.steps, args.warmup
     ms, loss, launches = timed(net, opt, steps, warmup)
     ref_ms = None
     if not args.no_cpu_baseline:
@@ -1045,7 +1073,16 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--ref-clips", type=int, default=0,
                     help="clips per reference-arm step (0 = the whole --batch, bounded only on very slow hosts)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the encoder output of the last timed step, gathered over the "
+                         "ranks ([gpus*batch,T,512]), as DIR/encoder_output.npy (float32; a seeded sample of clips above "
+                         "64 MiB); "
+                         "inputs and the dropout seed are fixed, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "visual_encoder"):
+        ap.error("--dump-outputs is supported for the visual_encoder workload of --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "b200" and args.gpus != world:

@@ -142,3 +142,88 @@ def test_input_pipeline_oracle_matches_reference_transforms():
     lut = synth.normalize_lut().float().numpy()
     ref = P.load_and_normalize(np.arange(256, dtype=np.uint8)).astype(np.float32)
     assert np.array_equal(lut, torch.from_numpy(ref).to(torch.bfloat16).float().numpy())
+
+
+# ------------------------------------------------------------- the module-form restatement (oracle/reference_modules.py)
+def test_reference_modules_state_dicts_match_the_reference_contract():
+    """Same keys, shapes and dtypes as the reference's Lipreading and 6-layer Encoder (tests/golden/state_dict_contract.json),
+    and the stage-1 model is those two plus its word and language heads."""
+    import json
+    import os
+    from oracle import reference_modules as RM
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "state_dict_contract.json")) as f:
+        contract = json.load(f)
+
+    def table(m):
+        return {k: [list(v.shape), str(v.dtype)] for k, v in m.state_dict().items()}
+    assert table(RM.Lipreading()) == contract["Lipreading"]
+    assert table(RM.Encoder(512, 6, 8, 64, 64, 512, 2048, dropout=0.1, pe_maxlen=5000)) == contract["Encoder6"]
+    s1 = table(RM.build_stage1())
+    want = {"visual_frontend." + k: v for k, v in contract["Lipreading"].items()}
+    want.update({"encoder_v." + k: v for k, v in contract["Encoder6"].items() if not k.startswith("layer_stack.")
+                 or int(k.split(".")[1]) < 3})
+    want.update({"fc_1500.weight": [[1500, 512], "torch.float32"], "fc_1500.bias": [[1500], "torch.float32"],
+                 "fc_2.weight": [[2, 512], "torch.float32"], "fc_2.bias": [[2], "torch.float32"]})
+    assert s1 == want
+
+
+def test_reference_modules_reproduce_the_reference_outputs(golden, golden_inputs):
+    """In eval mode, with the always-on frontend dropout left out (`_frontend_forward`, as the goldens were produced) and
+    encoder dropout inactive, the modules reproduce every golden vector of the reference modules."""
+    from oracle import reference_modules as RM
+    fe = RM.Lipreading()
+    fe.load_state_dict(synth.frontend_state_dict(1))
+    fe.eval()
+    enc6 = RM.Encoder(512, 6, 8, 64, 64, 512, 2048, dropout=0.1, pe_maxlen=5000)
+    enc6.load_state_dict(synth.encoder_state_dict(2, 6))
+    enc6.eval()
+    enc3 = RM.Encoder(512, 3, 8, 64, 64, 512, 2048, dropout=0.1, pe_maxlen=5000)
+    enc3.load_state_dict(synth.encoder_state_dict(3, 3))
+    enc3.eval()
+    with torch.no_grad():
+        x = synth.synthetic_clips(1, 2, seed=11)
+        close(fe.frontend3D(x), golden["frontend3d_T2"])
+        y = fe.frontend3D(x).transpose(1, 2).contiguous().view(-1, 64, 22, 22)
+        close(fe.resnet18.layer1[0](y.clone()), golden["layer1_0_T2"])
+        close(fe.resnet18.layer2[0](fe.resnet18.layer1(y.clone())), golden["layer2_0_T2"])
+        close(fe._frontend_forward(synth.synthetic_clips(1, 29, seed=7)), golden["frontend_c1"])
+        feat = fe._frontend_forward(synth.synthetic_clips(2, 6, seed=8, pad_frames=1))
+        close(feat, golden["frontend_N2_T6_pad1"])
+        close(enc6(torch.from_numpy(golden_inputs["xin"]), [29])[0], golden["encoder6_N1_T29"])
+        close(enc6(torch.from_numpy(golden_inputs["xin40"]), [40])[0], golden["encoder6_N1_T40"])
+        close(enc3(torch.from_numpy(golden_inputs["xin3"]), [31, 31])[0], golden["encoder3_N2_T31"])
+        out, attns = enc6(torch.from_numpy(golden_inputs["xin_r"]), [12, 7, 1], return_attns=True)
+        close(out, golden["encoder6_ragged_out"])
+        close(attns[0], golden["encoder6_ragged_attn0"])
+        close(attns[5], golden["encoder6_ragged_attn5"])
+        close(enc6(feat.view(2, 6, 512), [6, 6])[0], golden["visual_encoder_N2_T6"])
+
+
+def test_reference_modules_dropout_sites():
+    """Training-mode dropout: the frontend's always-on F.dropout(p=0.5) on the pooled features, and the encoder's four
+    draws in the reference's order and shapes — input [N,T,512], then per layer attention probabilities [H*N,T,T], the
+    fc output and the feed-forward output (both [N,T,512])."""
+    from oracle import reference_modules as RM
+    n, t, L = 2, 5, 2
+    enc = RM.Encoder(512, L, 8, 64, 64, 512, 2048, dropout=0.1, pe_maxlen=5000).train()
+    seen = []
+    for name, m in enc.named_modules():
+        if isinstance(m, torch.nn.Dropout):
+            m.register_forward_hook(lambda mod, i, o, name=name: seen.append((name, tuple(i[0].shape))))
+    enc(torch.randn(n, t, 512), [t] * n)
+    want = [("dropout", (n, t, 512))]
+    for i in range(L):
+        want += [(f"layer_stack.{i}.slf_attn.attention.dropout", (8 * n, t, t)),
+                 (f"layer_stack.{i}.slf_attn.dropout", (n, t, 512)), (f"layer_stack.{i}.pos_ffn.dropout", (n, t, 512))]
+    assert seen == want
+    fe = RM.Lipreading()
+    fe.load_state_dict(synth.frontend_state_dict(1))
+    fe.eval()
+    x = synth.synthetic_clips(1, 3, seed=3)
+    with torch.no_grad():
+        base = fe._frontend_forward(x).view(1, 3, 512)
+        torch.manual_seed(0)
+        dropped = fe(x)
+    kept = dropped != 0
+    assert 0.3 < float(kept.float().mean()) < 0.7
+    close(dropped[kept], 2.0 * base[kept])

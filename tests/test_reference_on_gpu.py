@@ -8,6 +8,11 @@ run ON TOP of the drop-in visual frontend + encoder (dropin.patch_reference), ne
   * teacher-forced `Transformer.forward` logits (transformer/transformer.py:22-43, decoder.py:79-191)
   * stage-by-stage error budget (stem, every ResNet layer, features, every encoder layer)
 
+The tests that need only the reference's frontend and encoder (the error budget, the always-on dropout mask, the
+decoder's CUDA-graph steps) run them as oracle/reference_modules.py restates them, with the forward pinned to the
+reference's own outputs by tests/test_oracle_golden.py, so they need no staged files; the others skip where
+oracle/_ref is not staged.
+
 Results are also written to gpurun_out/r02_*.json (copied to profiles/ by the builder).
 """
 import json
@@ -74,6 +79,26 @@ def models(dev):
     ours = ours.to(dev).eval()
     ours.visual_frontend.always_on_dropout = False
     return R, ref, ours
+
+
+@pytest.fixture(scope="module")
+def fe_enc(dev):
+    """The reference frontend + 6-layer encoder in fp32 (oracle/reference_modules.py) next to the drop-in frontend +
+    encoder, on cuda, with the synthetic weights of `models`; eval mode, the drop-in's always-on dropout off."""
+    import types
+    from oracle import ref_runtime, reference_modules as RM
+    from sbl_for_multilingual_lip_reading_b200 import synth
+    from sbl_for_multilingual_lip_reading_b200.encoder import Encoder as B200Encoder
+    from sbl_for_multilingual_lip_reading_b200.video_frontend import Lipreading as B200Lipreading
+    ref_runtime.fp32_exact()
+    fe_sd, enc_sd = synth.frontend_state_dict(1), synth.encoder_state_dict(2, 6)
+    m = types.SimpleNamespace(fe_ref=RM.Lipreading(), enc_ref=RM.Encoder(512, 6, 8, 64, 64, 512, 2048, dropout=0.1),
+                              fe=B200Lipreading(), enc=B200Encoder(512, 6, 8, 64, 64, 512, 2048, dropout=0.1))
+    for mod, sd in ((m.fe_ref, fe_sd), (m.enc_ref, enc_sd), (m.fe, fe_sd), (m.enc, enc_sd)):
+        mod.load_state_dict(sd)
+        mod.to(dev).eval()
+    m.fe.always_on_dropout = False
+    return m
 
 
 class _Tap:
@@ -186,26 +211,28 @@ def test_greedy_tokens_reference_decoder_on_dropins_1000_clips(models, dev):
         assert flips <= max(2 * ctl_flips, 10), f"{d}: {flips} flips vs {ctl_flips} for the bf16 control"
 
 
-def test_recognize_with_always_on_dropout_draws_the_reference_mask(models, dev):
-    """The production call, untouched on both sides: `recognize` with the always-on dropout(0.5) of
-    video_frontend.py:122 active.  Under the same CUDA seed the drop-in draws the very same Philox mask (same torch
-    call on the same shape), so encoder outputs stay within tolerance of the all-reference model."""
+def test_recognize_with_always_on_dropout_draws_the_reference_mask(fe_enc, dev):
+    """What `recognize` runs before the decoder (transformer.py:55-67), untouched on both sides: frontend with the
+    always-on dropout(0.5) of video_frontend.py:122 active, then the encoder.  Under the same CUDA seed the drop-in draws
+    the very same Philox mask (same torch call on the same shape), so encoder outputs stay within tolerance of the
+    reference's fp32 modules."""
     from sbl_for_multilingual_lip_reading_b200 import synth
-    R, ref, ours = models
-    x = synth.structured_clips(8, T, seed=77)[:, 0].to(dev)
-    ours.visual_frontend.always_on_dropout = True
+    m = fe_enc
+    n = 8
+    x = synth.structured_clips(n, T, seed=77).to(dev)                     # [N,1,T,88,88], as recognize views it
+    m.fe.always_on_dropout = True
     try:
         with torch.no_grad():
             torch.manual_seed(11)
-            a = _recognize(ref, x)
+            a, = m.enc_ref(m.fe_ref(x), [T] * n)
             torch.manual_seed(11)
-            b = _recognize(ours, x)
+            b, = m.enc(m.fe(x), [T] * n)
             torch.manual_seed(12)
-            c = _recognize(ours, x)
+            c, = m.enc(m.fe(x), [T] * n)
     finally:
-        ours.visual_frontend.always_on_dropout = False
-    assert rel_fro(b[2], a[2]) < 4e-3
-    assert rel_fro(c[2], a[2]) > 0.05          # a different seed really is a different mask
+        m.fe.always_on_dropout = False
+    assert rel_fro(b, a) < 4e-3
+    assert rel_fro(c, a) > 0.05          # a different seed really is a different mask
 
 
 def test_teacher_forced_forward_reference_decoder_on_dropins(models, dev):
@@ -238,25 +265,23 @@ def test_teacher_forced_forward_reference_decoder_on_dropins(models, dev):
     assert e_l2r < 1e-2 and e_r2l < 1e-2, (e_l2r, e_r2l)
 
 
-def test_stage_error_budget(models, dev):
+def test_stage_error_budget(fe_enc, dev):
     """Where the error comes from: relative Frobenius error of every stage boundary of the CUDA path against the
     all-reference fp32 model on the same 8 structured clips (each stage fed by the path's own previous stage, i.e.
     accumulated error).  bf16 trunk, enc16 encoder: features <= 4e-3, encoder output <= 4e-3 (north_star: 1e-2)."""
-    from oracle import ref_runtime
     from sbl_for_multilingual_lip_reading_b200 import ops, synth
     from sbl_for_multilingual_lip_reading_b200.encoder import Encoder
-    R, ref, ours = models
     n = 8
     x = synth.structured_clips(n, T, seed=4242).to(dev)                   # [N,1,T,88,88]
-    fe_ref, fe = ref.visual_frontend, ours.visual_frontend
+    fe_ref, fe, enc_ref = fe_enc.fe_ref, fe_enc.fe, fe_enc.enc_ref
     taps = {"stem": _Tap(fe_ref.frontend3D)}
     for li in range(1, 5):
         taps[f"layer{li}"] = _Tap(getattr(fe_ref.resnet18, f"layer{li}"))
-    for i, lyr in enumerate(ref.encoder.layer_stack):
+    for i, lyr in enumerate(enc_ref.layer_stack):
         taps[f"enc_layer{i}"] = _Tap(lyr, pick=lambda o: o[0])
-    with torch.no_grad(), ref_runtime.dropout_neutralised(R):
-        feat_ref = fe_ref(x)                                              # [N,T,512]
-        ref.encoder(feat_ref, [T] * n)
+    with torch.no_grad():
+        feat_ref = fe_ref._frontend_forward(x).view(n, T, 512)            # the frontend without its always-on dropout
+        enc_ref(feat_ref, [T] * n)
     want = {k: v.outs[0] for k, v in taps.items()}
     for v in taps.values():
         v.close()
@@ -430,17 +455,20 @@ def test_reference_transformer_on_all_dropins_recognize(models, dev):
     assert int((a_l2r == b_l2r).all(1).sum()) >= 38 and int((a_r2l == b_r2l).all(1).sum()) >= 36
 
 
-def test_native_decoder_cuda_graph_steps_equal_eager(models, native_decoder, dev):
+def test_native_decoder_cuda_graph_steps_equal_eager(fe_enc, dev):
     """The captured decode steps (one CUDA graph per prefix length, PDL on) return the bits of the eager launches, for
-    two different batch shapes in a row (plans are cached per shape) and after a weight change."""
-    from oracle import ref_runtime
+    two different batch shapes in a row (plans are cached per shape) and after a weight change.  Decoder weights: the
+    reference initialisation under a fixed seed; encoder outputs: the reference's fp32 frontend + encoder."""
     from sbl_for_multilingual_lip_reading_b200 import synth
-    R, ref, ours = models
-    with torch.no_grad(), ref_runtime.dropout_neutralised(R):
+    from sbl_for_multilingual_lip_reading_b200.decoder import Decoder
+    torch.manual_seed(7)
+    native_decoder = Decoder(0, 1, 58, 512, 6, 8, 64, 64, 512, 2048, dropout=0.1, tgt_emb_prj_weight_sharing=1,
+                             pe_maxlen=5000).to(dev).eval()
+    with torch.no_grad():
         for n, t, seed in ((5, 29, 1), (12, 40, 2), (5, 29, 3)):
-            x = synth.structured_clips(n, t, seed=600 + seed)[:, 0].to(dev)
-            feat = ref.visual_frontend(x.unsqueeze(4).permute(0, 4, 1, 2, 3))
-            enc, *_ = ref.encoder(feat, [t] * n)
+            x = synth.structured_clips(n, t, seed=600 + seed).to(dev)
+            feat = fe_enc.fe_ref._frontend_forward(x).view(n, t, 512)
+            enc, *_ = fe_enc.enc_ref(feat, [t] * n)
             native_decoder.use_cuda_graphs = True
             a = native_decoder._greedy(enc, want_logits=True)
             native_decoder.use_cuda_graphs = False

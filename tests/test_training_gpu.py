@@ -1,6 +1,7 @@
 """`-m gpu` tests of the training path (BASELINE configs[3]; SURVEY.md 8f.2): every new kernel against the torch op it
 replaces, then the drop-in modules in `model.train()` — forward with batch statistics, backward, running-stat updates —
-against autograd through the UNMODIFIED reference modules (oracle/_ref) in fp32 on the same B200.
+against autograd through the reference's modules in fp32 on the same B200 (oracle/reference_modules.py: the reference
+classes restated in torch.nn, pinned to the reference's own outputs by tests/test_oracle_golden.py).
 
 Tolerance: relative Frobenius error; 2e-2 for gradients (bf16 operands and bf16 gradient tensors, fp32 accumulation),
 stated per assertion where a deep chain needs more.
@@ -271,12 +272,12 @@ def _is_key_bias(k):
 
 def test_encoder_training_matches_reference_autograd(dev):
     """Encoder in model.train() with dropout = 0: output, input gradient and every parameter gradient against autograd
-    through the reference Encoder (encoder.py / attention.py / module.py from oracle/_ref), ragged lengths included.
+    through the reference Encoder (encoder.py / attention.py / module.py, restated in oracle/reference_modules.py), ragged
+    lengths included.
     Tolerance 3e-2: gradient tensors and GEMM operands of the backward are bf16 (measured 1e-2 .. 2.2e-2)."""
-    from oracle import ref_runtime
+    from oracle import reference_modules as R
     from sbl_for_multilingual_lip_reading_b200 import synth
     from sbl_for_multilingual_lip_reading_b200.encoder import Encoder
-    R = ref_runtime.load_reference("sbl")
     n, t, L = 6, 29, 3
     sd = synth.encoder_state_dict(2, L)
     ref = R.Encoder(512, L, 8, 64, 64, 512, 2048, dropout=0.0, pe_maxlen=5000).to(dev).train()
@@ -312,10 +313,9 @@ def test_encoder_training_matches_reference_autograd(dev):
 def test_encoder_training_dropout_draws_reference_masks(dev):
     """With dropout 0.1 and the same CUDA seed the training path draws its masks with the same torch calls, shapes and
     order as the reference's nn.Dropout modules, so outputs stay within tolerance of the seeded reference run."""
-    from oracle import ref_runtime
+    from oracle import reference_modules as R
     from sbl_for_multilingual_lip_reading_b200 import synth
     from sbl_for_multilingual_lip_reading_b200.encoder import Encoder
-    R = ref_runtime.load_reference("sbl")
     n, t, L = 4, 29, 2
     sd = synth.encoder_state_dict(2, L)
     ref = R.Encoder(512, L, 8, 64, 64, 512, 2048, dropout=0.1, pe_maxlen=5000).to(dev).train()
@@ -334,10 +334,9 @@ def test_encoder_training_dropout_draws_reference_masks(dev):
 
 
 def _frontend_pair(dev, matched):
-    from oracle import ref_runtime
+    from oracle import reference_modules as R
     from sbl_for_multilingual_lip_reading_b200 import synth
     from sbl_for_multilingual_lip_reading_b200.video_frontend import Lipreading
-    R = ref_runtime.load_reference("sbl")
     sd = synth.frontend_state_dict(1)
     if matched:
         sd = _bf16_values(sd)
@@ -390,10 +389,9 @@ def test_basic_block_training_backward_against_precision_matched_reference(dev, 
     activations rounded to bf16 at the drop-in's storage points (straight-through) and bf16-representable weights and
     input differentiates the same function up to accumulation order; what is left is the bf16 rounding of the gradient
     tensors (and the few ReLU masks a 1-ulp forward difference still flips)."""
-    from oracle import ref_runtime
+    from oracle import reference_modules as R
     from sbl_for_multilingual_lip_reading_b200 import synth, training as tr
     from sbl_for_multilingual_lip_reading_b200.video_frontend import Lipreading
-    R = ref_runtime.load_reference("sbl")
     sd = _bf16_values(synth.frontend_state_dict(1))
     ref_fe, our_fe = R.Lipreading().to(dev).train(), Lipreading().to(dev).train()
     ref_fe.load_state_dict(sd); our_fe.load_state_dict(sd)
@@ -431,10 +429,9 @@ def test_basic_block_training_backward_against_precision_matched_reference(dev, 
 def test_stem_training_backward_against_precision_matched_reference(dev):
     """Conv3d + BatchNorm3d(batch stats) + ReLU + MaxPool3d in training mode: output and parameter gradients against the
     reference frontend3D with bf16 storage points (see above)."""
-    from oracle import ref_runtime
+    from oracle import reference_modules as R
     from sbl_for_multilingual_lip_reading_b200 import synth, training as tr
     from sbl_for_multilingual_lip_reading_b200.video_frontend import Lipreading
-    R = ref_runtime.load_reference("sbl")
     sd = _bf16_values(synth.frontend_state_dict(1))
     ref_fe, our_fe = R.Lipreading().to(dev).train(), Lipreading().to(dev).train()
     ref_fe.load_state_dict(sd); our_fe.load_state_dict(sd)
@@ -462,26 +459,24 @@ def test_stem_training_backward_against_precision_matched_reference(dev):
 
 def test_stage1_training_step_with_reference_heads(dev):
     """One optimisation step of the stage-1 classification model the way ...classify/train.py:107-146 runs it (frontend +
-    3-layer encoder + fc_1500 / fc_2 heads, CrossEntropy losses, Adam): the reference's Transformer class assembled on
-    the drop-ins (dropin.patch_reference on the CLS sub-project) against the all-reference fp32 model; dropout 0 so that
-    both see the same function.  The reference forward's pooling line (transformer.py:31, `torch.mean(..., dim=2,
-    keepdim=True)` -> fc_1500 on a width-1 tensor) cannot run as written; the heads are applied as SURVEY.md states
-    their evident intent: word logits from the time average, language logits from frame 30."""
-    from oracle import ref_runtime
-    from sbl_for_multilingual_lip_reading_b200 import dropin, synth
-    R = ref_runtime.load_reference("cls")
+    3-layer encoder + fc_1500 / fc_2 heads, CrossEntropy losses, Adam): the project's stage1.Stage1Classifier (drop-in
+    frontend + encoder, the reference's attribute names and keys) against the all-reference fp32 model as
+    oracle/reference_modules.py restates it; dropout 0 so that both see the same function.  The reference side's loss
+    must equal the loss the original classes computed in the same step (tests/golden/reference_training.json).
+    Assembling the reference's own Transformer class on the drop-ins (dropin.patched_reference) needs the reference
+    sources and is not what this test runs.  The reference forward's pooling line (transformer.py:31,
+    `torch.mean(..., dim=2, keepdim=True)` -> fc_1500 on a width-1 tensor) cannot run as written; the heads are applied
+    as SURVEY.md states their evident intent: word logits from the time average, language logits from frame 30."""
+    from oracle import reference_modules as R
+    from sbl_for_multilingual_lip_reading_b200 import stage1, synth
     n, t = 8, 31
     sd = dict(synth.frontend_state_dict(1, prefix="visual_frontend."))
     sd.update(synth.encoder_state_dict(3, 3, prefix="encoder_v."))
-    ref = ref_runtime.build_cls_reference(R, sd).to(dev).train()
+    ref = R.build_stage1(sd).to(dev).train()
     for m_ in ref.modules():
         if isinstance(m_, torch.nn.Dropout):
             m_.p = 0.0
-    with dropin.patched_reference(R.dir):
-        import transformer.encoder as tenc
-        import transformer.transformer as ttr
-        enc = tenc.Encoder(512, 3, 8, 64, 64, 512, 2048, dropout=0.0, pe_maxlen=5000)
-        ours = ttr.Transformer(enc, None)
+    ours = stage1.Stage1Classifier(n_layers_enc=3, dropout=0.0)
     ours.load_state_dict(ref.state_dict())
     ours = ours.to(dev).train()
     assert type(ours.visual_frontend).__module__.startswith("sbl_for_multilingual_lip_reading_b200")
@@ -505,6 +500,9 @@ def test_stage1_training_step_with_reference_heads(dev):
 
     la, ga = step(ref, 3)
     lb, gb = step(ours, 3)
+    with open(os.path.join(ROOT, "tests", "golden", "reference_training.json")) as f:
+        want = json.load(f)["stage1_step_loss"]
+    assert abs(la - want) < 1e-5 * abs(want), (la, want)
     cos = {k: _cosine(gb[k], ga[k]) for k in ga if not _is_key_bias(k)}
     with open(os.path.join(OUT_DIR, "r02_train_stage1_step.json"), "w") as f:
         json.dump({"loss_reference": la, "loss_b200": lb, "grad_cosine": cos}, f, indent=1)
@@ -537,10 +535,9 @@ def test_ddp_gradient_allreduce_two_gpus():
 
 def test_stage1_module_has_the_reference_state_dict(dev):
     """stage1.Stage1Classifier mirrors ...classify/transformer/transformer.py key for key."""
-    from oracle import ref_runtime
+    from oracle import reference_modules as R
     from sbl_for_multilingual_lip_reading_b200 import stage1
-    R = ref_runtime.load_reference("cls")
-    ref = ref_runtime.build_cls_reference(R)
+    ref = R.build_stage1()
     ours = stage1.Stage1Classifier(n_layers_enc=3)
     a, b = ref.state_dict(), ours.state_dict()
     assert sorted(a) == sorted(b)
