@@ -124,20 +124,19 @@ class Encoder(nn.Module):
         # clip groups per cluster of the one-launch stack when stack_cluster_size is forced: 2 = two groups interleaved
         # (half the SMs for ~1.5x the time: the pipelined plan's co-running encoder); bit-identical to 1
         self.stack_groups_per_cluster = 1
-        self._resident_counter = None   # int32 [2] CUDA tensor while runner.PipelinedVisualEncoderPlan captures (ops.gate_wait)
-        self._x16_override = None       # bf16 [N*T, d_input] copy of the input the plan has already made (skips the cast launch)
 
     def __getstate__(self):
         st = self.__dict__.copy()
         st["_packed"] = None
         st["_len_cache"] = {}
         st["_streams"] = {}
-        st["_resident_counter"] = None
-        st["_x16_override"] = None
         return st
 
+    # attributes of modules pickled by earlier versions that nothing reads any more (the plans' former hooks)
+    _RETIRED = ("_resident_counter", "_x16_override")
+
     def __setstate__(self, st):
-        self.__dict__.update(st)
+        self.__dict__.update({k: v for k, v in st.items() if k not in self._RETIRED})
         self.__dict__.setdefault("_streams", {})
         self.__dict__.setdefault("_len_cache", {})
         self.__dict__.setdefault("parallel_chains", 4)
@@ -148,8 +147,6 @@ class Encoder(nn.Module):
         self.__dict__.setdefault("split_clusters", True)
         self.__dict__.setdefault("stack_cluster_size", 0)
         self.__dict__.setdefault("stack_groups_per_cluster", 1)
-        self.__dict__.setdefault("_resident_counter", None)
-        self.__dict__.setdefault("_x16_override", None)
 
     # ------------------------------------------------------------------------------------------
     def _check_config(self):
@@ -316,6 +313,17 @@ class Encoder(nn.Module):
             self._check_train_config(t, return_attns)
             from . import training
             return training.encoder_forward_train(self, padded_input.float(), lens)
+        return self._forward_eval(padded_input, lens, return_attns)
+
+    def _forward_eval(self, padded_input, lens, return_attns=False, *, x16=None, cluster_size=None,
+                      groups_per_cluster=None, resident_counter=None):
+        """The evaluation forward of checked arguments.  The CUDA-graph plans (runner.py) pass the 16-bit copy of the
+        input they already hold (`x16` [N*T, d_input]: no cast launch, `padded_input` only gives the shape; one-launch
+        stack only), the cluster size and clip groups per cluster of the one-launch stack (default: stack_cluster_size /
+        stack_groups_per_cluster) and the `resident_counter` of ops.gate_wait."""
+        cl = self.stack_cluster_size if cluster_size is None else cluster_size
+        gpc = self.stack_groups_per_cluster if groups_per_cluster is None else groups_per_cluster
+        n, t, d_in = padded_input.shape
         m = n * t
         x = padded_input.detach()
         if x.dtype != torch.float32:
@@ -342,7 +350,7 @@ class Encoder(nn.Module):
                 # the whole stack as ONE launch: a cluster per clip group, no inter-group synchronisation
                 stk = pk.stacked
                 scale = 1.0 / self.layer_stack[0].slf_attn.temperature
-                x16 = self._x16_override if self._x16_override is not None else ops.cast_enc16(x)
+                x16 = ops.cast_enc16(x) if x16 is None else x16
                 g_clips = max(1, 128 // t)
                 groups = -(-n // g_clips)
                 if groups > self.fused_stack_max_groups:
@@ -360,12 +368,12 @@ class Encoder(nn.Module):
                             ops.encoder_stack(x16[n0 * t:n1 * t], stk, n1 - n0, t,
                                               lengths=None if lengths is None else lengths[n0:n1], scale=scale,
                                               eps=self.layer_norm_in.eps, out=out[n0 * t:n1 * t],
-                                              cluster_size=self.stack_cluster_size or 8)
+                                              cluster_size=cl or 8)
                     join = torch.cuda.Event()
                     join.record(side)
                     main.wait_event(join)
                     return (out.view(n, t, self.d_model),)
-                if self.split_clusters and self.stack_cluster_size == 0 and 7 < groups <= 11:
+                if self.split_clusters and cl == 0 and 7 < groups <= 11:
                     # Only 7 clusters of 16 CTAs are co-resident on a B200, and 16-CTA clusters are the faster ones (each
                     # CTA streams half the weights).  The first 7 clip groups run as 16-CTA clusters; the remaining 1-4
                     # groups run at the same time, on a side stream, as 8-CTA clusters in the SMs the big clusters leave
@@ -386,9 +394,11 @@ class Encoder(nn.Module):
                     main.wait_event(ev2)
                 else:
                     ops.encoder_stack(x16, stk, n, t, lengths=lengths, scale=scale, eps=self.layer_norm_in.eps, out=out,
-                                      cluster_size=self.stack_cluster_size, resident_counter=self._resident_counter,
-                                      groups_per_cluster=self.stack_groups_per_cluster if self.stack_cluster_size else 1)
+                                      cluster_size=cl, resident_counter=resident_counter,
+                                      groups_per_cluster=gpc if cl else 1)
                 return (out.view(n, t, self.d_model),)
+            if x16 is not None:
+                raise RuntimeError("Encoder: a 16-bit input copy is only read by the one-launch stack")
             groups = 1 if return_attns else max(1, min(self.parallel_chains, n // 4))
             if groups == 1:
                 self._run_chain(x, out, pk, 0, n, t, lengths, return_attns, attns)

@@ -14,7 +14,8 @@ graph per input slot (streams + graphs instead of a tracing compiler) and expose
 (latency-bound, 64-SM) encoder stack of batch i-1 runs next to the clip prep + Conv3d stem of batch i.
 
 The modules stay ordinary drop-ins: a plan is an optional accelerator around them, owning only torch tensors,
-streams and graphs.
+streams and graphs.  It passes its schedule to them as arguments (`Lipreading._frontend_forward`,
+`Encoder._forward_eval`) and never changes their attributes.
 """
 from __future__ import annotations
 
@@ -65,9 +66,7 @@ class VisualEncoderPlan:
         of them (a cache eviction or a re-pack after `load_state_dict` can then never free memory a replay still reads
         or writes) and records the weight versions it was captured with; `_check_weights` refuses to replay stale ones."""
         fe, enc = self.frontend, self.encoder
-        self._pinned = (getattr(fe, "_packed", None), getattr(enc, "_packed", None),
-                        dict(getattr(fe, "_flat_ws", {})), dict(getattr(enc, "_len_cache", {})),
-                        dict(getattr(fe, "_lut", {})), getattr(fe, "l2_prefetch_extra", None))
+        self._pinned = (fe._packed, enc._packed, dict(fe._flat_ws), dict(enc._len_cache), dict(fe._lut))
         # the parameter / buffer OBJECTS are fixed for a module's life (load_state_dict, .to() and optimizers update them
         # in place), so the per-replay check walks a cached flat list instead of the module tree (~20 us)
         self._wtensors = [t for m in (fe, enc) for t in list(m.parameters()) + list(m.buffers())]
@@ -89,53 +88,64 @@ class VisualEncoderPlan:
             self._pin_captured_state()
 
     # -------------------------------------------------------------------------------------------
-    def _forward_eager(self, x):
+    def _u8_crop(self):
+        """The loader's 88x88 centre crop of the raw frames (CenterCrop, data_gen.py)."""
+        _, h0, w0 = self.u8_input
+        return (h0 - 88) // 2, (w0 - 88) // 2
+
+    def _frontend_eager(self, x):
         if self.u8_input is not None:
-            _, h0, w0 = self.u8_input
-            feat = self.frontend.forward_u8(x, frames=self.t, crop=((h0 - 88) // 2, (w0 - 88) // 2))
-        else:
-            feat = self.frontend(x)
-        out, = self.encoder(feat, self.lengths)
+            return self.frontend.forward_u8(x, frames=self.t, crop=self._u8_crop())
+        return self.frontend(x)
+
+    def _forward_eager(self, x):
+        out, = self.encoder(self._frontend_eager(x), self.lengths)
         return out
+
+    def _trunk(self, x, **schedule):
+        """The frontend of the input slot `x` with the plan's schedule (Lipreading._frontend_forward)."""
+        if self.u8_input is None:
+            return self.frontend._frontend_forward(x, **schedule)
+        x, frames, prep = self.frontend._u8_prep(x, self.t, self._u8_crop())
+        return self.frontend._frontend_forward(x, prep=prep, frames=frames, **schedule)
+
+    def _draw_dropout(self, drawn, out=None):
+        """Forks the draw of the always-on dropout's factor F.dropout(ones, p=0.5) (Lipreading.forward, reference :122: the
+        same generator draw as the module's F.dropout(features)) onto the tail stream and records `drawn` there once it
+        is done.  Returns the factor (`out` when given: the draw is copied into it)."""
+        fork = torch.cuda.Event()
+        fork.record(torch.cuda.current_stream())
+        self._tail_stream.wait_event(fork)
+        with torch.cuda.stream(self._tail_stream):
+            scale = torch.nn.functional.dropout(self._ones, p=0.5)
+            if out is not None:
+                scale = out.copy_(scale)
+            drawn.record(self._tail_stream)
+        return scale
 
     def _forward_fused_tail(self, s):
         """encoder(frontend(x[s])) with the dropout factor drawn off the critical path and the pooling launch writing the
         encoder's operand (capture-time only; see _capture)."""
-        fe, enc = self.frontend, self.encoder
         main = torch.cuda.current_stream()
         scale, join = None, None
-        if getattr(fe, "always_on_dropout", True):
-            fork, drawn = torch.cuda.Event(), torch.cuda.Event()
-            fork.record(main)
-            self._tail_stream.wait_event(fork)
-            with torch.cuda.stream(self._tail_stream):
-                scale = torch.nn.functional.dropout(self._ones, p=0.5)
-                drawn.record(self._tail_stream)
+        if self.frontend.always_on_dropout:
+            drawn = torch.cuda.Event()
+            scale = self._draw_dropout(drawn)
             join = lambda: main.wait_event(drawn)   # noqa: E731  (called right before the pooling launch)
-        saved = (fe._tail, enc._x16_override)
-        try:
-            fe._tail = (scale, self.feat16[s], join)
-            if self.u8_input is not None:
-                _, h0, w0 = self.u8_input
-                f = fe.forward_u8(self.x[s], frames=self.t, crop=((h0 - 88) // 2, (w0 - 88) // 2))
-            else:
-                f = fe(self.x[s])
-            del f   # unwritten: the pooling launch wrote the 16-bit features into feat16[s]
-            fe._tail = None
-            enc._x16_override = self.feat16[s]
-            out, = enc(self.feat, self.lengths)
-        finally:
-            fe._tail, enc._x16_override = saved
+        self._trunk(self.x[s], prefetch_extra=self._prefetch, scale=scale, out16=self.feat16[s], before_pool=join)
+        out, = self.encoder._forward_eval(self.feat, self.lengths, x16=self.feat16[s])
         return out
 
     def _capture(self):
         torch.cuda.synchronize(self.device)
+        fe, enc = self.frontend, self.encoder
         with torch.no_grad():
             # the frontend pulls the encoder's packed weights into L2 while its last layer runs (side stream)
-            if getattr(self.frontend, "l2_prefetch", False) and hasattr(self.encoder, "_get_packed"):
+            self._prefetch = []
+            if fe.l2_prefetch:
                 with torch.cuda.device(self.device):
-                    stk = self.encoder._get_packed().stacked
-                self.frontend.l2_prefetch_extra = [stk[k] for k in ("w_in", "w_heads", "w_fc", "w_1", "w_2")]
+                    stk = enc._get_packed().stacked
+                self._prefetch = [stk[k] for k in ("w_in", "w_heads", "w_fc", "w_1", "w_2")]
             # warm-up on the capture stream: packs weights, sizes kernels, stages the lengths vector
             with torch.cuda.stream(self.compute):
                 for _ in range(2):
@@ -144,14 +154,11 @@ class VisualEncoderPlan:
             # One private memory pool PER graph: with a shared pool the static output of one slot may alias an
             # intermediate buffer of the other slot's graph, and submit_host lets the device->host copy of slot s overlap
             # the replay of slot s^1 (a few hundred MB per pool; HBM is not the constraint here).
-            fe, enc = self.frontend, self.encoder
             # Fused tail (same as the pipelined plan): the always-on dropout factor of Lipreading.forward (reference :122)
             # is drawn on a side stream while the trunk runs and applied by the pooling launch, which writes the encoder's
             # 16-bit operand directly — no dropout / cast launches between the last conv and the encoder stack.
             # Bit-identical to the module path (same generator draw, same single rounding).
-            fused_tail = (hasattr(fe, "_tail") and hasattr(enc, "_x16_override") and hasattr(enc, "_use_fused_stack")
-                          and getattr(fe, "parallel_chains", 1) == 1 and not fe.training and not enc.training
-                          and enc._use_fused_stack(self.n, self.t, False))
+            fused_tail = not fe.training and not enc.training and enc._use_fused_stack(self.n, self.t, False)
             if fused_tail:
                 dev = self.device
                 self.feat16 = [torch.zeros((self.n * self.t, fe.inputDim), dtype=ops.enc16_dtype(), device=dev)
@@ -290,8 +297,6 @@ class PipelinedVisualEncoderPlan(VisualEncoderPlan):
         torch.cuda.synchronize(dev)
         self.enc_stream = torch.cuda.Stream(device=dev, priority=-1)
         self.gate = torch.zeros(2, dtype=torch.int32, device=dev)
-        if getattr(fe, "parallel_chains", 1) != 1:
-            raise RuntimeError("PipelinedVisualEncoderPlan needs frontend.parallel_chains == 1")
         # features cross the pipeline stages as the bf16 GEMM operand the encoder stack reads (written by the frontend's
         # last launch — average pool x dropout factor — so the encoder branch of the next replay is the stack kernel
         # alone); `feat` only carries the shape
@@ -300,82 +305,47 @@ class PipelinedVisualEncoderPlan(VisualEncoderPlan):
         self._ones = torch.ones((self.n * self.t, fe.inputDim), dtype=torch.float32, device=dev)
         self._tail_stream = torch.cuda.Stream(device=dev)
         self._scale = [torch.empty_like(self._ones) for _ in range(2)]
-        saved = (enc.stack_cluster_size, enc._resident_counter, fe._overlap, enc._x16_override, fe._tail,
-                 enc.stack_groups_per_cluster)
-        saved_pf = (getattr(fe, "l2_prefetch", False), getattr(fe, "l2_prefetch_extra", None))
-        try:
-            with torch.no_grad():
-                stk = enc._get_packed().stacked
-                fe.l2_prefetch = bool(saved_pf[0]) and self.l2_prefetch
-                fe.l2_prefetch_extra = None
-                if getattr(fe, "l2_prefetch", False):
-                    fe.l2_prefetch_extra = [stk[k] for k in ("w_in", "w_heads", "w_fc", "w_1", "w_2")]
-                enc.stack_cluster_size = cl
-                enc.stack_groups_per_cluster = gpc
-                with torch.cuda.stream(self.compute):   # warm-up: packs weights, sizes kernels, stages the lengths
-                    for _ in range(2):
-                        self._forward_eager(self.x[0])
-                self.compute.synchronize()
-                for s in range(2):   # one private pool per graph (see VisualEncoderPlan._capture)
-                    g = torch.cuda.CUDAGraph()
-                    before = ops.launch_count()
-                    with torch.cuda.graph(g, stream=self.compute):
-                        main = torch.cuda.current_stream()
-                        fork, done = torch.cuda.Event(), torch.cuda.Event()
-                        fork.record(main)
-                        self.enc_stream.wait_event(fork)
-                        with torch.cuda.stream(self.enc_stream):
-                            enc._resident_counter = self.gate if self.use_gate else None
-                            enc._x16_override = self.feat16[s ^ 1]
-                            self.out[s ^ 1], = enc(self.feat, self.lengths)
-                            enc._resident_counter = enc._x16_override = None
-                            done.record(self.enc_stream)
-                        if self.use_gate:
-                            ops.gate_wait(self.gate, enc_ctas, self.gate_timeout_us)
-                        # the always-on dropout of Lipreading.forward (reference :122): its factor mask / (1 - p) is drawn
-                        # here, in front of the (non-critical) head, and applied by the pooling launch that ends the trunk
-                        # The draw is forked onto a side stream right before layer 4 is enqueued: its two small launches
-                        # cost 10-12 us of the step at the start of the replay (in stream OR on a side stream: they take
-                        # SMs while the encoder's clusters and the gated stem are being placed, tools/exp/
-                        # pipeline_switches_probe.py), while the 132-CTA grids of layer 4 leave 16 SMs idle anyway.
-                        scale, tail_join = None, None
-                        if getattr(fe, "always_on_dropout", True):
-                            scale = self._scale[s]
-                            drawn = torch.cuda.Event()
-
-                            fired = []
-
-                            def draw(scale=scale, drawn=drawn, main=main, fired=fired):
-                                fired.append(True)
-                                ev = torch.cuda.Event()
-                                ev.record(main)
-                                self._tail_stream.wait_event(ev)
-                                with torch.cuda.stream(self._tail_stream):
-                                    scale.copy_(torch.nn.functional.dropout(self._ones, p=0.5))
-                                    drawn.record(self._tail_stream)
-                            fe._block_hook = (6, draw)
-                            tail_join = (lambda ev: (lambda: main.wait_event(ev)))(drawn)
-                        fe._tail = (scale, self.feat16[s], tail_join)
-                        fe._overlap = (self.head_sm_limit, self.head_blocks, lambda: main.wait_event(done),
-                                       self.head_frac)
-                        if self.u8_input is not None:
-                            _, h0, w0 = self.u8_input
-                            f = fe.forward_u8(self.x[s], frames=self.t, crop=((h0 - 88) // 2, (w0 - 88) // 2))
-                        else:
-                            f = fe(self.x[s])
-                        if fe._block_hook is not None and not fired:
-                            raise RuntimeError("PipelinedVisualEncoderPlan: the frontend never reached residual block 6 "
-                                               "(the dropout factor was not drawn)")
-                        fe._overlap = fe._tail = fe._block_hook = None
-                        del f   # unwritten: the pooling launch wrote the bf16 features into feat16[s]
-                    self.launches_per_forward = ops.launch_count() - before
-                    self.graphs[s] = g
-        finally:
-            (enc.stack_cluster_size, enc._resident_counter, fe._overlap, enc._x16_override, fe._tail,
-             enc.stack_groups_per_cluster) = saved
-            fe._block_hook = None
-            keep_extra = fe.l2_prefetch_extra if fe.l2_prefetch else saved_pf[1]
-            fe.l2_prefetch, fe.l2_prefetch_extra = saved_pf[0], keep_extra
+        stack = dict(cluster_size=cl, groups_per_cluster=gpc)
+        prefetch = fe.l2_prefetch and self.l2_prefetch
+        with torch.no_grad():
+            stk = enc._get_packed().stacked
+            self._prefetch = [stk[k] for k in ("w_in", "w_heads", "w_fc", "w_1", "w_2")] if prefetch else []
+            with torch.cuda.stream(self.compute):   # warm-up: packs weights, sizes kernels, stages the lengths
+                for _ in range(2):
+                    enc._forward_eval(self._frontend_eager(self.x[0]), self.lengths, **stack)
+            self.compute.synchronize()
+            for s in range(2):   # one private pool per graph (see VisualEncoderPlan._capture)
+                g = torch.cuda.CUDAGraph()
+                before = ops.launch_count()
+                with torch.cuda.graph(g, stream=self.compute):
+                    main = torch.cuda.current_stream()
+                    fork, done = torch.cuda.Event(), torch.cuda.Event()
+                    fork.record(main)
+                    self.enc_stream.wait_event(fork)
+                    with torch.cuda.stream(self.enc_stream):
+                        self.out[s ^ 1], = enc._forward_eval(self.feat, self.lengths, x16=self.feat16[s ^ 1],
+                                                             resident_counter=self.gate if self.use_gate else None,
+                                                             **stack)
+                        done.record(self.enc_stream)
+                    if self.use_gate:
+                        ops.gate_wait(self.gate, enc_ctas, self.gate_timeout_us)
+                    # the always-on dropout of Lipreading.forward (reference :122): its factor mask / (1 - p) is drawn
+                    # on a side stream and applied by the pooling launch that ends the trunk.  The draw is forked right
+                    # before layer 4 (residual block 6) is enqueued: its two small launches cost 10-12 us of the step at
+                    # the start of the replay (in stream OR on a side stream: they take SMs while the encoder's clusters
+                    # and the gated stem are being placed, tools/exp/pipeline_switches_probe.py), while the 132-CTA
+                    # grids of layer 4 leave 16 SMs idle anyway.
+                    scale, draw, join = None, None, None
+                    if fe.always_on_dropout:
+                        scale, drawn = self._scale[s], torch.cuda.Event()
+                        draw = lambda: self._draw_dropout(drawn, out=scale)   # noqa: E731
+                        join = lambda: main.wait_event(drawn)   # noqa: E731
+                    self._trunk(self.x[s], head_sm_limit=self.head_sm_limit, head_blocks=self.head_blocks,
+                                head_join=lambda: main.wait_event(done), head_frac=self.head_frac,
+                                hook=draw, hook_block=6, scale=scale, out16=self.feat16[s], before_pool=join,
+                                prefetch=prefetch, prefetch_extra=self._prefetch)
+                self.launches_per_forward = ops.launch_count() - before
+                self.graphs[s] = g
         torch.cuda.synchronize(dev)
         for ev in self.ev_out + self.ev_done:
             ev.record(torch.cuda.current_stream(dev))
@@ -413,18 +383,12 @@ class PipelinedVisualEncoderPlan(VisualEncoderPlan):
         """Encoder of the last submitted batch (eager, on the compute stream).  Returns its device output; also copies it
         to `out_host` when given."""
         s = (self._i - 1) % 2
-        enc = self.encoder
-        saved = (enc.stack_cluster_size, enc.stack_groups_per_cluster)
         with torch.no_grad(), torch.cuda.stream(self.compute):
             self.compute.wait_event(self.ev_out[s ^ 1])
-            try:
-                # nothing co-runs with this last encoder pass: the module's own (full-width, fastest) launch form instead
-                # of the 32-SM interleaved one the steady state uses — 195 vs 313 us at the BASELINE batch, same bits
-                enc.stack_cluster_size, enc._x16_override = 0, self.feat16[s]
-                enc.stack_groups_per_cluster = 1
-                out, = enc(self.feat, self.lengths)
-            finally:
-                (enc.stack_cluster_size, enc.stack_groups_per_cluster), enc._x16_override = saved, None
+            # nothing co-runs with this last encoder pass: the module's own (full-width, fastest) launch form instead
+            # of the 32-SM interleaved one the steady state uses — 195 vs 313 us at the BASELINE batch, same bits
+            out, = self.encoder._forward_eval(self.feat, self.lengths, x16=self.feat16[s], cluster_size=0,
+                                              groups_per_cluster=1)
             if out_host is not None:
                 out_host.copy_(out, non_blocking=True)
         return out

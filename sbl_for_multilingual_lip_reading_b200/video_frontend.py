@@ -114,17 +114,9 @@ class Lipreading(nn.Module):
         self._flat_ws = {}
         self._streams = {}
         self._lut = {}
-        self.parallel_chains = 1     # > 1: clip groups as concurrent kernel chains (measured SLOWER on B200, see _frontend_forward)
-        self.chain_sm_limit = 0      # > 0: each chain sizes its persistent grids for this many SMs
-        # L2 weight prefetch on a side stream (see _frontend_chain): layers 3-4 when layer 3 starts, and
-        # `l2_prefetch_extra` (a list of tensors: the encoder's packed weights, set by runner.VisualEncoderPlan) when
-        # layer 4 starts
+        # L2 weight prefetch on a side stream (see _frontend_forward): layers 1-2 while the stem runs, layers 3-4 when
+        # layer 3 starts.  The eager default; the CUDA-graph plans pass their own choice per call.
         self.l2_prefetch = True
-        self.l2_prefetch_extra = None
-        # (sm_limit, head_blocks, join[, head_frac]) set by runner.PipelinedVisualEncoderPlan while it captures: the clip prep, the stem
-        # and the first `head_blocks` residual blocks size their persistent grids for `sm_limit` SMs because another
-        # kernel chain (the previous batch's encoder stack) co-runs on the other SMs; `join()` is called once the head
-        # is enqueued and makes the current stream wait for that chain before the full-width kernels start
         # eval path: clip prep fused into the stem kernel (sblk_stem_fused_fwd: the stem's producer warps build the
         # row-Toeplitz entries from the fp32 clip, no prepped copy of the clip in HBM, one launch less; bit-identical).
         # Measured (tools/exp/stem_fused_probe.py, head_frac_probe.py): fp32 clips 91.1 -> 86.7 us alone, pipelined step
@@ -150,15 +142,6 @@ class Lipreading(nn.Module):
         # 45.7 vs 45.7 us and 58.0 vs 56.7 us per block, tools/exp/fuse_blocks_probe.py)
         self.fuse_blocks = True
         self.fuse_blocks_max = 256
-        self._overlap = None
-        # (scale | None, out_bf16) set by the same plan: the average pool writes mean * scale as bf16 straight into the
-        # plan's feature buffer — `scale` is F.dropout(ones, p=0.5) drawn at the start of the replay, i.e. the always-on
-        # dropout of forward() moved off the critical path (bit-identical) — and forward() skips its own dropout
-        self._tail = None
-        # (block index, callable) set by a plan while it captures: called on the main stream right before that residual
-        # block is enqueued (the pipelined plan forks its dropout draw in front of layer 4, whose 132-CTA grids leave
-        # SMs idle)
-        self._block_hook = None
 
     # ---- pickling / state: the packed cache holds plain tensors but is cheap to rebuild; drop it ----------
     def __getstate__(self):
@@ -167,30 +150,24 @@ class Lipreading(nn.Module):
         st["_flat_ws"] = {}
         st["_streams"] = {}
         st["_lut"] = {}
-        st["l2_prefetch_extra"] = None
-        st["_overlap"] = None
-        st["_tail"] = None
-        st["_block_hook"] = None
         return st
 
+    # attributes of modules pickled by earlier versions that nothing reads any more (the plans' former hooks, the
+    # retired multi-chain frontend)
+    _RETIRED = ("parallel_chains", "chain_sm_limit", "l2_prefetch_extra", "_overlap", "_tail", "_block_hook")
+
     def __setstate__(self, st):
-        self.__dict__.update(st)
+        self.__dict__.update({k: v for k, v in st.items() if k not in self._RETIRED})
         self.__dict__.setdefault("_flat_ws", {})
         self.__dict__.setdefault("_streams", {})
         self.__dict__.setdefault("_lut", {})
-        self.__dict__.setdefault("parallel_chains", 1)
-        self.__dict__.setdefault("chain_sm_limit", 0)
         self.__dict__.setdefault("l2_prefetch", True)
-        self.__dict__.setdefault("l2_prefetch_extra", None)
-        self.__dict__.setdefault("_overlap", None)
         self.__dict__.setdefault("fuse_prep", True)
         self.__dict__.setdefault("fuse_prep_u8", False)
         self.__dict__.setdefault("fold_downsample", True)
         self.__dict__.setdefault("alternate_tile_order", True)
         self.__dict__.setdefault("fuse_blocks", True)
         self.__dict__.setdefault("fuse_blocks_max", 256)
-        self.__dict__.setdefault("_tail", None)
-        self.__dict__.setdefault("_block_hook", None)
 
     def _initialize_weights(self):  # same as reference :127-157
         for m in self.modules():
@@ -260,12 +237,12 @@ class Lipreading(nn.Module):
         self._packed = pk
         return pk
 
-    def _flat_workspace(self, a, cout, stride, chain=0):
+    def _flat_workspace(self, a, cout, stride):
         """Two zero-initialised flat buffers for the outputs of a strided block head.  Only pixel rows are ever written
         (sblk_conv2d_dual_igemm_fwd, flat_out), so the halo rows stay zero across calls; cached per (device, shape)."""
         f, h, w_ = (a.f, a.h, a.w) if isinstance(a, ops.FlatActs) else a.shape[:3]
         p, q = (h - 1) // stride + 1, (w_ - 1) // stride + 1
-        key = (str(a.data.device if isinstance(a, ops.FlatActs) else a.device), f, p, q, cout, chain)
+        key = (str(a.data.device if isinstance(a, ops.FlatActs) else a.device), f, p, q, cout)
         ws = self._flat_ws.get(key)
         if ws is None:
             if len(self._flat_ws) > 16:   # (plans pin the entries their graphs use: runner._pin_captured_state)
@@ -287,22 +264,57 @@ class Lipreading(nn.Module):
             x = x.clone()
         return x
 
-    def _frontend_chain(self, x, pk, feat_out, chain, prep=ops.prep_clip):
-        """prep -> Conv3d stem -> ResNet-18 trunk -> average pool for the clips of `x`, on the current stream; writes
-        feat_out [n*T, 512] fp32.  `prep` turns `x` into the stem's prepped layout (fp32 clips: ops.prep_clip; raw
-        uint8 frames: ops.prep_clip_u8 with the normalisation table / crop / frame padding bound in)."""
-        ov = self._overlap if chain == 0 else None
-        head = {"limit": ops.set_sm_limit(ov[0])} if ov is not None else None
-        try:
-            self._frontend_chain_body(x, pk, feat_out, chain, prep, ov, head)
-        finally:
-            if head is not None and "limit" in head:
-                ops.set_sm_limit(head.pop("limit"))
+    def _prefetch_stream(self, device):
+        key = str(device)
+        if key not in self._streams:
+            self._streams[key] = torch.cuda.Stream(device=device)
+        return self._streams[key]
 
-    def _frontend_chain_body(self, x, pk, feat_out, chain, prep, ov, head):
+    def _frontend_forward(self, x, prep=ops.prep_clip, frames=None, *, head_sm_limit=None, out16=None, **schedule):
+        """reference :111-117 — prep -> Conv3d stem -> ResNet-18 trunk -> average pool on the current stream; returns the
+        pooled features [N*T,512] fp32 (before the always-on dropout).  `prep` turns `x` into the stem's prepped layout
+        (fp32 clips: ops.prep_clip; raw uint8 frames with `frames` output frames: the closure of _u8_prep).
+
+        The keyword arguments (these two and those of _trunk) are the schedule of the CUDA-graph plans (runner.py);
+        unset, they mean the eager path.
+        * head_sm_limit (0 = all SMs): the clip prep, the stem and the first `head_blocks` residual blocks size their
+          persistent grids for that many SMs because another kernel chain (the previous batch's encoder stack) co-runs
+          on the other SMs; `head_join()` is called once the head is enqueued and makes the current stream wait for that
+          chain before the full-width kernels start.  head_frac > 0: that share of the frames of the first conv after
+          the head still runs inside it.
+        * out16: the pooling launch writes mean * `scale` (the always-on dropout's factor drawn ahead of time, or None)
+          straight into this 16-bit encoder operand instead of the fp32 features (bit-identical), after `before_pool()`
+          has been called; returns None.
+        * hook(): called on the current stream right before residual block `hook_block` is enqueued.
+        * prefetch (default: the module's l2_prefetch): L2 weight hints on a side stream; the tensors of `prefetch_extra`
+          (the encoder's packed weights) are hinted when layer 4 starts."""
+        if frames is None:
+            x = self._check_input(x)
+            n, t = x.shape[0], x.shape[2]
+        else:           # raw uint8 frames, already validated by _u8_prep
+            n, t = x.shape[0], frames
+        pk = self._get_packed()
+        with torch.cuda.device(x.device):
+            feat = None if out16 is not None else torch.empty((n * t, self.inputDim), dtype=torch.float32,
+                                                               device=x.device)
+            head = [] if head_sm_limit is None else [ops.set_sm_limit(head_sm_limit)]   # the limit to restore
+            try:
+                self._trunk(x, pk, prep, feat, out16, head, **schedule)
+            finally:
+                if head:
+                    ops.set_sm_limit(head.pop())
+        return feat
+
+    def _trunk(self, x, pk, prep, feat, out16, head, *, head_blocks=0, head_join=None, head_frac=0.0, scale=None,
+               before_pool=None, hook=None, hook_block=0, prefetch=None, prefetch_extra=()):
+        if hook is not None and not 0 <= hook_block < len(pk.blocks):
+            raise RuntimeError(f"hook_block={hook_block}: the trunk has residual blocks 0..{len(pk.blocks) - 1}")
+        if prefetch is None:
+            prefetch = self.l2_prefetch
+
         def end_head():   # back to full-width grids; the co-running chain must be finished before they start
-            ops.set_sm_limit(head.pop("limit"))
-            ov[2]()
+            ops.set_sm_limit(head.pop())
+            head_join()
 
         # fuse_prep: the stem's producer warps build the row-Toeplitz entries themselves (ops.RawClip) instead of reading
         # a prepped copy of the clip written by a separate launch (bit-identical)
@@ -318,35 +330,34 @@ class Lipreading(nn.Module):
             return rev[0]
         for bi, (stride, w1, b1, w2, b2, ds) in enumerate(pk.blocks):
             split = 0
-            if ov is not None and bi == ov[1]:
+            if head and bi == head_blocks:
                 # head_frac > 0: the first conv of this block is run in two frame ranges — the first one still inside
                 # the head (limited width, next to the other chain), the rest at full width — to use the time by which
                 # the other chain outlasts the head.  Frame ranges of the flat layout are independent (ops.flat_frames).
-                if (len(ov) > 3 and ov[3] > 0 and isinstance(a, ops.FlatActs) and stride == 1 and ds is None
-                        and a.f >= 2):
-                    split = min(a.f - 1, max(1, int(round(a.f * float(ov[3])))))
+                if head_frac > 0 and isinstance(a, ops.FlatActs) and stride == 1 and ds is None and a.f >= 2:
+                    split = min(a.f - 1, max(1, int(round(a.f * float(head_frac)))))
                     y = ops.FlatActs(torch.empty_like(a.data), a.f, a.h, a.w)
                     split_rev = flip()
                     ops.conv3x3_flat(ops.flat_frames(a, 0, split), w1, b1, relu=True,
                                      out=ops.flat_frames(y, 0, split).data, reverse=split_rev)
                 end_head()
-            if self._block_hook is not None and chain == 0 and bi == self._block_hook[0]:
-                self._block_hook[1]()
-            if self.l2_prefetch and chain == 0 and bi in (0, 4, 6):
+            if hook is not None and bi == hook_block:
+                hook()
+            if prefetch and bi in (0, 4, 6):
                 # Weights of the layers still to come are pulled into L2 by a tiny kernel on a side stream while the
                 # current layer computes (layers 3-4 move few activation bytes, so the lines survive).  Benchmarks flush
                 # L2 between forwards and a serving loop evicts the 61 MB of weights with ~600 MB of activations per
                 # batch: without this, every kernel's first weight tiles and the encoder stack's whole dependent chain
                 # of weight loads pay DRAM latency.
                 if bi == 6:
-                    tensors = list(self.l2_prefetch_extra or ())
+                    tensors = list(prefetch_extra)
                 else:   # layers 1-2 (1.5 MB) while the stem runs, layers 3-4 (28 MB) when layer 3 starts
                     tensors = [t_ for blk in (pk.blocks[:4] if bi == 0 else pk.blocks[4:])
                                for t_ in (blk[1], blk[3]) + (tuple(blk[5][:1]) if blk[5] else ())]
                 if tensors:
                     main = torch.cuda.current_stream()
                     if pf_stream is None:
-                        pf_stream = self._side_streams(x.device, max(1, int(self.parallel_chains)))[-1]
+                        pf_stream = self._prefetch_stream(x.device)
                     ev = torch.cuda.Event()
                     ev.record(main)
                     pf_stream.wait_event(ev)
@@ -363,7 +374,7 @@ class Lipreading(nn.Module):
             if ds is not None:   # conv1 and the 1x1 downsample branch share one pass over the block input
                 if w2.dim() == 2:  # layer2: the block stays in the flat layout (conv2 is a flat stride-1 conv)
                     y, res = ops.conv2d_dual(a, w1, b1, ds[0], ds[1], stride=stride, relu=True,
-                                             flat_ws=self._flat_workspace(a, w1.shape[0], stride, chain))
+                                             flat_ws=self._flat_workspace(a, w1.shape[0], stride))
                     rev[0] = False   # the dual head writes its tiles front to back
                     a = ops.conv3x3_flat(y, w2, b2, relu=True, residual=res, reverse=flip())
                     continue
@@ -387,76 +398,21 @@ class Lipreading(nn.Module):
                         continue
                 y, res = ops.conv2d(a, w1, b1, stride=stride, relu=True), a
             a = ops.conv2d(y, w2, b2, stride=1, relu=True, residual=res)
-        if ov is not None and ov[1] >= len(pk.blocks):
+        if head:   # the whole trunk ran inside the head
             end_head()
-        tail = self._tail if chain == 0 else None
-        if tail is not None:
-            if len(tail) > 2 and tail[2] is not None:
-                tail[2]()   # the plan's side stream has drawn the dropout factor (VisualEncoderPlan._forward_fused_tail)
-            ops.avgpool(a, want_f32=False, out_bf16=tail[1], scale=tail[0], enc16=True)   # feat_out stays unwritten (plan-owned path)
+        if out16 is not None:
+            if before_pool is not None:
+                before_pool()
+            ops.avgpool(a, want_f32=False, out_bf16=out16, scale=scale, enc16=True)
         else:
-            ops.avgpool(a, out_f32=feat_out)
+            ops.avgpool(a, out_f32=feat)
         if pf_stream is not None:   # join (graph capture needs every forked stream back; no data dependency)
             ev = torch.cuda.Event()
             ev.record(pf_stream)
             torch.cuda.current_stream().wait_event(ev)
 
-    def _side_streams(self, device, k):
-        pool = self._streams.setdefault(str(device), [])
-        while len(pool) < k:
-            pool.append(torch.cuda.Stream(device=device))
-        return pool[:k]
-
-    def _frontend_forward(self, x, prep=ops.prep_clip, frames=None):
-        """reference :111-117 — returns pooled features [N*T,512] fp32 (before the always-on dropout).
-
-        `parallel_chains` > 1 splits the batch into contiguous clip groups whose kernel chains run on separate streams
-        (fork / join with events, capturable as parallel graph branches), optionally with each chain's persistent grids
-        sized for `chain_sm_limit` SMs.  Measured on B200 at the BASELINE batch (32 x 29 frames, graph replay): 1 chain
-        638 us, 2 chains 694 us, 2 chains x 74 SMs 704 us, 4 chains 792 us — the trunk kernels already fill the machine,
-        so concurrency only adds per-kernel fixed cost; the default stays 1 (the option is kept for small-SM parts)."""
-        if frames is None:
-            x = self._check_input(x)
-            n, t = x.shape[0], x.shape[2]
-        else:           # raw uint8 frames, already validated by forward_u8
-            n, t = x.shape[0], frames
-        pk = self._get_packed()
-        with torch.cuda.device(x.device):
-            feat = torch.empty((n * t, self.inputDim), dtype=torch.float32, device=x.device)
-            chains = max(1, min(int(self.parallel_chains), n // 8))
-            if chains == 1:
-                self._frontend_chain(x, pk, feat, 0, prep)
-                return feat
-            main = torch.cuda.current_stream()
-            side = self._side_streams(x.device, chains - 1)
-            fork = torch.cuda.Event()
-            fork.record(main)
-            bounds = [(g * n) // chains for g in range(chains + 1)]
-            prev_limit = ops.set_sm_limit(self.chain_sm_limit) if self.chain_sm_limit > 0 else None
-            try:
-                for g in range(chains):
-                    st = main if g == 0 else side[g - 1]
-                    if g > 0:
-                        st.wait_event(fork)
-                    with torch.cuda.stream(st):
-                        self._frontend_chain(x[bounds[g]:bounds[g + 1]], pk, feat[bounds[g] * t:bounds[g + 1] * t], g,
-                                             prep)
-            finally:
-                if prev_limit is not None:
-                    ops.set_sm_limit(prev_limit)
-            for g in range(1, chains):
-                ev = torch.cuda.Event()
-                ev.record(side[g - 1])
-                main.wait_event(ev)
-        return feat
-
-    def forward_u8(self, x_u8, frames=None, crop=(4, 4)):
-        """Fused input pipeline (SURVEY.md §8f.3): raw uint8 gray frames [N, T_in, H0, W0] (the loader's .npy layout,
-        H0 = W0 = 96 for LRW) -> the same [N, frames, 512] features `forward` returns for the clip the reference loader
-        would have built on the CPU (/255, ColorNormalize, 88x88 crop at `crop`, zero-padding to `frames` frames:
-        data_gen.py:122-125,276-296; cvtransforms.py:7-48).  `crop`: (y1, x1) or an int32 CUDA tensor [N*T_in, 2] of
-        per-frame offsets (RandomCrop).  Bit-identical to forward(reference-normalised fp32 clip); 4x fewer host->device
-        bytes."""
+    def _u8_prep(self, x_u8, frames, crop):
+        """Checks forward_u8's arguments; returns (x_u8, output frames, the prep closure for _frontend_forward)."""
         if self.training:
             raise RuntimeError("Lipreading.forward_u8 (libsblk) is the evaluation / serving input path; training runs "
                                "through forward() on the loader's augmented fp32 clips")
@@ -473,18 +429,25 @@ class Lipreading(nn.Module):
         if lut is None:
             from . import synth
             lut = self._lut[key] = synth.normalize_lut().to(x_u8.device)
-        if torch.is_tensor(crop):   # per-frame offsets are sliced with the clips when the batch is split into chains
+        if torch.is_tensor(crop):
             crop = crop.to(device=x_u8.device, dtype=torch.int32).contiguous()
-            if self.parallel_chains != 1:
-                raise RuntimeError("forward_u8: per-frame crop offsets need parallel_chains == 1")
 
         def prep(xs):
             if self.fuse_prep_u8:
                 return ops.raw_clip_u8(xs, lut, t_out, crop)
             return ops.prep_clip_u8(xs, lut, t_out, crop)
+        return x_u8, t_out, prep
 
+    def forward_u8(self, x_u8, frames=None, crop=(4, 4)):
+        """Fused input pipeline (SURVEY.md §8f.3): raw uint8 gray frames [N, T_in, H0, W0] (the loader's .npy layout,
+        H0 = W0 = 96 for LRW) -> the same [N, frames, 512] features `forward` returns for the clip the reference loader
+        would have built on the CPU (/255, ColorNormalize, 88x88 crop at `crop`, zero-padding to `frames` frames:
+        data_gen.py:122-125,276-296; cvtransforms.py:7-48).  `crop`: (y1, x1) or an int32 CUDA tensor [N*T_in, 2] of
+        per-frame offsets (RandomCrop).  Bit-identical to forward(reference-normalised fp32 clip); 4x fewer host->device
+        bytes."""
+        x_u8, t_out, prep = self._u8_prep(x_u8, frames, crop)
         feat = self._frontend_forward(x_u8, prep=prep, frames=t_out)
-        if self.always_on_dropout and self._tail is None:
+        if self.always_on_dropout:
             feat = F.dropout(feat, p=0.5)  # functional default training=True, exactly as reference :122
         return feat.view(-1, t_out, self.inputDim)
 
@@ -507,7 +470,7 @@ class Lipreading(nn.Module):
             feat = F.dropout(feat, p=0.5)  # reference :122 (functional default training=True); torch autograd
             return feat.view(-1, frameLen, self.inputDim)
         feat = self._frontend_forward(x)
-        if self.always_on_dropout and self._tail is None:
+        if self.always_on_dropout:
             feat = F.dropout(feat, p=0.5)  # functional default training=True, exactly as reference :122
         return feat.view(-1, frameLen, self.inputDim)
 

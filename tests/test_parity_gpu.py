@@ -677,19 +677,38 @@ def test_config2_batch_independence_and_determinism(frontend, encoder6, dev):
     assert rel_fro(out[16:], part) < 1e-6
 
 
+_CACHES = ("_packed", "_flat_ws", "_streams", "_lut", "_len_cache")
+
+
+def _settings(*mods):
+    """Every attribute of the modules but their caches (the dicts of parameters, submodules, hooks copied one level)."""
+    return [{k: dict(v) if isinstance(v, dict) else v for k, v in m.__dict__.items() if k not in _CACHES} for m in mods]
+
+
+def _eager_launches(fe, enc, x, lens):
+    """libsblk launches of one eager enc(fe(x))."""
+    from sbl_for_multilingual_lip_reading_b200 import ops
+    before = ops.launch_count()
+    with torch.no_grad():
+        enc(fe(x), lens)
+    torch.cuda.synchronize()
+    return ops.launch_count() - before
+
+
 @pytest.mark.parametrize("n,t,lens", [(32, 29, None), (8, 40, None), (6, 29, [29, 11, 29, 3, 20, 29])])
-def test_pipelined_plan_is_bit_identical_to_eager_modules(frontend, encoder6, dev, n, t, lens):
+def test_pipelined_plan_is_bit_identical_and_leaves_modules_unchanged(frontend, encoder6, dev, n, t, lens):
     """runner.PipelinedVisualEncoderPlan (the encoder stack of batch i-1 co-running with the clip prep + stem of batch i
     on the SMs it leaves free, ordered by the sblk_gate_wait kernel) must return, one step late, exactly what the
     drop-in modules return for each batch: same kernels, only grid sizes and scheduling differ.  Shapes: BASELINE
     configs[1], the configs[2] per-GPU shard (8 clips x 40 frames), a ragged-length batch.  Also through submit_host
-    (pinned host in / out) and drain()."""
+    (pinned host in / out) and drain(); building, replaying and draining the plan leaves the modules as they were."""
     from sbl_for_multilingual_lip_reading_b200 import synth
     from sbl_for_multilingual_lip_reading_b200.runner import PipelinedVisualEncoderPlan
     lens = [t] * n if lens is None else lens
     xs = [synth.synthetic_clips(n, t, seed=50 + i) for i in range(4)]
     with torch.no_grad():
         want = [encoder6(frontend(x.to(dev)), lens)[0].cpu() for x in xs]
+    settings, launches = _settings(frontend, encoder6), _eager_launches(frontend, encoder6, xs[0].to(dev), lens)
     plan = PipelinedVisualEncoderPlan(frontend, encoder6, n, t, device=dev, lengths=lens)
     try:
         # device-resident inputs
@@ -721,21 +740,23 @@ def test_pipelined_plan_is_bit_identical_to_eager_modules(frontend, encoder6, de
             assert torch.equal(hout[i + 1], want[i]), f"host path, batch {i}"
     finally:
         plan.close()
-    # the modules are left as they were
-    assert encoder6.stack_cluster_size == 0 and encoder6._resident_counter is None and frontend._overlap is None
+    assert _settings(frontend, encoder6) == settings
+    assert _eager_launches(frontend, encoder6, xs[0].to(dev), lens) == launches
 
 
 @pytest.mark.parametrize("n,t,lens", [(32, 29, None), (8, 40, None), (5, 29, [29, 11, 29, 3, 20])])
-def test_plain_plan_with_fused_tail_is_bit_identical_to_eager_modules(frontend, encoder6, dev, n, t, lens):
+def test_plain_plan_with_fused_tail_is_bit_identical_and_leaves_modules_unchanged(frontend, encoder6, dev, n, t, lens):
     """runner.VisualEncoderPlan (one batch per replay) with its fused tail — dropout factor drawn on a side stream, the
     pooling launch writes the encoder's 16-bit operand — returns exactly what the drop-in modules return, through
-    forward_device and through submit_host, and leaves the modules' hooks untouched."""
+    forward_device and through submit_host, and leaves the modules as they were: the same settings, the same eager
+    launches (no hint for the encoder's weights added to the frontend's forward)."""
     from sbl_for_multilingual_lip_reading_b200 import synth
     from sbl_for_multilingual_lip_reading_b200.runner import VisualEncoderPlan
     lens = [t] * n if lens is None else lens
     xs = [synth.synthetic_clips(n, t, seed=70 + i) for i in range(3)]
     with torch.no_grad():
         want = [encoder6(frontend(x.to(dev)), lens)[0].cpu() for x in xs]
+    settings, launches = _settings(frontend, encoder6), _eager_launches(frontend, encoder6, xs[0].to(dev), lens)
     plan = VisualEncoderPlan(frontend, encoder6, n, t, device=dev, lengths=lens)
     try:
         assert hasattr(plan, "feat16")          # the fused tail is in use for these shapes
@@ -754,7 +775,25 @@ def test_plain_plan_with_fused_tail_is_bit_identical_to_eager_modules(frontend, 
             assert torch.equal(hout[i], want[i]), f"host path, batch {i}"
     finally:
         plan.close()
-    assert frontend._tail is None and encoder6._x16_override is None
+    assert _settings(frontend, encoder6) == settings
+    assert _eager_launches(frontend, encoder6, xs[0].to(dev), lens) == launches
+
+
+def test_modules_pickled_by_an_earlier_version_run(frontend, encoder6, dev):
+    """Modules pickled before the plans passed their schedule as arguments carry the retired attributes (the plans'
+    hooks, the multi-chain frontend's settings): they load without them and compute what the current modules compute."""
+    from sbl_for_multilingual_lip_reading_b200 import synth
+    from sbl_for_multilingual_lip_reading_b200.encoder import Encoder
+    from sbl_for_multilingual_lip_reading_b200.video_frontend import Lipreading
+    fe, enc = Lipreading.__new__(Lipreading), Encoder.__new__(Encoder)
+    fe.__setstate__(dict(frontend.__getstate__(), parallel_chains=2, chain_sm_limit=74, l2_prefetch_extra=None,
+                         _overlap=None, _tail=None, _block_hook=None))
+    enc.__setstate__(dict(encoder6.__getstate__(), _x16_override=None, _resident_counter=None))
+    x = synth.synthetic_clips(16, 29, seed=11).to(dev)
+    with torch.no_grad():
+        want, = encoder6(frontend(x), [29] * 16)
+        got, = enc(fe(x), [29] * 16)
+    assert torch.equal(got, want)
 
 
 def test_plain_plan_draws_a_fresh_dropout_mask_every_replay(encoder6, dev):

@@ -51,7 +51,7 @@ for pf in (True, False):
                     a = ops.conv3x3_flat(y, w2, b2, relu=True, residual=a)
                 elif ds is not None and w2.dim() == 2:
                     y, res = ops.conv2d_dual(a, w1, b1, ds[0], ds[1], stride=stride, relu=True,
-                                             flat_ws=fe._flat_workspace(a, w1.shape[0], stride, 0))
+                                             flat_ws=fe._flat_workspace(a, w1.shape[0], stride))
                     a = ops.conv3x3_flat(y, w2, b2, relu=True, residual=res)
                 elif ds is not None:
                     y = ops.conv2d(a, w1, b1, stride=stride, relu=True)

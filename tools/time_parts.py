@@ -43,10 +43,7 @@ def graph_time(fn, reps=30):
 with torch.no_grad():
     feat = fe(x)
 fe.l2_prefetch = False
-for ch, lim in ((1, 0),) + (((2, 0), (2, 74), (4, 0)) if os.environ.get("FE_SWEEP") else ()):
-    fe.parallel_chains, fe.chain_sm_limit = ch, lim
-    print(f"frontend (prep+stem+trunk+pool+dropout), {ch} chains, SM limit {lim}: {graph_time(lambda: fe(x)):.1f} us")
-fe.parallel_chains, fe.chain_sm_limit = int(os.environ.get("FE_CHAINS", 1)), int(os.environ.get("FE_LIMIT", 0))
+print(f"frontend (prep+stem+trunk+pool+dropout): {graph_time(lambda: fe(x)):.1f} us")
 for cl, mc in (("16", "1"), ("8", "1")):
     os.environ["SBLK_ENC_STACK_CL"], os.environ["SBLK_ENC_STACK_MC"] = cl, mc
     enc.fused_stack = True
@@ -57,7 +54,6 @@ for sc in (False, True, False, True):
     print(f"encoder  (6 layers), one launch, split clusters {sc}: {graph_time(lambda: enc(feat, [T] * N)):.1f} us")
 for pf in (False, True, False, True, False, True):
     fe.l2_prefetch = pf
-    fe.l2_prefetch_extra = [enc._get_packed().stacked[k] for k in ("w_in", "w_heads", "w_fc", "w_1", "w_2")] if pf else None
     print(f"whole path (one-launch encoder), L2 weight prefetch {pf}: {graph_time(lambda: enc(fe(x), [T] * N)):.1f} us")
 enc.fused_stack = False
 for pc in [int(v) for v in os.environ.get("CHAINS", "4").split(",")]:
