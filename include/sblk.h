@@ -372,11 +372,13 @@ int sblk_attention_train_bwd(const void* qkv, const float* drop, const float* pr
 int sblk_xattention_fwd(const void* q, const void* k, const void* v, void* out, const int* klens, int ldq, int ldk,
                         int ldv, int ldo, int N, int Lq, int Lk, int H, int causal, float scale, void* stream);
 /* x[n*L + l, :] = emb[tokens[n*ld_tokens + l], :] * scale + pe[l, :] (tokens int64, rows = N*L): fp32 [rows, D] and
- * (optional) enc16.  replaces: tgt_word_emb(ys) * x_logit_scale + positional_encoding(ys), decoder.py:323-327 */
+ * (optional) enc16.  Token ids outside [0, vocab) are clamped to 0 / vocab - 1 (no error is reported).
+ * replaces: tgt_word_emb(ys) * x_logit_scale + positional_encoding(ys), decoder.py:323-327 */
 int sblk_embed_pe_fwd(const void* tokens_i64, int ld_tokens, const float* emb, const float* pe, float* out_f32,
                       void* out_16, int rows, int L, int D, int vocab, float scale, void* stream);
 /* Synchronous bidirectional mixing of the two directions' hidden states [N, L, D] fp32 (the reference's aliased in-place
- * loops): l2r' = l2r + flip_L(r2l); r2l' = r2l + flip_L(l2r') = 2 r2l + flip_L(l2r).  Writes fp32 + enc16 copies.
+ * loops): l2r' = l2r + flip_L(r2l); r2l' = r2l + flip_L(l2r') = 2 r2l + flip_L(l2r).  Writes fp32 + enc16 copies
+ * (fp32 pointers 16-byte aligned, enc16 pointers 8-byte aligned; outputs must not alias inputs).
  * replaces: decoder.py:336-346,358-362 */
 int sblk_bidir_mix_fwd(const float* l2r, const float* r2l, float* l2r_out, float* r2l_out, void* l2r_16, void* r2l_16,
                        int N, int L, int D, void* stream);

@@ -115,23 +115,27 @@ def attn_pad_mask(n, t, input_lengths, expand_length):
     return pad.unsqueeze(1).expand(-1, expand_length, -1)
 
 
-def multi_head_attention(x, sd, prefix, n_head, d_k, d_v, mask):
-    """MultiHeadAttention.forward (q = k = v = x), attention.py:32-60, with
-    ScaledDotProductAttention.forward, attention.py:72-83 (temperature = d_k ** 0.5, attention.py:23)."""
-    sz_b, length, _ = x.shape
+def multi_head_attention(x, sd, prefix, n_head, d_k, d_v, mask, kv=None):
+    """MultiHeadAttention.forward, attention.py:32-60, with ScaledDotProductAttention.forward, attention.py:72-83
+    (temperature = d_k ** 0.5, attention.py:23).  Queries and the residual come from x; keys and values from kv
+    (default x: self-attention; the decoder's enc_attn passes the encoder outputs).  mask: bool [N, len_q, len_k],
+    True = masked, or None."""
+    kv = x if kv is None else kv
+    sz_b, len_q, _ = x.shape
+    len_k = kv.shape[1]
     residual = x
-    q = F.linear(x, sd[prefix + ".w_qs.weight"], sd[prefix + ".w_qs.bias"]).view(sz_b, length, n_head, d_k)
-    k = F.linear(x, sd[prefix + ".w_ks.weight"], sd[prefix + ".w_ks.bias"]).view(sz_b, length, n_head, d_k)
-    v = F.linear(x, sd[prefix + ".w_vs.weight"], sd[prefix + ".w_vs.bias"]).view(sz_b, length, n_head, d_v)
-    q = q.permute(2, 0, 1, 3).contiguous().view(-1, length, d_k)  # (n_head*b) x T x d_k, index h*b + i
-    k = k.permute(2, 0, 1, 3).contiguous().view(-1, length, d_k)
-    v = v.permute(2, 0, 1, 3).contiguous().view(-1, length, d_v)
+    q = F.linear(x, sd[prefix + ".w_qs.weight"], sd[prefix + ".w_qs.bias"]).view(sz_b, len_q, n_head, d_k)
+    k = F.linear(kv, sd[prefix + ".w_ks.weight"], sd[prefix + ".w_ks.bias"]).view(sz_b, len_k, n_head, d_k)
+    v = F.linear(kv, sd[prefix + ".w_vs.weight"], sd[prefix + ".w_vs.bias"]).view(sz_b, len_k, n_head, d_v)
+    q = q.permute(2, 0, 1, 3).contiguous().view(-1, len_q, d_k)  # (n_head*b) x T x d_k, index h*b + i
+    k = k.permute(2, 0, 1, 3).contiguous().view(-1, len_k, d_k)
+    v = v.permute(2, 0, 1, 3).contiguous().view(-1, len_k, d_v)
     attn = torch.bmm(q, k.transpose(1, 2)) / float(d_k ** 0.5)
     if mask is not None:
         attn = attn.masked_fill(mask.repeat(n_head, 1, 1).bool(), float("-inf"))
     attn = torch.softmax(attn, dim=2)
     out = torch.bmm(attn, v)
-    out = out.view(n_head, sz_b, length, d_v).permute(1, 2, 0, 3).contiguous().view(sz_b, length, -1)
+    out = out.view(n_head, sz_b, len_q, d_v).permute(1, 2, 0, 3).contiguous().view(sz_b, len_q, -1)
     out = F.linear(out, sd[prefix + ".fc.weight"], sd[prefix + ".fc.bias"])
     out = F.layer_norm(out + residual, (out.size(-1),), sd[prefix + ".layer_norm.weight"],
                        sd[prefix + ".layer_norm.bias"], LN_EPS)

@@ -1696,6 +1696,9 @@ int sblk_bidir_mix_fwd(const float* l2r, const float* r2l, float* l2r_out, float
   if (N <= 0 || L <= 0 || D <= 0 || D % 4 != 0) return fail(-1, "sblk_bidir_mix_fwd: bad shape");
   if (l2r == l2r_out || r2l == r2l_out || l2r == r2l_out || r2l == l2r_out) return fail(-1, "sblk_bidir_mix_fwd: outputs must not alias inputs");
   if (!aligned16(l2r) || !aligned16(r2l) || !aligned16(l2r_out) || !aligned16(r2l_out)) return fail(-1, "sblk_bidir_mix_fwd: pointers must be 16-byte aligned");
+  // the enc16 copies are stored four elements (one uint2) at a time
+  if ((reinterpret_cast<uintptr_t>(l2r_16) & 7u) || (reinterpret_cast<uintptr_t>(r2l_16) & 7u))
+    return fail(-1, "sblk_bidir_mix_fwd: 16-bit outputs must be 8-byte aligned");
   return launch(sblk::bidir_mix_kernel, dim3(elementwise_grid(static_cast<long long>(N) * L * (D / 4), 256, sms)), dim3(256), 0,
                 static_cast<cudaStream_t>(stream), false, "bidir_mix_kernel", l2r, r2l, l2r_out, r2l_out,
                 static_cast<uint16_t*>(l2r_16), static_cast<uint16_t*>(r2l_16), N, L, D, SBLK_ENC_FP16 ? 1 : 0);

@@ -277,8 +277,9 @@ class Decoder(nn.Module):
         """CUDA graphs of the 16 decode steps for one (batch, encoder length): a step is ~150 short launches, so eager
         decoding is host-bound (38 ms per 16-clip call against ~8 ms of GPU work).  Static buffers: encoder outputs,
         the 12 cached K|V projections, both token buffers [N, 17] and the per-step logits; graph L recomputes the prefix
-        of length L.  All graphs share one memory pool (they never run concurrently)."""
-        key = (n, t_enc, str(dev), pk["key"])
+        of length L.  All graphs share one memory pool (they never run concurrently).  The settings the captured steps
+        depend on (fused_ln, two_streams) are part of the key, so changing one takes effect at the next call."""
+        key = (n, t_enc, str(dev), pk["key"], self.fused_ln, self.two_streams)
         plan = self._plans.get(key)
         if plan is not None:
             return plan
