@@ -112,7 +112,7 @@ long long sblk_flat_rows(int F, int H, int W);
 /* Stride-1 3x3 / pad 1 Conv2d (C -> C, C == 64 or 128) + folded BN (+ residual) (+ ReLU) over the flat layout
  * (flat_out of sblk_conv3d_bn_relu_pool_fwd / sblk_conv2d_dual_igemm_fwd or a previous call); output is again flat
  * with zero halos.  w_packed_bf16 is [C][10*C]: the 9 taps of sblk_pack_conv2d's [C][3][3][C] followed by a CxC
- * identity (used only by the single-CTA C == 64 kernel, which accumulates the residual on the tensor core as R*I).
+ * identity.  Those last C columns are not read; they are kept so that the packed layout does not change.
  * W + 2 <= 31 for C == 64, <= 15 for C == 128.  CTA-pair (cta_group::2) shifted-window implicit GEMM.
  * replaces: the stride-1 convs of ResNet layer1 and layer2, transformer/video_frontend.py:10-12,28-41 */
 int sblk_flatconv3x3_fwd(const void* x_flat, const void* w_packed_bf16, const float* bias, const void* residual_flat,

@@ -17,9 +17,6 @@
 #include "sblk_igemm2_block.cuh"
 #include "sblk_conv3d.cuh"
 #include "sblk_stem_t.cuh"
-#ifdef SBLK_DEBUG
-#include "sblk_flatconv.cuh"   // v1 single-CTA flat conv: A/B timing baseline only (SBLK_FLATCONV2=0)
-#endif
 #include "sblk_flatconv2.cuh"
 #include "sblk_aux.cuh"
 #include "sblk_attention.cuh"
@@ -38,14 +35,6 @@ std::atomic<long long> g_launches{0};
 thread_local int g_pdl = 0;        // != 0: launches carry the programmatic-dependent-launch attribute
 thread_local int g_sm_limit = 0;   // > 0: size persistent grids for at most this many SMs (concurrent kernel chains)
 thread_local int g_stem_variant = 0;   // 0: transposed stem with the filter in tensor memory; 1: pixel-major stem
-
-// Tuning / profiling switches read from the environment exist only in -DSBLK_DEBUG builds (tools/, experiments): the
-// release library never calls getenv and cannot be steered into its timing-experiment modes.
-#ifdef SBLK_DEBUG
-inline const char* dbg_env(const char* name) { return getenv(name); }
-#else
-inline const char* dbg_env(const char*) { return nullptr; }
-#endif
 
 int fail(int code, const char* fmt, ...) {
   va_list ap;
@@ -131,7 +120,6 @@ int ensure_init(int* num_sms_out) {
     if ((rc = set_smem(sblk::igemm_kernel<64, true>, sblk::IgemmCfg<64>::SMEM_BYTES))) return rc;
     if ((rc = set_smem(sblk::igemm_kernel<128, true>, sblk::IgemmCfg<128>::SMEM_BYTES))) return rc;
     if ((rc = set_smem(sblk::igemm_kernel<256, true>, sblk::IgemmCfg<256>::SMEM_BYTES))) return rc;
-    if ((rc = set_smem(sblk::igemm_kernel<128, true, true>, sblk::IgemmCfg<128, true>::SMEM_BYTES))) return rc;
     if ((rc = set_smem(sblk::igemm2_kernel<128, true>, sblk::Igemm2Cfg<128>::SMEM_BYTES))) return rc;
     if ((rc = set_smem(sblk::igemm2_kernel<256, true>, sblk::Igemm2Cfg<256>::SMEM_BYTES))) return rc;
     if ((rc = set_smem(sblk::igemm2_kernel<128, true, true>, sblk::Igemm2Cfg<128, true>::SMEM_BYTES))) return rc;
@@ -143,9 +131,6 @@ int ensure_init(int* num_sms_out) {
     if ((rc = set_smem(sblk::stem_t_kernel<0>, sblk::stt::SMEM_BYTES))) return rc;
     if ((rc = set_smem(sblk::stem_t_kernel<1>, sblk::stt::SMEM_BYTES))) return rc;
     if ((rc = set_smem(sblk::stem_t_kernel<2>, sblk::stt::SMEM_BYTES))) return rc;
-#ifdef SBLK_DEBUG
-    if ((rc = set_smem(sblk::flatconv3x3_c64_kernel, sblk::fc::SMEM_BYTES))) return rc;
-#endif
     if ((rc = set_smem(sblk::flatconv2_kernel<1>, sblk::Fc2Cfg<1>::SMEM_BYTES))) return rc;
     if ((rc = set_smem(sblk::flatconv2_kernel<2>, sblk::Fc2Cfg<2>::SMEM_BYTES))) return rc;
     if ((rc = set_smem(sblk::gemm_ln512_kernel, sblk::gln::SMEM_BYTES))) return rc;
@@ -217,32 +202,22 @@ int pick_block_n(int m_tiles, int N, int num_sms) {
 template <bool IM2COL>
 int launch_igemm(int bn, const CUtensorMap& tmA, const CUtensorMap& tmB, sblk::IgemmParams p, int num_sms,
                  cudaStream_t stream) {
-  {
-    const char* dm = dbg_env("SBLK_IGEMM_DEBUG_MODE");  // timing experiments only (wrong results when != 0)
-    p.debug_mode = dm ? atoi(dm) : 0;
-  }
   const int m_tiles = (p.M + 127) / 128;
   const int tiles = m_tiles * (p.N / bn) * p.splits;
   const int grid = tiles < num_sms ? tiles : num_sms;
   switch (bn) {
     case 64:
       return launch(sblk::igemm_kernel<64, IM2COL>, dim3(grid), dim3(192), sblk::IgemmCfg<64>::SMEM_BYTES, stream,
-                    true, "igemm_kernel<64>", tmA, tmB, tmB, p);
+                    true, "igemm_kernel<64>", tmA, tmB, p);
     case 128:
       return launch(sblk::igemm_kernel<128, IM2COL>, dim3(grid), dim3(192), sblk::IgemmCfg<128>::SMEM_BYTES, stream,
-                    true, "igemm_kernel<128>", tmA, tmB, tmB, p);
+                    true, "igemm_kernel<128>", tmA, tmB, p);
     case 256:
       return launch(sblk::igemm_kernel<256, IM2COL>, dim3(grid), dim3(192), sblk::IgemmCfg<256>::SMEM_BYTES, stream,
-                    true, "igemm_kernel<256>", tmA, tmB, tmB, p);
+                    true, "igemm_kernel<256>", tmA, tmB, p);
     default:
       return fail(-11, "no BLOCK_N for N=%d", p.N);
   }
-}
-
-// SBLK_CTA_PAIRS=0 routes every conv through the 1-CTA kernel (A/B timing experiments); default on.
-bool use_cta_pairs() {
-  const char* e = dbg_env("SBLK_CTA_PAIRS");
-  return e == nullptr || atoi(e) != 0;
 }
 
 int elementwise_grid(long long work_items, int block, int num_sms) {
@@ -343,29 +318,22 @@ int sblk_l2_prefetch(const void* const* ptrs, const long long* bytes, int n, voi
   // throttled hints or demand loads 223 us, warm 221 us), while demand loads running next to the persistent conv kernels
   // slow the whole graph down (818 -> 980 us: their CTAs finish late and the join holds the encoder back).  One hint
   // launch PER RANGE keeps the bursts small (launch gaps let the memory system drain) and costs nothing when a hint
-  // is dropped: whole path 820 -> 808 us.  SBLK_L2_PREFETCH_MODE / _CTAS override for experiments.
-  int cap = 2 * sms, mode = 0;
-  if (const char* e = dbg_env("SBLK_L2_PREFETCH_CTAS")) cap = atoi(e);
-  if (const char* e = dbg_env("SBLK_L2_PREFETCH_MODE")) mode = atoi(e);
-  long long chunk_lines = (64ll << 20) / 128;   // one hint launch per range (<= 64 MB); smaller bursts only add launches (graph: 808 us per tensor, 816 at 4 MB, 871 at 1 MB)
-  if (const char* e = dbg_env("SBLK_L2_PREFETCH_CHUNK_KB")) chunk_lines = (static_cast<long long>(atoi(e)) << 10) / 128;
-  if (chunk_lines < 1) chunk_lines = 1;
+  // is dropped: whole path 820 -> 808 us.
+  const long long cap = 2 * sms;
+  const long long chunk_lines = (64ll << 20) / 128;   // one hint launch per range (<= 64 MB); smaller bursts only add launches (graph: 808 us per tensor, 816 at 4 MB, 871 at 1 MB)
   for (int i = 0; i < n; ++i) {
     if (!ptrs[i] || bytes[i] <= 0) return fail(-1, "sblk_l2_prefetch: null pointer / empty range %d", i);
     const uintptr_t a = reinterpret_cast<uintptr_t>(ptrs[i]);
     const uintptr_t base = a & ~static_cast<uintptr_t>(127);
     const long long lines = (static_cast<long long>(a - base) + bytes[i] + 127) / 128;
     for (long long l0 = 0; l0 < lines; l0 += chunk_lines) {
-      sblk::L2PrefetchRanges r;
-      r.n = 1;
-      r.base[0] = reinterpret_cast<const uint8_t*>(base) + l0 * 128;
-      r.first_line[0] = 0;
-      r.first_line[1] = lines - l0 < chunk_lines ? lines - l0 : chunk_lines;
-      long long grid = (r.first_line[1] + 255) / 256;
+      const long long chunk = lines - l0 < chunk_lines ? lines - l0 : chunk_lines;
+      long long grid = (chunk + 255) / 256;
       if (grid > cap) grid = cap;
       if (grid < 1) grid = 1;
       if ((rc = launch(sblk::l2_prefetch_kernel, dim3(static_cast<unsigned>(grid)), dim3(256), 0,
-                       static_cast<cudaStream_t>(stream), false, "l2_prefetch_kernel", r, mode)))
+                       static_cast<cudaStream_t>(stream), false, "l2_prefetch_kernel",
+                       reinterpret_cast<const uint8_t*>(base) + l0 * 128, chunk)))
         return rc;
     }
   }
@@ -501,12 +469,6 @@ static int launch_stem_t(sblk::StemTParams& q, const void* wp, const float* bias
   q.bias = bias;
   q.out = static_cast<__nv_bfloat16*>(out);
   q.flat_out = flat_out ? 1 : 0;
-  {
-    const char* dm = dbg_env("SBLK_C3D_DEBUG_MODE");  // timing experiments only (wrong results when != 0)
-    q.debug_mode = dm ? atoi(dm) : 0;
-    const char* st = dbg_env("SBLK_C3D_STAMPS");      // device pointer (hex) of a [grid][8] uint64 stamp buffer
-    q.dbg = st ? reinterpret_cast<unsigned long long*>(strtoull(st, nullptr, 16)) : nullptr;
-  }
   // every CTA gets an equal-cost contiguous share of the (frame pair, row pair) steps; at least two tiles per CTA
   long long g = steps / 2 < 1 ? 1 : steps / 2;
   if (g > sms) g = sms;
@@ -580,10 +542,6 @@ int sblk_conv3d_bn_relu_pool_fwd(const void* xp, const void* wp, const float* bi
   p.bias = bias;
   p.out = static_cast<__nv_bfloat16*>(out);
   p.flat_out = flat_out ? 1 : 0;
-  {
-    const char* dm = dbg_env("SBLK_C3D_DEBUG_MODE");  // timing experiments only (wrong results when != 0)
-    p.debug_mode = dm ? atoi(dm) : 0;
-  }
   const int units = p.frames * 2;
   const int grid = units < sms ? units : sms;
   return launch(sblk::conv3d_bn_relu_pool_kernel, dim3(grid), dim3(THREADS), SMEM_BYTES,
@@ -630,32 +588,6 @@ static int launch_flatconv2(const void* x, const void* wp, const float* bias, co
   p.bias = bias;
   p.reverse = reverse ? 1 : 0;
   const int pairs = p.num_tiles < sms / 2 ? p.num_tiles : sms / 2;
-  p.dbg = nullptr;
-  {
-    const char* dm = dbg_env("SBLK_FLAT_DEBUG_MODE");  // timing experiments only (wrong results when != 0)
-    p.debug_mode = dm ? atoi(dm) : 0;
-  }
-  if (dbg_env("SBLK_FLAT_STAMPS")) {   // profiling aid: per-tile clock stamps of CTA 0, printed after a synchronise
-    static unsigned long long* d_dbg = nullptr;
-    const int tiles0 = (p.num_tiles + pairs - 1) / pairs;
-    if (!d_dbg) cudaMalloc(&d_dbg, 4096 * 16 * 8);
-    cudaMemsetAsync(d_dbg, 0, 4096 * 16 * 8, stream);
-    p.dbg = d_dbg;
-    int rc2 = launch(sblk::flatconv2_kernel<CB>, dim3(2 * pairs), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, stream, true,
-                     "flatconv2_kernel", tmX, tmW, tmR, tmO, p);
-    cudaStreamSynchronize(stream);
-    static unsigned long long h[4096 * 16];
-    cudaMemcpy(h, d_dbg, sizeof(h), cudaMemcpyDeviceToHost);
-    const unsigned long long t0 = h[0];
-    fprintf(stderr, "[flatconv2<%d> stamps, CTA 0, cycles since first] tile: mma(wait_a wait_acc issue_done) "
-            "epi(top bar tfull res released bar2 stored)\n", CB);
-    for (int t = 0; t < tiles0 && t < 40; ++t) {
-      fprintf(stderr, "%3d:", t);
-      for (int k = 0; k < 11; ++k) fprintf(stderr, " %7lld", h[t * 16 + k] ? (long long)(h[t * 16 + k] - t0) : -1LL);
-      fprintf(stderr, "\n");
-    }
-    return rc2;
-  }
   return launch(sblk::flatconv2_kernel<CB>, dim3(2 * pairs), dim3(Cfg::THREADS), Cfg::SMEM_BYTES, stream, true,
                 "flatconv2_kernel", tmX, tmW, tmR, tmO, p);
 }
@@ -668,9 +600,6 @@ int sblk_flatconv3x3_fwd(const void* x, const void* wp, const float* bias, const
 
 int sblk_flatconv3x3_dir_fwd(const void* x, const void* wp, const float* bias, const void* residual, void* out, int F,
                              int H, int W, int C, int relu, int reverse, void* stream) {
-#ifdef SBLK_DEBUG
-  using namespace sblk::fc;
-#endif
   int sms, rc;
   if ((rc = ensure_init(&sms))) return rc;
   if (!x || !wp || !bias || !out) return fail(-1, "sblk_flatconv3x3_fwd: null pointer");
@@ -683,44 +612,7 @@ int sblk_flatconv3x3_dir_fwd(const void* x, const void* wp, const float* bias, c
   const long long rows = sblk_flat_rows(F, H, W);
   if (rows > 0x7fffffffLL - 1024) return fail(-1, "sblk_flatconv3x3_fwd: problem too large");
   if (C == 128) return launch_flatconv2<2>(x, wp, bias, residual, out, rows, H, W, relu, sms, static_cast<cudaStream_t>(stream), reverse);
-#ifndef SBLK_DEBUG
   return launch_flatconv2<1>(x, wp, bias, residual, out, rows, H, W, relu, sms, static_cast<cudaStream_t>(stream), reverse);
-#else
-  const char* v2 = dbg_env("SBLK_FLATCONV2");   // 0 = v1 single-CTA kernel for C == 64 (A/B timing experiments)
-  if (v2 == nullptr || atoi(v2) != 0)
-    return launch_flatconv2<1>(x, wp, bias, residual, out, rows, H, W, relu, sms, static_cast<cudaStream_t>(stream), reverse);
-  CUtensorMap tmX, tmW, tmR;
-  {
-    cuuint64_t dims[2] = {static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(rows)};
-    cuuint64_t strides[1] = {static_cast<cuuint64_t>(C) * 2};
-    cuuint32_t box[2] = {64, BOX_PIX};
-    if ((rc = encode_tiled(&tmX, x, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-    cuuint32_t rbox[2] = {64, TILE_M};
-    if ((rc = encode_tiled(&tmR, residual ? residual : x, 2, dims, strides, rbox, CU_TENSOR_MAP_SWIZZLE_128B)))
-      return rc;
-  }
-  {
-    // packed filter [64][10*64]: taps (r,s) at K columns (3r+s)*64.., a 64x64 identity at columns 576..639
-    cuuint64_t dims[2] = {static_cast<cuuint64_t>(W_TAPS * C), static_cast<cuuint64_t>(C)};
-    cuuint64_t strides[1] = {static_cast<cuuint64_t>(W_TAPS * C) * 2};
-    cuuint32_t box[2] = {64, 64};
-    if ((rc = encode_tiled(&tmW, wp, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
-  }
-  sblk::FlatConvParams p;
-  p.m_total = static_cast<int>(rows);
-  p.num_tiles = (p.m_total + TILE_M - 1) / TILE_M;
-  p.H = H; p.W = W; p.relu = relu;
-  p.bias = bias;
-  p.has_res = residual ? 1 : 0;
-  p.out = static_cast<__nv_bfloat16*>(out);
-  {
-    const char* dm = dbg_env("SBLK_FLAT_DEBUG_MODE");  // timing experiments only (wrong results when != 0)
-    p.debug_mode = dm ? atoi(dm) : 0;
-  }
-  const int grid = p.num_tiles < sms ? p.num_tiles : sms;
-  return launch(sblk::flatconv3x3_c64_kernel, dim3(grid), dim3(THREADS), SMEM_BYTES,
-                static_cast<cudaStream_t>(stream), true, "flatconv3x3_c64_kernel", tmX, tmW, tmR, p);
-#endif
 }
 
 // K-extension of a conv (sblk_conv2d_igemm_ext_fwd): a 1x1 / pad 0 / stride `stride` conv of a second tensor x2
@@ -920,7 +812,7 @@ static int conv2d_igemm_impl(const void* x, const void* wp, const float* bias, c
     if ((ext->H2 - 1) / ext->stride + 1 != P || (ext->W2 - 1) / ext->stride + 1 != Q)
       return fail(-1, "sblk_conv2d_igemm_ext_fwd: the extension's output grid %dx%d does not match the conv's %dx%d",
                   (ext->H2 - 1) / ext->stride + 1, (ext->W2 - 1) / ext->stride + 1, P, Q);
-    if (!(use_cta_pairs() && Cout % 128 == 0))
+    if (Cout % 128 != 0)
       return fail(-1, "sblk_conv2d_igemm_ext_fwd: needs the CTA-pair kernel (Cout %% 128 == 0)");
     if ((rc = encode_im2col(&tmA2, ext->x2, ext->Cin2, ext->W2, ext->H2, ext->row_pitch, ext->frame_pitch, 1, 1, 0,
                             ext->stride)))
@@ -931,7 +823,7 @@ static int conv2d_igemm_impl(const void* x, const void* wp, const float* bias, c
     cuuint64_t strides[1] = {static_cast<cuuint64_t>(Ktot) * 2};
     const int m_tiles = (M + 127) / 128;
     // CTA-pair kernel (sblk_igemm2.cuh) for every conv with Cout >= 128: half the B bytes per SM
-    int bn2 = use_cta_pairs() && Cout % 128 == 0 ? ((wp_ds || Cout % 256 != 0) ? 128 : 256) : 0;
+    int bn2 = Cout % 128 == 0 ? ((wp_ds || Cout % 256 != 0) ? 128 : 256) : 0;
     if (bn2 == 256) {
       // small problems (the 8-clip shard of BASELINE configs[2]: 24 pair tiles of 256 x 256 at layer 4 on 74 CTA pairs):
       // 256 x 128 tiles when they still run as one wave — twice the CTAs, half the k-loop time each.  A tile's time is
@@ -943,37 +835,14 @@ static int conv2d_igemm_impl(const void* x, const void* wp, const float* bias, c
       const long long time128 = (2 * t256 + pairs_avail - 1) / pairs_avail;
       if (time128 < time256) bn2 = 128;
     }
-    const int bn = bn2 ? bn2 : wp_ds ? 128 : pick_block_n(m_tiles, Cout, sms);
+    const int bn = bn2 ? bn2 : pick_block_n(m_tiles, Cout, sms);
     if (flat_out && !bn2) return fail(-1, "sblk_conv2d_dual_igemm_fwd: flat_out needs the CTA-pair kernel (Cout %% 128 == 0)");
     cuuint32_t box[2] = {64, static_cast<cuuint32_t>(bn2 ? bn2 / 2 : bn)};
     if ((rc = encode_tiled(&tmB, wp, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
     sblk::IgemmParams p;
-    p.splits = 1; p.split_stride = 0; p.flat_out = flat_out; p.dbg = nullptr; p.staged = 0; p.fp16 = 0;
+    p.splits = 1; p.split_stride = 0; p.flat_out = flat_out; p.fp16 = 0;
     p.bias2 = bias_ds;
     p.out2_bf16 = static_cast<__nv_bfloat16*>(out_ds);
-    p.debug_mode = 0;
-    // profiling aid (SBLK_IGEMM2_STAMPS=1): run the CTA-pair launch with clock stamps of CTA 0 and print them
-    auto with_stamps = [&](auto&& do_launch, int tiles2, int pairs) -> int {
-      if (!dbg_env("SBLK_IGEMM2_STAMPS")) return do_launch();
-      static unsigned long long* d_dbg = nullptr;
-      if (!d_dbg) cudaMalloc(&d_dbg, 64 * 8);
-      cudaMemsetAsync(d_dbg, 0, 64 * 8, static_cast<cudaStream_t>(stream));
-      p.dbg = d_dbg;
-      const int rc2 = do_launch();
-      cudaStreamSynchronize(static_cast<cudaStream_t>(stream));
-      unsigned long long h[64];
-      cudaMemcpy(h, d_dbg, sizeof(h), cudaMemcpyDeviceToHost);
-      auto rel = [&](int i) { return h[i] ? static_cast<long long>(h[i] - h[0]) : -1LL; };
-      const int nkb = R * S * (Cin / 64);
-      fprintf(stderr, "[igemm2 stamps CTA0, cycles since entry; Cout %d, %d pair tiles on %d pairs, %d k-blocks, staged %d] "
-              "first tile: mma issued %lld, acc ready %lld, epilogue done %lld | last tile: mma issued %lld, acc ready "
-              "%lld, epilogue done %lld | kernel end %lld | k-block arrival every 8:", Cout, tiles2, pairs, nkb, p.staged,
-              rel(1), rel(3), rel(4), rel(2), rel(5), rel(6), rel(7));
-      for (int i = 8; i < 8 + (nkb + 7) / 8 && i < 64; ++i) fprintf(stderr, " %lld", rel(i));
-      fprintf(stderr, "\n");
-      p.dbg = nullptr;
-      return rc2;
-    };
     if (wp_ds) {
       // fused 1x1 downsample branch: its [Cout][Cin] filter rides along with the centre-tap k-blocks
       cuuint64_t dims2[2] = {static_cast<cuuint64_t>(Cin), static_cast<cuuint64_t>(Cout)};
@@ -983,22 +852,11 @@ static int conv2d_igemm_impl(const void* x, const void* wp, const float* bias, c
       p.stride = stride; p.pad = pad; p.relu = relu; p.ldo = Cout;
       p.bias = bias; p.residual = nullptr;
       p.out_bf16 = static_cast<__nv_bfloat16*>(out); p.out_f32 = nullptr;
-      if (bn2) {
-        const int tiles2 = ((M + 255) / 256) * (Cout / 128);
-        const int pairs = tiles2 < sms / 2 ? tiles2 : sms / 2;
-        // staged coalesced epilogue stores (they take the place of the last ring stage); measured in the whole graph:
-        // frontend 607 us (always staged) vs 644 us (never); SBLK_IGEMM2_STAGED=0/1 overrides for A/B timing
-        p.staged = 1;
-        if (const char* e = dbg_env("SBLK_IGEMM2_STAGED")) p.staged = atoi(e) != 0;
-        return with_stamps([&]() {
-          return launch(sblk::igemm2_kernel<128, true, true>, dim3(2 * pairs), dim3(sblk::Igemm2Cfg<128, true>::THREADS),
-                        sblk::Igemm2Cfg<128, true>::SMEM_BYTES, static_cast<cudaStream_t>(stream), true,
-                        "igemm2_kernel<128,dual>", tmA, tmB, tmB2, tmA2, p); }, tiles2, pairs);
-      }
-      const int tiles = m_tiles * (Cout / 128);
-      const int grid = tiles < sms ? tiles : sms;
-      return launch(sblk::igemm_kernel<128, true, true>, dim3(grid), dim3(192), sblk::IgemmCfg<128, true>::SMEM_BYTES,
-                    static_cast<cudaStream_t>(stream), true, "igemm_kernel<128,dual>", tmA, tmB, tmB2, p);
+      const int tiles2 = ((M + 255) / 256) * (Cout / 128);
+      const int pairs = tiles2 < sms / 2 ? tiles2 : sms / 2;
+      return launch(sblk::igemm2_kernel<128, true, true>, dim3(2 * pairs), dim3(sblk::Igemm2Cfg<128, true>::THREADS),
+                    sblk::Igemm2Cfg<128, true>::SMEM_BYTES, static_cast<cudaStream_t>(stream), true,
+                    "igemm2_kernel<128,dual>", tmA, tmB, tmB2, tmA2, p);
     }
     p.M = M; p.N = Cout; p.taps_r = R; p.taps_s = S; p.cblocks = Cin / 64; p.P = P; p.Q = Q;
     p.stride = stride; p.pad = pad; p.relu = relu; p.ldo = Cout;
@@ -1018,13 +876,10 @@ static int conv2d_igemm_impl(const void* x, const void* wp, const float* bias, c
     if (bn2) {
       const int tiles2 = ((M + 255) / 256) * (Cout / bn2);
       const int pairs = tiles2 < sms / 2 ? tiles2 : sms / 2;
-      p.staged = 1;
-      if (const char* e = dbg_env("SBLK_IGEMM2_STAGED")) p.staged = atoi(e) != 0;
       if (bn2 == 256) {
-        return with_stamps([&]() {
-          return launch(sblk::igemm2_kernel<256, true>, dim3(2 * pairs), dim3(sblk::Igemm2Cfg<256>::THREADS),
-                        sblk::Igemm2Cfg<256>::SMEM_BYTES, static_cast<cudaStream_t>(stream), true, "igemm2_kernel<256>",
-                        tmA, tmB, tmB2, tmA2, p); }, tiles2, pairs);
+        return launch(sblk::igemm2_kernel<256, true>, dim3(2 * pairs), dim3(sblk::Igemm2Cfg<256>::THREADS),
+                      sblk::Igemm2Cfg<256>::SMEM_BYTES, static_cast<cudaStream_t>(stream), true, "igemm2_kernel<256>",
+                      tmA, tmB, tmB2, tmA2, p);
       }
       return launch(sblk::igemm2_kernel<128, true>, dim3(2 * pairs), dim3(sblk::Igemm2Cfg<128>::THREADS), sblk::Igemm2Cfg<128>::SMEM_BYTES,
                     static_cast<cudaStream_t>(stream), true, "igemm2_kernel<128>", tmA, tmB, tmB2, tmA2, p);
@@ -1072,11 +927,7 @@ static int gemm_impl(const void* a, const void* w, const float* bias, const void
     if ((rc = encode_tiled(&tmA, a, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
   }
   const int m_tiles = (M + 127) / 128;
-  int bn = pick_block_n_linear(m_tiles, N, splits, sms);
-  {
-    const char* e = dbg_env("SBLK_GEMM_BN");   // tuning experiments only
-    if (e && atoi(e) > 0 && N % atoi(e) == 0) bn = atoi(e);
-  }
+  const int bn = pick_block_n_linear(m_tiles, N, splits, sms);
   {
     cuuint64_t dims[2] = {static_cast<cuuint64_t>(K), static_cast<cuuint64_t>(N)};
     cuuint64_t strides[1] = {static_cast<cuuint64_t>(K) * 2};
@@ -1084,14 +935,14 @@ static int gemm_impl(const void* a, const void* w, const float* bias, const void
     if ((rc = encode_tiled(&tmB, w, 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B))) return rc;
   }
   sblk::IgemmParams p;
-  p.bias2 = nullptr; p.out2_bf16 = nullptr; p.debug_mode = 0;
+  p.bias2 = nullptr; p.out2_bf16 = nullptr;
   p.M = M; p.N = N; p.taps_r = 1; p.taps_s = 1; p.cblocks = K / 64; p.P = 1; p.Q = 1;
   p.stride = 1; p.pad = 0; p.relu = relu; p.ldo = N;
   p.bias = bias;
   p.residual = static_cast<const __nv_bfloat16*>(residual);
   p.out_bf16 = static_cast<__nv_bfloat16*>(out_bf16);
   p.out_f32 = out_f32;
-  p.splits = splits; p.flat_out = 0; p.dbg = nullptr; p.staged = 0; p.fp16 = fp16;
+  p.splits = splits; p.flat_out = 0; p.fp16 = fp16;
   p.split_stride = static_cast<long long>(M) * N;
   return launch_igemm<false>(bn, tmA, tmB, p, sms, static_cast<cudaStream_t>(stream));
 }
@@ -1319,12 +1170,6 @@ static int launch_encoder_stack(const CUtensorMap* tm, const sblk::EncStackParam
   }
   cfg.attrs = attr;
   cfg.numAttrs = nattr;
-  if (dbg_env("SBLK_ENC_STACK_VERBOSE")) {
-    int ncl = -1;
-    cudaError_t oe = cudaOccupancyMaxActiveClusters(&ncl, kernel, &cfg);
-    fprintf(stderr, "[libsblk] encoder_stack CL=%d: max active clusters %d (%s), grid %d CTAs\n", CL, ncl,
-            cudaGetErrorName(oe), groups * CL);
-  }
   cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], tm[6], tm[7], tm[8], p);
   if (e != cudaSuccess) return cuda_fail(e, "encoder_stack_kernel");
   g_launches.fetch_add(1, std::memory_order_relaxed);

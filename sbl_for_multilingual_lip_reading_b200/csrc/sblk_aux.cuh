@@ -196,40 +196,16 @@ cast_f32_bf16_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ 
   }
 }
 
-// L2 prefetch of read-only ranges (packed weights of the layers that run later in the same forward): every 32-byte
-// sector is touched by a demand load (mode 2; prefetch.global.L2 hints, modes 0 / 1, are dropped when issued in large
-// bursts), no shared memory and few registers, so the few CTAs co-reside with the persistent conv kernels.  The bench flushes L2 between steps, so without it every kernel's first weight tiles (and the
-// whole dependent chain of the encoder stack) pay DRAM latency.
-struct L2PrefetchRanges {
-  static constexpr int MAX = 24;
-  const uint8_t* base[MAX];     // 128-byte aligned
-  long long first_line[MAX + 1];   // exclusive prefix sum of the ranges' line counts
-  int n;
-};
+// L2 prefetch of one read-only range (packed weights of the layers that run later in the same forward):
+// prefetch.global.L2 of every 128-byte line, no shared memory and few registers, so the few CTAs co-reside with the
+// persistent conv kernels.  The bench flushes L2 between steps, so without it every kernel's first weight tiles (and
+// the whole dependent chain of the encoder stack) pay DRAM latency.
 __global__ void __launch_bounds__(256)
-l2_prefetch_kernel(const L2PrefetchRanges r, int mode) {
-  const long long total = r.first_line[r.n];
-  unsigned int sink = 0;
-  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
-       i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    int k = 0;
-    while (k + 1 < r.n && i >= r.first_line[k + 1]) ++k;
-    const uint8_t* a = r.base[k] + (i - r.first_line[k]) * 128;
-    if (mode == 0) {
-      asm volatile("prefetch.global.L2 [%0];" ::"l"(a));
-    } else if (mode == 1) {
-      asm volatile("prefetch.global.L2::evict_last [%0];" ::"l"(a));
-    } else {
-      // demand loads of every 32-byte sector (cannot be dropped like a hint)
-      unsigned int v0, v1, v2, v3;
-      asm volatile("ld.global.cg.u32 %0, [%1];" : "=r"(v0) : "l"(a));
-      asm volatile("ld.global.cg.u32 %0, [%1];" : "=r"(v1) : "l"(a + 32));
-      asm volatile("ld.global.cg.u32 %0, [%1];" : "=r"(v2) : "l"(a + 64));
-      asm volatile("ld.global.cg.u32 %0, [%1];" : "=r"(v3) : "l"(a + 96));
-      sink += v0 ^ v1 ^ v2 ^ v3;
-    }
-  }
-  if (sink == 0x9e3779b9u && total < 0) asm volatile("trap;");   // keeps the loads alive; never true
+l2_prefetch_kernel(const uint8_t* base, long long lines) {   // base 128-byte aligned
+#pragma unroll 1
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < lines;
+       i += static_cast<long long>(gridDim.x) * blockDim.x)
+    asm volatile("prefetch.global.L2 [%0];" ::"l"(base + i * 128));
 }
 
 // --------------------------------------------------------------------------------------------

@@ -83,9 +83,8 @@ struct Conv3dParams {
   int T;                      // frames per clip
   const uint4* x8;            // row-Toeplitz clip [N][T+4][2][47][44] entries of 8 bf16
   const float* bias;          // [64] folded BN shift
-  __nv_bfloat16* out;         // [F,22,22,64], or the zero-haloed flat layout of sblk_flatconv.cuh when flat_out
+  __nv_bfloat16* out;         // [F,22,22,64], or the zero-haloed flat layout of sblk_flatconv2.cuh when flat_out
   int flat_out;               // 1: pixel (f,y,x) -> row (f*23 + 1 + y)*24 + 1 + x, halo rows/columns written as zeros
-  int debug_mode;             // 0 = normal; timing experiments only: 1 = no MMAs, 2 = no loads
 };
 
 __global__ void __launch_bounds__(c3d::THREADS, 1)
@@ -157,13 +156,9 @@ conv3d_bn_relu_pool_kernel(const __grid_constant__ CUtensorMap tmW, const Conv3d
           uint8_t* dst = smem + OFF_A + stage * A_STAGE_BYTES;
           const uint4* src = p.x8 + static_cast<size_t>(n * TP + t + dt) * FRAME_ENTRIES + m0;
           if (elect_one()) {
-            if (p.debug_mode == 2) {
-              mbar_arrive(&full_bar[stage]);
-            } else {
-              mbar_arrive_expect_tx(&full_bar[stage], A_STAGE_BYTES);
-              bulk_load(dst, src, STAGE_PLANE_BYTES, &full_bar[stage]);
-              bulk_load(dst + STAGE_PLANE_BYTES, src + PLANE_ENTRIES, STAGE_PLANE_BYTES, &full_bar[stage]);
-            }
+            mbar_arrive_expect_tx(&full_bar[stage], A_STAGE_BYTES);
+            bulk_load(dst, src, STAGE_PLANE_BYTES, &full_bar[stage]);
+            bulk_load(dst + STAGE_PLANE_BYTES, src + PLANE_ENTRIES, STAGE_PLANE_BYTES, &full_bar[stage]);
           }
           __syncwarp();
           if (++stage == A_STAGES) { stage = 0; phase ^= 1u; }
@@ -194,7 +189,6 @@ conv3d_bn_relu_pool_kernel(const __grid_constant__ CUtensorMap tmW, const Conv3d
           if (elect_one()) {
 #pragma unroll
             for (int j = 0; j < TILES_PER_GROUP; ++j) {
-              if (p.debug_mode == 1) break;
               const uint32_t d_tmem = tmem_base + static_cast<uint32_t>((set * TILES_PER_GROUP + j) * COUT);
 #pragma unroll
               for (int q = 0; q < 4; ++q) {

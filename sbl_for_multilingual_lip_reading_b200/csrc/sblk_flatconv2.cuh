@@ -3,10 +3,14 @@
 // Reference: BasicBlock conv1/bn1/relu and conv2/bn2/+=residual/relu of ResNet layer1 (64 ch, 22x22) and layer2
 //            (128 ch, 11x11), SBL/transformer/video_frontend.py:10-12,28-41.
 //
-// Layout and trick are those of sblk_flatconv.cuh: pixel (f, y, x) lives at row (f*(H+1) + 1 + y)*(W+2) + 1 + x of a
-// [rows, C] bf16 matrix whose other rows are zero, so tap (r, s) of 128 consecutive output rows is the SAME staged
-// pixel run shifted by (r-1)*(W+2) + (s-1) rows; each run is staged once (TMA, SWIZZLE_128B) and the 9 taps are UMMA
-// descriptors with row-shifted start addresses.  What changes here:
+// Why not the im2col kernel (sblk_igemm.cuh): with N = 64 a 128 x 64 tile re-fetches 9 shifted copies of its
+// activations plus the whole filter from L2 (216 KB per tile, at the L2 -> SM fabric limit).  Here activations live in
+// a zero-haloed flat layout: pixel (f, y, x) lives at row (f*(H+1) + 1 + y)*(W+2) + 1 + x of a [rows, C] bf16 matrix
+// whose other rows are zero (one zero row between frames, zero columns left / right), so tap (r, s) of 128 consecutive
+// output rows is the SAME staged pixel run shifted by (r-1)*(W+2) + (s-1) rows; each run is staged once (TMA,
+// SWIZZLE_128B) and the 9 taps are UMMA descriptors with start addresses shifted by whole 128-byte rows (the swizzle is a
+// function of the absolute smem address, so row-shifted descriptors read the staged pixels correctly).  Outputs that
+// fall on halo positions are written as zeros, so the result is again a valid flat layout.  Further:
 //   * two CTAs (one TPC) compute 256 rows x C with ONE tcgen05.mma.cta_group::2 stream: each CTA stages its own 128-row
 //     pixel run but only HALF of the filter rows, so the shared-memory operand bytes per MMA drop from A+B to A+B/2
 //     (the N = 64 MMA of layer1 is bound by exactly that fetch: 6 KB -> 5 KB per M128xN64xK16) and layer2 gets the
@@ -81,8 +85,6 @@ struct FlatConv2Params {
   int relu;
   int has_res;
   const float* bias;           // [C] folded BN shift
-  unsigned long long* dbg;     // profiling aid (SBLK_FLAT_STAMPS=1): per-tile clock64 stamps of CTA 0, or nullptr
-  int debug_mode;              // SBLK_DEBUG builds, timing experiments (wrong results): 16 = issue the MMAs with N = 32
   // 1 = every CTA pair walks its tile range from the last tile to the first.  Consecutive convs of a stage alternate the
   // direction: the activation rows a pair wrote (and read) LAST in one conv are the first it reads in the next, i.e. the
   // ones most likely still in L2 (a layer-1 tensor is 65.6 MB, conv + residual + output 197 MB against 126 MB of L2).
@@ -284,18 +286,13 @@ flatconv2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
       uint32_t acc_phase = 0;
       const uint64_t db0 = make_desc_sw128(smem_base + Cfg::OFF_B);
       const uint32_t db0_lo = static_cast<uint32_t>(db0);
-      const uint32_t idesc = (p.debug_mode & 16) ? make_idesc_bf16(256, 32) : IDESC;
       uint32_t tap_off[9];   // (r*Wp + s) rows of 128 B, in descriptor units of 16 B
 #pragma unroll
       for (int t = 0; t < 9; ++t) tap_off[t] = static_cast<uint32_t>(((t / 3) * Wp + (t % 3)) * 8);
       if (Cfg::B_RESIDENT) mbar_wait(&b_full[0], 0, 0x0706);
-      unsigned long long* const dbg = (p.dbg != nullptr && blockIdx.x == 0 && lane == 0) ? p.dbg : nullptr;
       for (int tile = tile_begin; tile < tile_end; ++tile) {
-        if (dbg) dbg[(tile - tile_begin) * 16 + 0] = clock64();
         mbar_wait(&a_full[stage], phase, 0x0707);
-        if (dbg) dbg[(tile - tile_begin) * 16 + 1] = clock64();
         mbar_wait(&tempty_bar[acc], acc_phase ^ 1u, 0x0708);
-        if (dbg) dbg[(tile - tile_begin) * 16 + 2] = clock64();
         tc_fence_after_sync();
         const uint64_t da0 = make_desc_sw128(smem_base + Cfg::OFF_A + stage * Cfg::A_STAGE_BYTES);
         const uint32_t da0_lo = static_cast<uint32_t>(da0);
@@ -317,7 +314,7 @@ flatconv2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
 #pragma unroll
               for (int k = 0; k < 4; ++k)
                 umma2_bf16(d_tmem, desc_with_lo(da0, a_lo + static_cast<uint32_t>(2 * k)),
-                           desc_with_lo(db0, b_lo + static_cast<uint32_t>(2 * k)), idesc,
+                           desc_with_lo(db0, b_lo + static_cast<uint32_t>(2 * k)), IDESC,
                            (cb > 0 || t > 0 || k > 0) ? 1u : 0u);
               if (!Cfg::B_RESIDENT) umma2_commit_mc(&b_empty[slot]);
             }
@@ -332,7 +329,6 @@ flatconv2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
           umma2_commit_mc(&a_empty[stage]);
         }
         __syncwarp();
-        if (dbg) dbg[(tile - tile_begin) * 16 + 3] = clock64();
         if (++acc == ACC_STAGES) { acc = 0; acc_phase ^= 1u; }
         if (++stage == A_STAGES) { stage = 0; phase ^= 1u; }
       }
@@ -357,16 +353,11 @@ flatconv2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
       const int rb = j % Cfg::R_BUFS;
       const uint32_t rphase = static_cast<uint32_t>(j / Cfg::R_BUFS) & 1u;
       uint8_t* stg = smem + Cfg::OFF_R + rb * Cfg::R_BYTES;
-      unsigned long long* const dbg =
-          (p.dbg != nullptr && blockIdx.x == 0 && (ew & 3) == 0 && lane == 0) ? p.dbg + j * 16 : nullptr;
-      if (dbg) dbg[5] = clock64();
       mbar_wait(&tfull_bar[acc], acc_phase, 0x070a);
       tc_fence_after_sync();
-      if (dbg) dbg[6] = clock64();
       // the staging tile is usable: residual landed (has_res), or its previous store has been read out (first round of a
       // residual-free conv: nothing to wait for, hence the inverted parity)
       mbar_wait(&r_full[rb], p.has_res ? rphase : (rphase ^ 1u), 0x070b);
-      if (dbg) dbg[7] = clock64();
       const int m = row0 + arow;
       const int R = m / Wp;
       const int cpos = m - R * Wp;
@@ -419,11 +410,9 @@ flatconv2_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant_
       tc_fence_before_sync();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(tempty_leader + static_cast<uint32_t>(acc * 8));
-      if (dbg) dbg[8] = clock64();
       fence_proxy_async_smem();               // generic-proxy tile writes -> visible to the TMA store
       __syncwarp();
       if (lane == 0) mbar_arrive(&s_ready[rb]);   // 4 warps -> the store warp issues the tile's TMA store
-      if (dbg) dbg[9] = clock64();
     }
   }
 

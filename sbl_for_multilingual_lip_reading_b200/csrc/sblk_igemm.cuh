@@ -32,21 +32,17 @@ struct IgemmParams {
   const __nv_bfloat16* residual;   // [M, ldo] bf16 or nullptr
   __nv_bfloat16* out_bf16;         // [M, ldo] or nullptr
   float* out_f32;                  // [M, ldo] or nullptr
-  int debug_mode;                  // timing experiments only: bit0 = skip B loads, bit1 = skip A loads
-  // DUAL only: the 1x1 / same-stride downsample conv of a BasicBlock shares the centre-tap A tiles of conv1
+  // sblk_igemm2.cuh's dual-head kernel only: the 1x1 / same-stride downsample conv of a BasicBlock shares the
+  // centre-tap A tiles of conv1
   const float* bias2;              // [N] folded BN shift of the downsample branch
   __nv_bfloat16* out2_bf16;        // [M, ldo] downsample output (no ReLU)
   // split-K (linear layers at small M): K is cut into `splits` ranges, one tile per (split, m, n); split s writes its
   // fp32 partial to out_f32 + s * split_stride (bias added by split 0 only); the consumer sums the partials
   int splits;                      // >= 1
   long long split_stride;          // elements between partial outputs
-  // CTA-pair kernel only: write out / out2 into the zero-haloed flat layout of sblk_flatconv.cuh (halo rows are not
+  // CTA-pair kernel only: write out / out2 into the zero-haloed flat layout of sblk_flatconv2.cuh (halo rows are not
   // touched: the caller keeps them zero), output pixel (f, y, x) -> row (f*(P+1) + 1 + y)*(Q+2) + 1 + x
   int flat_out;
-  unsigned long long* dbg;         // profiling aid (SBLK_IGEMM2_STAMPS=1): clock64 stamps of CTA 0, or nullptr
-  // CTA-pair kernel only: 1 = epilogue stores go through per-warp staging tiles (coalesced rows) that take the place of
-  // the last ring stage; 0 = direct per-thread stores and the full ring (L2-latency-bound shapes need every stage)
-  int staged;
   // 16-bit float format of A, B, residual and out_bf16: 0 = bf16 (every conv), 1 = IEEE fp16 (the encoder's linear
   // layers, sblk_common.cuh "enc16"); both run as tcgen05 kind::f16 at the same rate
   int fp16;
@@ -59,26 +55,24 @@ struct IgemmParams {
   int ext_stride = 1;
 };
 
-template <int BLOCK_N, bool DUAL = false>
+template <int BLOCK_N>
 struct IgemmCfg {
   static constexpr int BLOCK_M = 128;
   static constexpr int BLOCK_K = 64;
   static constexpr int A_BYTES = BLOCK_M * BLOCK_K * 2;
   static constexpr int B_BYTES = BLOCK_N * BLOCK_K * 2;
-  static constexpr int STAGE_BYTES = A_BYTES + (DUAL ? 2 : 1) * B_BYTES;
-  static constexpr int STAGES = DUAL ? 4 : (BLOCK_N == 256) ? 4 : (BLOCK_N == 128) ? 6 : 8;
+  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
+  static constexpr int STAGES = (BLOCK_N == 256) ? 4 : (BLOCK_N == 128) ? 6 : 8;
   static constexpr int ACC_STAGES = 2;
-  static constexpr int TMEM_COLS = (DUAL ? 2 : 1) * ACC_STAGES * BLOCK_N;
+  static constexpr int TMEM_COLS = ACC_STAGES * BLOCK_N;
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024;  // + manual 1024-B alignment slack
   static constexpr int THREADS = 192;
 };
 
-template <int BLOCK_N, bool IM2COL, bool DUAL = false>
+template <int BLOCK_N, bool IM2COL>
 __global__ void __launch_bounds__(192, 1)
-igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-             const __grid_constant__ CUtensorMap tmB2, const IgemmParams p) {
-  using Cfg = IgemmCfg<BLOCK_N, DUAL>;
-  static_assert(!DUAL || (IM2COL && BLOCK_N <= 128), "DUAL needs im2col and 4 accumulators of <= 128 columns");
+igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const IgemmParams p) {
+  using Cfg = IgemmCfg<BLOCK_N>;
   constexpr int STAGES = Cfg::STAGES;
   const uint32_t IDESC = (!IM2COL && p.fp16) ? make_idesc_f16(Cfg::BLOCK_M, BLOCK_N)
                                               : make_idesc_bf16(Cfg::BLOCK_M, BLOCK_N);
@@ -107,7 +101,6 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
-    if (DUAL) tma_prefetch_desc(&tmB2);
 #pragma unroll
     for (int i = 0; i < STAGES; ++i) {
       mbar_init(&full_bar[i], 1);
@@ -156,21 +149,15 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
         mbar_wait(&empty_bar[stage], phase ^ 1u, 0x0101);
         uint8_t* a_dst = smem + stage * Cfg::STAGE_BYTES;
         uint8_t* b_dst = a_dst + Cfg::A_BYTES;
-        const bool centre = DUAL && r == p.taps_r / 2 && s == p.taps_s / 2;
         if (elect_one()) {
-          mbar_arrive_expect_tx(&full_bar[stage], ((p.debug_mode & 2) ? 0 : Cfg::A_BYTES) +
-                                                      ((p.debug_mode & 1) ? 0 : Cfg::B_BYTES) +
-                                                      (centre ? Cfg::B_BYTES : 0));
-          if (centre) tma_load_2d(b_dst + Cfg::B_BYTES, &tmB2, &full_bar[stage], cb * 64, n_blk * BLOCK_N);
-          if (!(p.debug_mode & 2)) {
-            if (IM2COL) {
-              tma_load_im2col_4d(a_dst, &tmA, &full_bar[stage], cb * 64, base_w, base_h, img,
-                                 static_cast<uint16_t>(s), static_cast<uint16_t>(r));
-            } else {
-              tma_load_2d(a_dst, &tmA, &full_bar[stage], (kb0 + kb) * 64, m0);
-            }
+          mbar_arrive_expect_tx(&full_bar[stage], Cfg::A_BYTES + Cfg::B_BYTES);
+          if (IM2COL) {
+            tma_load_im2col_4d(a_dst, &tmA, &full_bar[stage], cb * 64, base_w, base_h, img,
+                               static_cast<uint16_t>(s), static_cast<uint16_t>(r));
+          } else {
+            tma_load_2d(a_dst, &tmA, &full_bar[stage], (kb0 + kb) * 64, m0);
           }
-          if (!(p.debug_mode & 1)) tma_load_2d(b_dst, &tmB, &full_bar[stage], (kb0 + kb) * 64, n_blk * BLOCK_N);
+          tma_load_2d(b_dst, &tmB, &full_bar[stage], (kb0 + kb) * 64, n_blk * BLOCK_N);
         }
         __syncwarp();
         if (++cb == p.cblocks) {
@@ -190,8 +177,6 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
       mbar_wait(&tempty_bar[acc], acc_phase ^ 1u, 0x0102);
       tc_fence_after_sync();
       const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(acc * BLOCK_N);
-      const uint32_t d_tmem2 = tmem_base + static_cast<uint32_t>((Cfg::ACC_STAGES + acc) * BLOCK_N);
-      const int centre_kb0 = ((p.taps_r / 2) * p.taps_s + p.taps_s / 2) * p.cblocks;
       for (int kb = 0; kb < num_kb; ++kb) {
         mbar_wait(&full_bar[stage], phase, 0x0103);
         tc_fence_after_sync();
@@ -205,14 +190,6 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
             // advance 16 bf16 = 32 B inside the 128-B swizzle atom: +2 in the (addr >> 4) field
             umma_bf16(d_tmem, desc_with_lo(da, da_lo + 2 * k), desc_with_lo(db, db_lo + 2 * k), IDESC,
                       (kb > 0 || k > 0) ? 1u : 0u);
-          }
-          if (DUAL && kb >= centre_kb0 && kb < centre_kb0 + p.cblocks) {
-            // centre tap: the same A tile feeds the 1x1 downsample conv (second accumulator, filter tile behind B)
-#pragma unroll
-            for (int k = 0; k < Cfg::BLOCK_K / 16; ++k)
-              umma_bf16(d_tmem2, desc_with_lo(da, da_lo + 2 * k),
-                        desc_with_lo(db, db_lo + static_cast<uint32_t>(Cfg::B_BYTES / 16 + 2 * k)), IDESC,
-                        (kb > centre_kb0 || k > 0) ? 1u : 0u);
           }
           umma_commit(&empty_bar[stage]);  // frees this smem slot once the MMAs above retire
           if (kb == num_kb - 1) umma_commit(&tfull_bar[acc]);  // accumulator complete -> epilogue
@@ -298,31 +275,6 @@ igemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CU
             float4* op = reinterpret_cast<float4*>(p.out_f32 + static_cast<size_t>(split) * p.split_stride + row_off + n0);
 #pragma unroll
             for (int j = 0; j < 8; ++j) op[j] = make_float4(f[4 * j], f[4 * j + 1], f[4 * j + 2], f[4 * j + 3]);
-          }
-        }
-      }
-      if (DUAL) {
-        // downsample branch: accumulator 2, + bias2, no ReLU, no residual
-        const uint32_t t_row2 = t_row + static_cast<uint32_t>(Cfg::ACC_STAGES * BLOCK_N);
-#pragma unroll 1
-        for (int c = 0; c < BLOCK_N / 32; ++c) {
-          uint32_t v[32];
-          tmem_ld_32x32b_x32(t_row2 + static_cast<uint32_t>(c * 32), v);
-          tmem_ld_wait();
-          if (row_ok) {
-            const int n0 = n_blk * BLOCK_N + c * 32;
-            const float4* bp = reinterpret_cast<const float4*>(p.bias2 + n0);
-            uint4* op = reinterpret_cast<uint4*>(p.out2_bf16 + row_off + n0);
-#pragma unroll
-            for (int j = 0; j < 4; ++j) {
-              const float4 b0 = __ldg(bp + 2 * j), b1 = __ldg(bp + 2 * j + 1);
-              uint4 o;
-              o.x = pack_bf16x2(__uint_as_float(v[8 * j + 0]) + b0.x, __uint_as_float(v[8 * j + 1]) + b0.y);
-              o.y = pack_bf16x2(__uint_as_float(v[8 * j + 2]) + b0.z, __uint_as_float(v[8 * j + 3]) + b0.w);
-              o.z = pack_bf16x2(__uint_as_float(v[8 * j + 4]) + b1.x, __uint_as_float(v[8 * j + 5]) + b1.y);
-              o.w = pack_bf16x2(__uint_as_float(v[8 * j + 6]) + b1.z, __uint_as_float(v[8 * j + 7]) + b1.w);
-              op[j] = o;
-            }
           }
         }
       }

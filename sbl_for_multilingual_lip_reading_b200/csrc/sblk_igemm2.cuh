@@ -133,9 +133,10 @@ struct Igemm2Cfg {
   static constexpr int A_BYTES = BLOCK_M * BLOCK_K * 2;
   static constexpr int B_BYTES = BH * BLOCK_K * 2;
   static constexpr int STAGE_BYTES = A_BYTES + (DUAL ? 2 : 1) * B_BYTES;
-  // per-warp staging tiles of the 8 epilogue warps (32 rows x 128 B for BLOCK_N = 256, x 64 B for 128).  When a launch
-  // asks for staged stores (IgemmParams::staged) they take the place of the LAST ring stage; otherwise the ring keeps
-  // every stage: the L2-latency-bound shapes (strided block heads of layers 3-4) lose 14 % with one stage less.
+  // per-warp staging tiles of the 8 epilogue warps (32 rows x 128 B for BLOCK_N = 256, x 64 B for 128) for coalesced
+  // epilogue stores.  They take the place of the LAST ring stage: the L2-latency-bound shapes (strided block heads of
+  // layers 3-4) lose 14 % with one stage less, but the whole frontend graph measured 607 us with staged stores against
+  // 644 us with direct per-thread stores and the full ring.
   static constexpr int STG_WARP_BYTES = BLOCK_N == 256 ? 4096 : 2048;
   static constexpr int STG_BYTES = 8 * STG_WARP_BYTES;
   static constexpr int STAGES = (227 * 1024 - 2048) / STAGE_BYTES;
@@ -157,7 +158,7 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
   static_assert(BLOCK_N == 128 || BLOCK_N == 256, "BLOCK_N");
   static_assert(!DUAL || (IM2COL && BLOCK_N == 128), "DUAL needs im2col and BLOCK_N = 128");
   static_assert(Cfg::TMEM_COLS <= 512, "TMEM");
-  constexpr int STAGES = Cfg::STAGES;   // barrier arrays; the ring uses `nstages` of them
+  constexpr int STAGES = Cfg::STAGES - 1;   // ring stages: the last stage's bytes hold the staging tiles
   constexpr uint32_t IDESC = make_idesc_bf16(Cfg::PAIR_M, BLOCK_N);
 
   extern __shared__ uint8_t smem_raw[];
@@ -184,7 +185,6 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
   const int num_kb = num_kb_main + ((IM2COL && !DUAL) ? p.ext_cblocks : 0);
   const int pair_id = blockIdx.x >> 1;
   const int num_pairs = gridDim.x >> 1;
-  const int nstages = p.staged ? STAGES - 1 : STAGES;
 
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tmA);
@@ -213,8 +213,6 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
   grid_dep_launch();  // PDL: let the next kernel start its prologue now; its own wait orders the data
   // griddepcontrol.wait is executed by the roles that touch the previous kernel's data (producer: A tiles; epilogue:
   // residual / output)
-  unsigned long long* const dbg = (p.dbg != nullptr && blockIdx.x == 0 && lane == 0) ? p.dbg : nullptr;
-  if (dbg && warp == 0) dbg[0] = clock64();
 
   if (warp == 0) {
     // ------------------------------------------------ TMA producer (both CTAs): own A rows, own half of the B tile
@@ -268,13 +266,13 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
           cb = 0;
           if (++s == p.taps_s) { s = 0; ++r; }
         }
-        if (++stage == nstages) { stage = 0; phase ^= 1u; }
+        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
       }
     }
     // drain: every slot this CTA filled has been released (no multicast arrive can land after this CTA retires)
-    for (int i = 0; i < nstages; ++i) {
+    for (int i = 0; i < STAGES; ++i) {
       mbar_wait(&empty_bar[stage], phase ^ 1u, 0x0405);
-      if (++stage == nstages) { stage = 0; phase ^= 1u; }
+      if (++stage == STAGES) { stage = 0; phase ^= 1u; }
     }
   } else if (warp == 1) {
     // ------------------------------------------------ MMA issuer: leader CTA only (one elected lane issues)
@@ -292,7 +290,6 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
         for (int kb = 0; kb < num_kb; ++kb) {
           mbar_wait(&full_bar[stage], phase, 0x0403);
           tc_fence_after_sync();
-          if (dbg && tile == pair_id && (kb & 7) == 0) dbg[8 + (kb >> 3)] = clock64();
           const uint32_t a_addr = smem_u32(smem + stage * Cfg::STAGE_BYTES);
           const uint64_t da = make_desc_sw128(a_addr);
           const uint64_t db = make_desc_sw128(a_addr + Cfg::A_BYTES);
@@ -314,9 +311,8 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
             if (kb == num_kb - 1) umma2_commit_mc(&tfull_bar[acc]);  // accumulators complete in both CTAs
           }
           __syncwarp();
-          if (++stage == nstages) { stage = 0; phase ^= 1u; }
+          if (++stage == STAGES) { stage = 0; phase ^= 1u; }
         }
-        if (dbg) dbg[1 + (tile != pair_id)] = clock64();   // all MMAs of the first / last tile issued
         if (++acc == Cfg::ACC_STAGES) { acc = 0; acc_phase ^= 1u; }
       }
     }
@@ -373,7 +369,6 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
       }
       mbar_wait(&tfull_bar[acc], acc_phase, 0x0404);
       tc_fence_after_sync();
-      if (dbg && ew == 0) dbg[3 + 2 * (tile != pair_id)] = clock64();   // accumulator of the first / last tile ready
       const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16) +
                              static_cast<uint32_t>(acc * BLOCK_N + c_begin * 32);
       size_t out_row = static_cast<size_t>(m);
@@ -420,13 +415,7 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
           }
         }
         const int n0 = ncol0 + c2 * 64;
-        if (p.out_bf16 != nullptr && !p.staged) {
-          if (row_ok) {
-            uint4* op = reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(p.out_bf16 + n0) + row_off_b);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) op[j] = o[j];
-          }
-        } else if (p.out_bf16 != nullptr) {
+        if (p.out_bf16 != nullptr) {
           if (BLOCK_N == 256) {
             warp_store_rows128_idx(stg, o, reinterpret_cast<uint8_t*>(p.out_bf16 + n0), row_off_b, row_ok, lane);
           } else {
@@ -460,25 +449,16 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
               o[hh * 4 + j].w = pack_bf16x2(__uint_as_float(v2[hh][8 * j + 6]) + b1.z, __uint_as_float(v2[hh][8 * j + 7]) + b1.w);
             }
           }
-          if (!p.staged) {
-            if (row_ok) {
-              uint4* op = reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(p.out2_bf16 + ncol0 + c2 * 64) + row_off_b);
-#pragma unroll
-              for (int j = 0; j < 8; ++j) op[j] = o[j];
-            }
-          } else {
-            const uint4 (&o0)[4] = *reinterpret_cast<const uint4 (*)[4]>(&o[0]);
-            const uint4 (&o1)[4] = *reinterpret_cast<const uint4 (*)[4]>(&o[4]);
-            uint8_t* g2 = reinterpret_cast<uint8_t*>(p.out2_bf16 + ncol0 + c2 * 64);
-            warp_store_rows64_idx(stg, o0, g2, row_off_b, row_ok, lane);
-            warp_store_rows64_idx(stg, o1, g2 + 64, row_off_b, row_ok, lane);
-          }
+          const uint4 (&o0)[4] = *reinterpret_cast<const uint4 (*)[4]>(&o[0]);
+          const uint4 (&o1)[4] = *reinterpret_cast<const uint4 (*)[4]>(&o[4]);
+          uint8_t* g2 = reinterpret_cast<uint8_t*>(p.out2_bf16 + ncol0 + c2 * 64);
+          warp_store_rows64_idx(stg, o0, g2, row_off_b, row_ok, lane);
+          warp_store_rows64_idx(stg, o1, g2 + 64, row_off_b, row_ok, lane);
         }
       }
       tc_fence_before_sync();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(mapa_u32(smem_u32(&tempty_bar[acc]), 0));   // the leader's barrier
-      if (dbg && ew == 0) dbg[4 + 2 * (tile != pair_id)] = clock64();   // epilogue of the first / last tile done
       if (++acc == Cfg::ACC_STAGES) { acc = 0; acc_phase ^= 1u; }
     }
   }
@@ -486,7 +466,6 @@ igemm2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
   tc_fence_before_sync();
   __syncthreads();
   cluster_sync_all();   // both CTAs are done with each other's smem / TMEM / barriers
-  if (dbg && warp == 0) dbg[7] = clock64();
   if (warp == 1) {
     __syncwarp();
     tmem_dealloc_2cta(tmem_base, Cfg::TMEM_COLS);

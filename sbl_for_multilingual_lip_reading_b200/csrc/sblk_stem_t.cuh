@@ -92,8 +92,6 @@ struct StemTParams {
   const float* bias;          // [64] folded BN shift
   __nv_bfloat16* out;         // [F,22,22,64], or the zero-haloed flat layout when flat_out
   int flat_out;
-  unsigned long long* dbg;    // optional clock stamps of every CTA [grid][8] (SBLK_DEBUG builds), or nullptr
-  int debug_mode;             // 0 = normal; timing experiments (SBLK_DEBUG builds), bit mask: 1 no MMAs, 2 no loads, 4 no accumulator reads, 8 no pooling / stores, 16 MMAs with N = 32, 32 no stores, 64 fused producers load nothing, 128 fused producers store nothing
 };
 
 // Epilogue of one warp: pooled columns [11 * HALF, 11 * HALF + 11) of every tile step, for the 32 (frame, channel) lanes
@@ -156,13 +154,6 @@ __device__ __forceinline__ void stem_t_epilogue(const StemTParams& p, uint32_t t
     tc_fence_after_sync();
     uint32_t r0[32], r1[32];
     const uint32_t taddr = t_lane + static_cast<uint32_t>(buf * TILE_N);
-    if (p.debug_mode & 4) {   // no accumulator reads at all: MMA stream + barriers only
-      tc_fence_before_sync();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&accempty_bar[buf]);
-      if (++buf == ACC_BUFS) { buf = 0; buf_phase ^= 1u; }
-      continue;
-    }
     tmem_ld_32x32b_x32(taddr, r0);
     tmem_ld_32x32b_x32(taddr + static_cast<uint32_t>(CONV_HW), r1);
     tmem_ld_wait();
@@ -170,7 +161,6 @@ __device__ __forceinline__ void stem_t_epilogue(const StemTParams& p, uint32_t t
     __syncwarp();
     if (lane == 0) mbar_arrive(&accempty_bar[buf]);
     if (++buf == ACC_BUFS) { buf = 0; buf_phase ^= 1u; }
-    if (p.debug_mode & 8) continue;
 
     float o[HP];
 #pragma unroll
@@ -186,7 +176,7 @@ __device__ __forceinline__ void stem_t_epilogue(const StemTParams& p, uint32_t t
       o[x] = fmaxf(fmaxf(top, h0), h1);
       carry[x] = h1;
     }
-    const bool store = s >= s_own && (t0 + j) < T && !(p.debug_mode & 32);
+    const bool store = s >= s_own && (t0 + j) < T;
     if (store) {
       const long long f = static_cast<long long>(n) * T + t0 + j;
       if (p.flat_out) {
@@ -280,7 +270,7 @@ __device__ __forceinline__ void stem_t_produce(const StemTParams& p, uint8_t* sm
         dsto[b] = static_cast<uint32_t>((pp * 2 + pl) * WIN_BYTES + (r * CONV_HW + 4 * q) * 16);
         edge0[b] = q == 0;
         edge3[b] = q == 10;
-        bool row = item[b] && y >= 0 && y < c3d::IN_HW && !(p.debug_mode & 64);   // else: zero entries
+        bool row = item[b] && y >= 0 && y < c3d::IN_HW;   // else: zero entries
         if (SRC == 1) {
           const float4* src = reinterpret_cast<const float4*>(
                                   p.x_f32 + ((static_cast<size_t>(n) * T + tp) * c3d::IN_HW + y) * c3d::IN_HW) + (2 * q - 1);
@@ -337,7 +327,7 @@ __device__ __forceinline__ void stem_t_produce(const StemTParams& p, uint8_t* sm
         for (int e = 0; e < 4; ++e) E[e] = make_uint4(F[e], F[e + 1], F[e + 2], F[e + 3]);
         if (rho & 1) { const uint4 t = E[0]; E[0] = E[1]; E[1] = E[2]; E[2] = E[3]; E[3] = t; }
         if (rho & 2) { uint4 t = E[0]; E[0] = E[2]; E[2] = t; t = E[1]; E[1] = E[3]; E[3] = t; }
-        if (item[b] && !(p.debug_mode & 128)) {
+        if (item[b]) {
           uint8_t* const dst = sbase + dsto[b];
 #pragma unroll
           for (int st = 0; st < 4; ++st) *reinterpret_cast<uint4*>(dst + (((st + rho) & 3) << 4)) = E[st];
@@ -374,11 +364,6 @@ stem_t_kernel(const StemTParams p) {
 
   const int warp = uniform_warp_idx();
   const int lane = threadIdx.x & 31;
-  unsigned long long* const dbg = (p.dbg != nullptr && lane == 0) ? p.dbg + blockIdx.x * 8 : nullptr;
-  auto stamp = [&](int which) {
-    if (dbg != nullptr) dbg[which] = static_cast<unsigned long long>(clock64());
-  };
-  if (warp == 0) stamp(0);
   const int T = p.T;
   const int TP = T + 2 * c3d::TPAD;
   const int ppc = (T + 1) >> 1;                      // frame pairs per clip (the last one is half empty when T is odd)
@@ -441,9 +426,7 @@ stem_t_kernel(const StemTParams p) {
     if (threadIdx.x < 256) lut_s[threadIdx.x] = __ldg(p.lut_bf16 + threadIdx.x);
     __syncthreads();
   }
-  if (warp == 0) stamp(1);
   grid_dep_wait();
-  if (warp == 0) stamp(2);
 
   if (warp == 0 && !FUSED) {
     // ------------------------------------------------ loader: per group of <= G tiles, the entry windows of the
@@ -468,26 +451,21 @@ stem_t_kernel(const StemTParams p) {
       }
       mbar_wait(&empty_bar[stage], phase ^ 1u, 0x0901);
       if (elect_one()) {
-        if (p.debug_mode & 2) {
-          mbar_arrive(&full_bar[stage]);
-        } else {
-          mbar_arrive_expect_tx(&full_bar[stage], static_cast<uint32_t>(2 * nvalid) * bytes);
+        mbar_arrive_expect_tx(&full_bar[stage], static_cast<uint32_t>(2 * nvalid) * bytes);
 #pragma unroll 1
-          for (int pp = 0; pp < NP; ++pp) {
-            const int tp = t0 - 2 + pp;
-            if (tp < 0 || tp >= T) continue;   // zero padding frames contribute nothing: no load, no MMA
-            const uint4* src = p.x8 + static_cast<size_t>(n * TP + t0 + pp) * c3d::FRAME_ENTRIES + i0 * TILE_PX;
-            uint8_t* dst = smem + stage * STAGE_BYTES + pp * (2 * WIN_BYTES);
-            bulk_load(dst, src, bytes, &full_bar[stage]);
-            bulk_load(dst + WIN_BYTES, src + c3d::PLANE_ENTRIES, bytes, &full_bar[stage]);
-          }
+        for (int pp = 0; pp < NP; ++pp) {
+          const int tp = t0 - 2 + pp;
+          if (tp < 0 || tp >= T) continue;   // zero padding frames contribute nothing: no load, no MMA
+          const uint4* src = p.x8 + static_cast<size_t>(n * TP + t0 + pp) * c3d::FRAME_ENTRIES + i0 * TILE_PX;
+          uint8_t* dst = smem + stage * STAGE_BYTES + pp * (2 * WIN_BYTES);
+          bulk_load(dst, src, bytes, &full_bar[stage]);
+          bulk_load(dst + WIN_BYTES, src + c3d::PLANE_ENTRIES, bytes, &full_bar[stage]);
         }
       }
       __syncwarp();
       if (++stage == STAGES) { stage = 0; phase ^= 1u; }
       s += gn;
     }
-    stamp(6);
   } else if (FUSED && (warp == 0 || warp >= 3 + EPI_WARPS)) {
     stem_t_produce<SRC>(p, smem, lut_s, full_bar, empty_bar, s_begin, s_end,
                         (warp == 0 ? 0 : (warp - (2 + EPI_WARPS)) * 32) + lane, lane);
@@ -500,7 +478,6 @@ stem_t_kernel(const StemTParams p) {
     const uint64_t db0 = make_desc_kmajor_noswizzle(smem_base, WIN_BYTES, 128);
     mbar_wait(&filter_bar, 0, 0x0905);
     tc_fence_after_sync();
-    const uint32_t idesc = (p.debug_mode & 16) ? make_idesc_bf16(128, 32) : IDESC;   // 16: same issue stream, a third of the math
     const uint32_t db0_lo = static_cast<uint32_t>(db0);
     const uint32_t a_tmem = tmem_base + static_cast<uint32_t>(A_COL0);
     int s = s_begin;
@@ -533,23 +510,20 @@ stem_t_kernel(const StemTParams p) {
         if (!waited) {
           mbar_wait(&full_bar[stage], phase, 0x0903);
           waited = true;
-          if (s == s_begin) stamp(3 + 4 * me);
         }
         tc_fence_after_sync();
         const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(buf * TILE_N);
         const uint32_t b_lo = db0_lo + static_cast<uint32_t>((stage * STAGE_BYTES + k * (TILE_PX * 16)) >> 4);
         bool last_mine = k == gn - 1 || k == gn - 2;   // no later tile of this group is this warp's
         if (elect_one()) {
-          if (!(p.debug_mode & 1)) {
 #pragma unroll
-            for (int pp = 0; pp < NP; ++pp) {
-              if (vmask & (1u << pp)) {
+          for (int pp = 0; pp < NP; ++pp) {
+            if (vmask & (1u << pp)) {
 #pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                  umma_bf16_ts(d_tmem, a_tmem + static_cast<uint32_t>((pp * 4 + q) * A_CHUNK_COLS),
-                               desc_with_lo(db0, b_lo + static_cast<uint32_t>((pp * (2 * WIN_BYTES) + q * CONV_HW * 16) >> 4)),
-                               idesc, (pp == first_pp && q == 0) ? 0u : 1u);
-                }
+              for (int q = 0; q < 4; ++q) {
+                umma_bf16_ts(d_tmem, a_tmem + static_cast<uint32_t>((pp * 4 + q) * A_CHUNK_COLS),
+                             desc_with_lo(db0, b_lo + static_cast<uint32_t>((pp * (2 * WIN_BYTES) + q * CONV_HW * 16) >> 4)),
+                             IDESC, (pp == first_pp && q == 0) ? 0u : 1u);
               }
             }
           }
@@ -565,13 +539,11 @@ stem_t_kernel(const StemTParams p) {
       ++grp;
       s += gn;
     }
-    if (me == 0) stamp(4);
   } else {
     // ------------------------------------------------ epilogue: warp pairs (ew, ew + 4) share a TMEM lane quarter;
     // thread = one (frame j, channel co) lane and one half of the 22 pooled columns
     if (warp < 6) stem_t_epilogue<0>(p, tmem_base, accfull_bar, accempty_bar, s_begin, s_own, s_end, warp, lane);
     else stem_t_epilogue<1>(p, tmem_base, accfull_bar, accempty_bar, s_begin, s_own, s_end, warp, lane);
-    if (warp == 2) stamp(5);
   }
 
   tc_fence_before_sync();

@@ -199,7 +199,7 @@ def prep_clip(x, out=None):
 
 
 class FlatActs:
-    """Activations in the zero-haloed flat layout of csrc/sblk_flatconv.cuh: `data` is bf16 [rows, C] with pixel
+    """Activations in the zero-haloed flat layout of csrc/sblk_flatconv2.cuh: `data` is bf16 [rows, C] with pixel
     (f, y, x) at row (f*(H+1) + 1 + y)*(W+2) + 1 + x and zeros everywhere else."""
     __slots__ = ("data", "f", "h", "w")
 
