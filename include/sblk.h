@@ -317,6 +317,21 @@ int sblk_im2col_t(const void* x, void* out, int F, int H, int W, int C, int R, i
 /* im2col of the Conv3d stem (x fp32 [N,T,88,88]; k = (dt*7 + r)*7 + s, 245 taps zero-padded to 256):
  * transposed = 0 -> bf16 [N*T*44*44, 256] (A operand of the training-forward GEMM); 1 -> bf16 [256, ld_out] (wgrad). */
 int sblk_stem_im2col(const float* x, void* out, int N, int T, int transposed, long long ld_out, void* stream);
+/* im2col of the Conv3d stem straight from raw uint8 gray frames x_u8 [N, T_in, H0, W0]:
+ * value = lut_bf16[x_u8[n, t, y1 + y, x1 + xm]], xm = flip[n] ? 87 - x : x, with (y1, x1) = crop_yx[n*T_in + t]
+ * (or (crop_y0, crop_x0) for every frame when crop_yx == NULL); frames t >= T_in are zero (padding in normalised
+ * space); flip may be NULL (no clip mirrored).  Same output layout as sblk_stem_im2col with T = T_out:
+ * transposed = 0 -> bf16 [N*T_out*44*44, 256]; 1 -> bf16 [256, ld_out].
+ * The crop comes first, in source coordinates; the flip mirrors the 88 x 88 crop (torch.flip(clip, dims=[-1])).
+ * Per-frame offsets in crop_yx live in device memory and are not checked here: the kernel clamps each into
+ * [0, H0-88] x [0, W0-88], so it never reads outside its frame.  A uniform crop outside the frame is an error.
+ * With lut_bf16 = bf16(float32((u / 255. - mean) / std)) the output is bit-identical to sblk_stem_im2col of the clip
+ * the reference loader builds on the host.
+ * replaces: load_file / ColorNormalize / RandomCrop / HorizontalFlip / frame zero-padding of the training loader
+ * + the stem's im2col, SBL/data_gen.py:122-125,276-296, cvtransforms.py:7-48 */
+int sblk_stem_im2col_u8(const void* x_u8, const void* lut_bf16, const int* crop_yx, int crop_y0, int crop_x0,
+                        const int* flip, void* out, int N, int T_in, int T_out, int H0, int W0, int transposed,
+                        long long ld_out, void* stream);
 /* Deterministic per-channel reductions over the rows of [M, C] -> out_2C = (first[C], second[C]):
  *   mode 0: a 16-bit -> (sum, sum of squares)        mode 2: a fp32 -> (sum, -)        mode 4: a 16-bit -> (sum, -)
  *   mode 1: BatchNorm backward sums (sum dz, sum dz * xhat): a = dy bf16, b = BN output bf16 (ReLU mask) or NULL,

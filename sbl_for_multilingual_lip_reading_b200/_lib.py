@@ -84,6 +84,7 @@ SIGNATURES = {
     "sblk_transpose16": (_i, [_vp, _vp, _ll, _i, _ll, _ll, _i, _vp]),
     "sblk_im2col_t": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _ll, _vp]),
     "sblk_stem_im2col": (_i, [_vp, _vp, _i, _i, _i, _ll, _vp]),
+    "sblk_stem_im2col_u8": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _ll, _vp]),
     "sblk_colreduce_workspace_floats": (_ll, [_i]),
     "sblk_colreduce": (_i, [_i, _vp, _vp, _vp, _vp, _vp, _ll, _i, _i, _vp, _vp, _vp]),
     "sblk_bn_finalize": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _f, _f, _f, _vp]),

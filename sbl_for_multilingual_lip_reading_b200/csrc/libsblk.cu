@@ -1321,6 +1321,36 @@ int sblk_stem_im2col(const float* x, void* out, int N, int T, int transposed, lo
                 "stem_im2col_kernel", x, static_cast<uint16_t*>(out), N, T, transposed, ld_out);
 }
 
+int sblk_stem_im2col_u8(const void* x_u8, const void* lut_bf16, const int* crop_yx, int crop_y0, int crop_x0,
+                        const int* flip, void* out, int N, int T_in, int T_out, int H0, int W0, int transposed,
+                        long long ld_out, void* stream) {
+  int sms, rc;
+  if ((rc = ensure_init(&sms))) return rc;
+  if (!x_u8 || !lut_bf16 || !out) return fail(-1, "sblk_stem_im2col_u8: null pointer");
+  if (N <= 0 || T_in <= 0 || T_out < T_in || H0 < 88 || W0 < 88)
+    return fail(-1, "sblk_stem_im2col_u8: bad shape N=%d T_in=%d T_out=%d H0=%d W0=%d (T_out >= T_in, frames >= 88x88)",
+                N, T_in, T_out, H0, W0);
+  if (!crop_yx && (crop_y0 < 0 || crop_x0 < 0 || crop_y0 + 88 > H0 || crop_x0 + 88 > W0))
+    return fail(-1, "sblk_stem_im2col_u8: crop offset (%d, %d) leaves the %dx%d frame", crop_y0, crop_x0, H0, W0);
+  const long long M = static_cast<long long>(N) * T_out * 44 * 44;
+  if (transposed && (ld_out < M || (ld_out & 1))) return fail(-1, "sblk_stem_im2col_u8: ld_out must be even and >= M");
+  if (!aligned16(out)) return fail(-1, "sblk_stem_im2col_u8: output must be 16-byte aligned");
+  const long long rows = static_cast<long long>(N) * T_out * 44;
+  if (!transposed && rows > 0x7fffffffLL) return fail(-1, "sblk_stem_im2col_u8: too many frames for one launch (%lld rows)", rows);
+  // transposed: one block per (temporal tap, 1936-column frame slot), the sixth tap group writes the zero rows 245..255
+  const dim3 grid = transposed ? dim3(6, static_cast<unsigned>((ld_out + 1935) / 1936)) : dim3(static_cast<unsigned>(rows));
+  if (transposed && grid.y > 65535u) return fail(-1, "sblk_stem_im2col_u8: too many frames for one launch (%u)", grid.y);
+  sblk::StemU8Src s;
+  s.x = static_cast<const uint8_t*>(x_u8);
+  s.lut = static_cast<const uint16_t*>(lut_bf16);
+  s.crop_yx = crop_yx;
+  s.flip = flip;
+  s.crop_y0 = crop_y0; s.crop_x0 = crop_x0;
+  s.N = N; s.T_in = T_in; s.T = T_out; s.H0 = H0; s.W0 = W0;
+  return launch(sblk::stem_im2col_u8_kernel, grid, dim3(256), 0, static_cast<cudaStream_t>(stream), false,
+                "stem_im2col_u8_kernel", s, static_cast<uint16_t*>(out), transposed, ld_out);
+}
+
 static const int kColReduceBlocks = 592;
 long long sblk_colreduce_workspace_floats(int C) { return C > 0 ? static_cast<long long>(kColReduceBlocks) * 2 * C : -1; }
 

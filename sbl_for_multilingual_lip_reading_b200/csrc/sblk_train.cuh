@@ -208,6 +208,130 @@ stem_im2col_kernel(const float* __restrict__ x, uint16_t* __restrict__ out, int 
 }
 
 // ----------------------------------------------------------------------------------------------------------------
+// The same im2col straight from the training loader's raw uint8 gray frames x [N, T_in, H0, W0]: the clip value at
+// (n, t, y, x) is lut[x[n, t, cy + y, cx + (flip[n] ? 87 - x : x)]] for t < T_in and 0 for T_in <= t < T (frame
+// zero-padding in normalised space), with (cy, cx) = crop_yx[n*T_in + t] clamped into [0, H0-88] x [0, W0-88] (the
+// offsets live in device memory, where the C ABI cannot check them), or (crop_y0, crop_x0) when crop_yx is null.
+// lut[u] = bf16(float32((u/255 - mean)/std)) is what pack_bf16x2 makes of the reference loader's fp32 clip, so the
+// output is bit-identical to stem_im2col_kernel on that clip.  Same grids and output layouts as stem_im2col_kernel.
+// ----------------------------------------------------------------------------------------------------------------
+struct StemU8Src {
+  const uint8_t* x;
+  const uint16_t* lut;   // bf16 bits [256]
+  const int* crop_yx;    // [N*T_in][2] (y, x) or nullptr
+  const int* flip;       // [N] or nullptr
+  int crop_y0, crop_x0, N, T_in, T, H0, W0;
+};
+
+// top-left pixel of the 88x88 crop of clip frame (n, t), t < T_in
+__device__ __forceinline__ const uint8_t* stem_u8_crop(const StemU8Src& s, long long n, int t) {
+  const long long fr = n * s.T_in + t;
+  int cy = s.crop_y0, cx = s.crop_x0;
+  if (s.crop_yx != nullptr) {
+    cy = min(max(__ldg(s.crop_yx + 2 * fr), 0), s.H0 - 88);
+    cx = min(max(__ldg(s.crop_yx + 2 * fr + 1), 0), s.W0 - 88);
+  }
+  return s.x + (fr * s.H0 + cy) * s.W0 + cx;
+}
+
+// transposed == 0: blockIdx.x = output row (f, y); the 5 frames x 7 rows x 94 columns (88 + the 3-pixel halo on either
+//   side) its 44 x 245 taps read are normalised once into shared memory, then the taps are stored as in stem_im2col_kernel
+// transposed == 1: blockIdx.x = temporal tap dt (5: the zero rows 245..255), blockIdx.y = frame slot; the one source frame
+//   the 49 taps (dt, r, s) read is normalised (and mirrored) once into a zero-haloed 94 x 94 tile in shared memory, then
+//   each of the 49 output rows gets the slot's 1936 pixels as 2-pixel 4-byte stores
+constexpr int kStemU8Tile = 94 * 96;       // uint16 elements: the transposed tile (row pitch 96); holds the 35 x 96 window
+__global__ void __launch_bounds__(256)
+stem_im2col_u8_kernel(StemU8Src s, uint16_t* __restrict__ out, int transposed, long long ld_out) {
+  __shared__ uint16_t lut[256];
+  __shared__ __align__(16) uint16_t tile[kStemU8Tile];
+  __shared__ const uint8_t* crop[5];          // transposed == 0: crops of the frames t-2 .. t+2 (nullptr: zero frame)
+  lut[threadIdx.x] = __ldg(s.lut + threadIdx.x);
+  if (!transposed) {
+    uint16_t (*win)[96] = reinterpret_cast<uint16_t (*)[96]>(tile);   // [5 * 7][96]
+    const int fy = blockIdx.x;                  // f * 44 + y
+    const int y = fy % 44;
+    const int f = fy / 44;
+    const int t = f % s.T;
+    const long long n = f / s.T;
+    if (threadIdx.x < 5) {
+      const int tt = t + static_cast<int>(threadIdx.x) - 2;
+      crop[threadIdx.x] = (tt >= 0 && tt < s.T_in) ? stem_u8_crop(s, n, tt) : nullptr;
+    }
+    __syncthreads();
+    const bool mirror = s.flip != nullptr && __ldg(s.flip + n) != 0;
+    for (int i = threadIdx.x; i < 5 * 7 * 94; i += blockDim.x) {
+      const int row = i / 94, col = i - row * 94;
+      const int dt = row / 7, r = row - dt * 7;
+      const int yy = 2 * y + r - 3, xx = col - 3;
+      const uint8_t* src = crop[dt];
+      uint16_t v = 0;
+      if (src != nullptr && yy >= 0 && yy < 88 && xx >= 0 && xx < 88)
+        v = lut[__ldg(src + yy * s.W0 + (mirror ? 87 - xx : xx))];
+      win[row][col] = v;
+    }
+    __syncthreads();
+    uint4* dst = reinterpret_cast<uint4*>(out) + static_cast<long long>(fy) * 44 * 32;
+    for (int i = threadIdx.x; i < 44 * 32; i += blockDim.x) {
+      const int xo = i >> 5;
+      const int k0 = (i & 31) * 8;
+      uint32_t w[4];
+#pragma unroll
+      for (int j = 0; j < 8; j += 2) {
+        uint32_t h[2];
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          const int k = k0 + j + e;
+          const int dt = k / 49, rs = k - dt * 49, r = rs / 7, sx = rs - r * 7;
+          h[e] = k < 245 ? win[dt * 7 + r][2 * xo + sx] : 0u;
+        }
+        w[j >> 1] = h[0] | (h[1] << 16);
+      }
+      dst[i] = make_uint4(w[0], w[1], w[2], w[3]);
+    }
+  } else {
+    const int dt = blockIdx.x;
+    const int f = blockIdx.y;
+    const long long m0 = static_cast<long long>(f) * 1936;
+    const int t = f % s.T;
+    const int tt = t + dt - 2;
+    const bool real = dt < 5 && f < s.N * s.T && tt >= 0 && tt < s.T_in;   // block-uniform
+    __syncthreads();
+    if (real) {
+      const long long n = f / s.T;
+      const uint8_t* src = stem_u8_crop(s, n, tt);
+      const bool mirror = s.flip != nullptr && __ldg(s.flip + n) != 0;
+      for (int i = threadIdx.x; i < 94 * 94; i += blockDim.x) {
+        const int yy = i / 94 - 3, xx = i - (yy + 3) * 94 - 3;
+        uint16_t v = 0;
+        if (yy >= 0 && yy < 88 && xx >= 0 && xx < 88) v = lut[__ldg(src + yy * s.W0 + (mirror ? 87 - xx : xx))];
+        tile[(yy + 3) * 96 + xx + 3] = v;
+      }
+      __syncthreads();
+    }
+    const int k0 = dt * 49;
+    const int rows = dt < 5 ? 49 : 256 - 245;
+    for (int rr = 0; rr < rows; ++rr) {
+      const int r = rr / 7, sx = rr - r * 7;
+      uint32_t* dst = reinterpret_cast<uint32_t*>(out + static_cast<long long>(k0 + rr) * ld_out + m0);
+      for (int i = threadIdx.x; i < 968; i += blockDim.x) {      // 968 pixel pairs of one frame
+        const long long m = m0 + 2 * i;
+        if (m >= ld_out) break;
+        uint32_t a = 0u, b = 0u;
+        if (real) {
+          const int px = 2 * i;
+          const int y = px / 44, xo = px - y * 44;              // 44 is even: both pixels in the same row
+          const uint16_t* p = tile + (2 * y + r) * 96 + 2 * xo + sx;
+          a = p[0];
+          b = p[2];
+        }
+        if (m + 1 < ld_out) dst[i] = a | (b << 16);
+        else *reinterpret_cast<uint16_t*>(dst + i) = static_cast<uint16_t>(a);
+      }
+    }
+  }
+}
+
+// ----------------------------------------------------------------------------------------------------------------
 // Per-channel (column) reductions over the rows of a [M, C] matrix, deterministic two-stage: every block writes its
 // partial sums to part[block][2][C], colreduce_finish_kernel adds the blocks in order.  Modes:
 //   0  x 16-bit                    -> (sum x, sum x^2)                          BatchNorm batch statistics

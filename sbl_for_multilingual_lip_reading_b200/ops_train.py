@@ -91,6 +91,63 @@ def stem_im2col(x, transposed=False, ld_out=None):
     return out
 
 
+def stem_im2col_u8(x_u8, lut, t_out, crop, flip=None, transposed=False, ld_out=None):
+    """Raw uint8 gray frames [N,T_in,H0,W0] -> the stem_im2col of the clip the training loader builds from them (/255,
+    ColorNormalize, 88x88 crop, optional horizontal mirror of the crop, zero-padding to `t_out` frames), bit for bit.
+    `lut`: bf16 [256] (synth.normalize_lut()).  `crop`: (y1, x1) for every frame, or int32 [N*T_in, 2] per-frame (y1, x1)
+    offsets (RandomCrop; a CPU tensor is range-checked here and uploaded, offsets already on the GPU are clamped into the
+    frame by the kernel).  `flip`: None or a bool / integer tensor [N], nonzero = mirror that clip."""
+    if not torch.is_tensor(x_u8) or not x_u8.is_cuda or x_u8.dtype != torch.uint8 or x_u8.dim() != 4:
+        raise RuntimeError("stem_im2col_u8: expected a CUDA uint8 tensor [N,T,H0,W0] (no CPU fallback exists)")
+    if not x_u8.is_contiguous():
+        raise RuntimeError("stem_im2col_u8: expected a contiguous tensor")
+    _req(lut, BF16, "lut")
+    if lut.numel() != 256:
+        raise RuntimeError("stem_im2col_u8: lut must hold 256 bf16 values")
+    n, t_in, h0, w0 = x_u8.shape
+    t_out = int(t_out)
+    crop_t, cy, cx = None, 0, 0
+    if torch.is_tensor(crop):
+        crop_t = crop_offsets_to(crop, n * t_in, h0, w0, x_u8.device)
+    else:
+        cy, cx = int(crop[0]), int(crop[1])
+    flip_t = None if flip is None else flip_flags_to(flip, n, x_u8.device)
+    m = n * t_out * 44 * 44
+    if transposed:
+        ld_out = m if ld_out is None else int(ld_out)
+        out = torch.empty((256, ld_out), dtype=BF16, device=x_u8.device)
+    else:
+        ld_out = 256
+        out = torch.empty((m, 256), dtype=BF16, device=x_u8.device)
+    _call("sblk_stem_im2col_u8", "stem_im2col_u8", 0, x_u8.numel() + 2 * out.numel(), _p(x_u8), _p(lut), _p(crop_t), cy,
+          cx, _p(flip_t), _p(out), n, t_in, t_out, h0, w0, 1 if transposed else 0, ld_out, _stream())
+    return out
+
+
+def crop_offsets_to(crop, frames, h0, w0, device):
+    """Per-frame crop offsets as the int32 [frames, 2] (y1, x1) CUDA tensor the uint8 stem reads.  Offsets that arrive on
+    the CPU must keep the 88x88 crop inside the h0 x w0 frame (RuntimeError otherwise); on the GPU they cannot be read
+    without a synchronisation, and the kernel clamps them."""
+    if crop.dtype != torch.int32 or tuple(crop.shape) != (frames, 2):
+        raise RuntimeError(f"crop: per-frame offsets must be int32 [{frames}, 2], got {crop.dtype} {tuple(crop.shape)}")
+    if not crop.is_cuda:
+        y, x = crop[:, 0], crop[:, 1]
+        bad = (y < 0) | (y > h0 - 88) | (x < 0) | (x > w0 - 88)
+        if bool(bad.any()):
+            i = int(bad.nonzero()[0, 0])
+            raise RuntimeError(f"crop: offset ({int(y[i])}, {int(x[i])}) of frame {i} leaves the {h0}x{w0} frame")
+    return crop.to(device=device).contiguous()
+
+
+def flip_flags_to(flip, n, device):
+    """Per-clip mirror flags (bool / integer [n], nonzero = mirror) as the int32 CUDA tensor the uint8 stem reads."""
+    if not torch.is_tensor(flip) or flip.dtype.is_floating_point or flip.dtype.is_complex or tuple(flip.shape) != (n,):
+        raise RuntimeError(f"flip: expected a bool or integer tensor [{n}], got "
+                           f"{flip.dtype if torch.is_tensor(flip) else type(flip).__name__} "
+                           f"{tuple(flip.shape) if torch.is_tensor(flip) else ''}")
+    return flip.to(device=device, dtype=torch.int32).contiguous()
+
+
 def colreduce(mode, a, b=None, c=None, mean=None, rstd=None):
     """Deterministic per-channel reductions (see include/sblk.h: sblk_colreduce) -> fp32 [2, C]."""
     if mode == 2:

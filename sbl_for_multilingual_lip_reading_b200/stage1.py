@@ -37,13 +37,24 @@ class Stage1Classifier(nn.Module):
         self.encoder_v.load_state_dict(synth.encoder_state_dict(encoder_seed, len(self.encoder_v.layer_stack)))
         return self
 
-    def forward(self, padded_input_visual):
+    def forward(self, padded_input_visual=None, *, u8=None, frames=None, crop=None, flip=None):
         """padded_input_visual: [N,T,88,88] (as train.py:112-116 feeds it) or [N,1,T,88,88] -> (word logits [N,1500],
-        language logits [N,2])."""
-        x = padded_input_visual
-        if x.dim() == 4:
-            x = x.view(x.size(0), -1, x.size(1), x.size(2), x.size(3))          # transformer.py:23
-        feat = self.visual_frontend(x)
+        language logits [N,2]).  Or, instead of it, `u8`: the loader's raw uint8 gray frames [N,T_in,H0,W0], cropped at
+        `crop` (default the centre of 96x96 frames; per-frame offsets from video_frontend.random_crop_offsets),
+        mirrored where `flip` [N] is set (model.train() only) and zero-padded to `frames` frames, all on the GPU
+        (Lipreading.forward_u8).  The uint8 input goes through forward so that DistributedDataParallel, which prepares
+        its gradient all-reduce inside forward, sees the step."""
+        if (padded_input_visual is None) == (u8 is None):
+            raise RuntimeError("Stage1Classifier.forward: pass exactly one of padded_input_visual and u8")
+        if u8 is not None:
+            feat = self.visual_frontend.forward_u8(u8, frames=frames, crop=(4, 4) if crop is None else crop, flip=flip)
+        else:
+            if frames is not None or crop is not None or flip is not None:
+                raise RuntimeError("Stage1Classifier.forward: frames / crop / flip apply to the u8 input only")
+            x = padded_input_visual
+            if x.dim() == 4:
+                x = x.view(x.size(0), -1, x.size(1), x.size(2), x.size(3))          # transformer.py:23
+            feat = self.visual_frontend(x)
         n, t = feat.size(0), feat.size(1)
         out, *_ = self.encoder_v(feat, [t] * n)
         pooled = torch.mean(out, dim=1)

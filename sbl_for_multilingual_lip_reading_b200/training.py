@@ -124,16 +124,39 @@ def _add16(a, b):
 # ------------------------------------------------------------------------------------------------------------------
 # frontend Functions
 # ------------------------------------------------------------------------------------------------------------------
+class StemSource:
+    """What StemFn reads its clip from: the fp32 clip `x` [N,T,88,88] (lut None), or the loader's raw uint8 frames `x`
+    [N,T_in,H0,W0] with the normalisation table, the crop ((y1, x1) or int32 CUDA [N*T_in, 2]), the per-clip flip
+    (int32 CUDA [N] or None) and the padded frame count `t` (ops_train.stem_im2col_u8).  The forward and the wgrad of
+    the backward both build their im2col from it, so a uint8 source keeps no fp32 clip alive between them."""
+    __slots__ = ("x", "lut", "crop", "flip", "t")
+
+    def __init__(self, x, lut=None, crop=None, flip=None, t=None):
+        self.x, self.lut, self.crop, self.flip = x, lut, crop, flip
+        self.t = x.shape[1] if t is None else int(t)
+
+    @classmethod
+    def clip(cls, x):
+        x = x.detach()
+        return cls((x[:, 0] if x.dim() == 5 else x).contiguous().float())
+
+    def im2col(self, transposed=False, ld_out=None):
+        if self.lut is None:
+            return ot.stem_im2col(self.x, transposed=transposed, ld_out=ld_out)
+        return ot.stem_im2col_u8(self.x, self.lut, self.t, self.crop, self.flip, transposed=transposed, ld_out=ld_out)
+
+
 class StemFn(torch.autograd.Function):
     """frontend3D in training mode (video_frontend.py:99-104): Conv3d -> BatchNorm3d(batch stats) -> ReLU -> MaxPool3d,
-    output bf16 NHWC [N*T, 22, 22, 64] (the reference's transpose(1,2).contiguous().view, :113-115, is the layout)."""
+    output bf16 NHWC [N*T, 22, 22, 64] (the reference's transpose(1,2).contiguous().view, :113-115, is the layout).
+    `src`: a StemSource, or the fp32 clip itself."""
 
     @staticmethod
-    def forward(ctx, x, w, gamma, beta, bn):
-        x = x.detach()
-        xs = (x[:, 0] if x.dim() == 5 else x).contiguous().float()
-        n, t = xs.shape[0], xs.shape[1]
-        col = ot.stem_im2col(xs)
+    def forward(ctx, src, w, gamma, beta, bn):
+        if not isinstance(src, StemSource):
+            src = StemSource.clip(src)
+        n, t = src.x.shape[0], src.t
+        col = src.im2col()
         w2d = torch.zeros((64, 256), dtype=F32, device=w.device)
         w2d[:, :245] = w.detach().reshape(64, 245)
         wp = ops.cast_bf16(w2d)
@@ -142,17 +165,19 @@ class StemFn(torch.autograd.Function):
         act, st = bn_forward_train(raw, bn, relu=True)                    # [M, 64] = [F,44,44,64]
         act4 = act.view(n * t, 44, 44, 64)
         out = ot.maxpool_fwd(act4)
-        ctx.save_for_backward(xs, raw, act4, gamma, out)
+        crop = src.crop if torch.is_tensor(src.crop) else None
+        ctx.save_for_backward(src.x, src.lut, crop, src.flip, raw, act4, gamma, out)
         ctx.st = st
+        ctx.t, ctx.crop = src.t, (src.crop if crop is None else None)
         return out
 
     @staticmethod
     def backward(ctx, dout):
-        xs, raw, act4, gamma, pooled = ctx.saved_tensors
+        x, lut, crop, flip, raw, act4, gamma, pooled = ctx.saved_tensors
+        src = StemSource(x, lut, ctx.crop if crop is None else crop, flip, ctx.t)
         dact = ot.maxpool_bwd(act4, pooled, dout.contiguous())
         draw, dgamma, dbeta, _ = bn_backward_train(dact.view(-1, 64), act4.view(-1, 64), raw, ctx.st, gamma)
-        n, t = xs.shape[0], xs.shape[1]
-        dw = _wgrad_gemm(draw, lambda ld: ot.stem_im2col(xs, transposed=True, ld_out=ld), 256)
+        dw = _wgrad_gemm(draw, lambda ld: src.im2col(transposed=True, ld_out=ld), 256)
         dw = dw[:, :245].reshape(64, 1, 5, 7, 7).contiguous()
         return None, dw, dgamma, dbeta, None
 
@@ -218,7 +243,8 @@ class AvgPoolFn(torch.autograd.Function):
 
 
 def frontend_forward_train(fe, x):
-    """Lipreading._frontend_forward in training mode -> fp32 features [N*T, 512] (autograd-connected)."""
+    """Lipreading._frontend_forward in training mode -> fp32 features [N*T, 512] (autograd-connected).  `x`: the fp32
+    clip [N,1,T,88,88] or a StemSource (the loader's raw uint8 frames)."""
     conv, bn = fe.frontend3D[0], fe.frontend3D[1]
     a = StemFn.apply(x, conv.weight, bn.weight, bn.bias, bn)
     for layer in (fe.resnet18.layer1, fe.resnet18.layer2, fe.resnet18.layer3, fe.resnet18.layer4):

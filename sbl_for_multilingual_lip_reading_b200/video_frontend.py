@@ -411,11 +411,8 @@ class Lipreading(nn.Module):
             ev.record(pf_stream)
             torch.cuda.current_stream().wait_event(ev)
 
-    def _u8_prep(self, x_u8, frames, crop):
-        """Checks forward_u8's arguments; returns (x_u8, output frames, the prep closure for _frontend_forward)."""
-        if self.training:
-            raise RuntimeError("Lipreading.forward_u8 (libsblk) is the evaluation / serving input path; training runs "
-                               "through forward() on the loader's augmented fp32 clips")
+    def _u8_input(self, x_u8, frames):
+        """Checks the raw frames and the frame count of forward_u8; returns (x_u8, output frames, normalisation table)."""
         if not torch.is_tensor(x_u8) or x_u8.dtype != torch.uint8 or x_u8.dim() != 4:
             raise RuntimeError("forward_u8 expects a uint8 tensor [N, T, H0, W0]")
         if not x_u8.is_cuda:
@@ -429,6 +426,15 @@ class Lipreading(nn.Module):
         if lut is None:
             from . import synth
             lut = self._lut[key] = synth.normalize_lut().to(x_u8.device)
+        return x_u8, t_out, lut
+
+    def _u8_prep(self, x_u8, frames, crop):
+        """Checks forward_u8's arguments for the evaluation path; returns (x_u8, output frames, the prep closure for
+        _frontend_forward)."""
+        if self.training:
+            raise RuntimeError("Lipreading: the evaluation path's uint8 input prep runs in model.eval(); in model.train() "
+                               "call forward_u8 (or forward) directly")
+        x_u8, t_out, lut = self._u8_input(x_u8, frames)
         if torch.is_tensor(crop):
             crop = crop.to(device=x_u8.device, dtype=torch.int32).contiguous()
 
@@ -438,13 +444,35 @@ class Lipreading(nn.Module):
             return ops.prep_clip_u8(xs, lut, t_out, crop)
         return x_u8, t_out, prep
 
-    def forward_u8(self, x_u8, frames=None, crop=(4, 4)):
+    def forward_u8(self, x_u8, frames=None, crop=(4, 4), flip=None):
         """Fused input pipeline (SURVEY.md §8f.3): raw uint8 gray frames [N, T_in, H0, W0] (the loader's .npy layout,
         H0 = W0 = 96 for LRW) -> the same [N, frames, 512] features `forward` returns for the clip the reference loader
         would have built on the CPU (/255, ColorNormalize, 88x88 crop at `crop`, zero-padding to `frames` frames:
-        data_gen.py:122-125,276-296; cvtransforms.py:7-48).  `crop`: (y1, x1) or an int32 CUDA tensor [N*T_in, 2] of
-        per-frame offsets (RandomCrop).  Bit-identical to forward(reference-normalised fp32 clip); 4x fewer host->device
-        bytes."""
+        data_gen.py:122-125,276-296; cvtransforms.py:7-48).  `crop`: (y1, x1) or an int32 tensor [N*T_in, 2] of
+        per-frame offsets (RandomCrop; random_crop_offsets draws them).  Bit-identical to forward(reference-normalised
+        fp32 clip); 4x fewer host->device bytes.
+
+        model.train(): the training path of `forward` (batch-statistics BatchNorm, running-stat updates, autograd) with
+        the stem's im2col built straight from the frames (ops_train.stem_im2col_u8).  `flip`: None or a bool / integer
+        tensor [N]; a nonzero entry mirrors that clip's crop horizontally (torch.flip(clip, dims=[-1])).  Per-frame
+        offsets given on the CPU are range-checked; offsets already on the GPU are clamped into the frame.
+        model.eval(): test-time input is not mirrored, so `flip` is rejected."""
+        if self.training:
+            from . import ops_train, training
+            x_u8, t_out, lut = self._u8_input(x_u8, frames)
+            n, t_in, h0, w0 = x_u8.shape
+            if torch.is_tensor(crop):
+                crop = ops_train.crop_offsets_to(crop, n * t_in, h0, w0, x_u8.device)
+            else:
+                crop = (int(crop[0]), int(crop[1]))
+            if flip is not None:
+                flip = ops_train.flip_flags_to(flip, n, x_u8.device)
+            src = training.StemSource(x_u8, lut, crop, flip, t_out)
+            feat = training.frontend_forward_train(self, src)
+            feat = F.dropout(feat, p=0.5)  # reference :122 (functional default training=True); torch autograd
+            return feat.view(-1, t_out, self.inputDim)
+        if flip is not None:
+            raise RuntimeError("forward_u8: flip is a training augmentation; the evaluation path does not mirror clips")
         x_u8, t_out, prep = self._u8_prep(x_u8, frames, crop)
         feat = self._frontend_forward(x_u8, prep=prep, frames=t_out)
         if self.always_on_dropout:
@@ -473,6 +501,22 @@ class Lipreading(nn.Module):
         if self.always_on_dropout:
             feat = F.dropout(feat, p=0.5)  # functional default training=True, exactly as reference :122
         return feat.view(-1, frameLen, self.inputDim)
+
+
+def random_crop_offsets(n, t_in, h0=96, w0=96, rng=None):
+    """Per-frame 88x88 crop offsets drawn the way the reference loader's RandomCrop draws them (cvtransforms.py:23-33):
+    for every frame of every clip in order, x1 = randint(0, w0 - 88) then y1 = randint(0, h0 - 88), from `rng` (a
+    random.Random) or the module `random`.  -> int32 CPU tensor [n * t_in, 2] of (y1, x1), the `crop` of forward_u8."""
+    import random
+    rng = random if rng is None else rng
+    if h0 < 88 or w0 < 88:
+        raise ValueError(f"random_crop_offsets: frames of {h0}x{w0} are smaller than the 88x88 crop")
+    offs = []
+    for _ in range(int(n) * int(t_in)):
+        x1 = rng.randint(0, w0 - 88)
+        y1 = rng.randint(0, h0 - 88)
+        offs.append((y1, x1))
+    return torch.tensor(offs, dtype=torch.int32).view(-1, 2)
 
 
 device = torch.device('cuda' if torch.cuda.is_available() else 'cpu')  # reference :174
