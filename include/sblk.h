@@ -375,6 +375,22 @@ int sblk_attention_train_fwd(const void* qkv, const float* drop, float* probs, v
                              int T, int H, float scale, void* stream);
 int sblk_attention_train_bwd(const void* qkv, const float* drop, const float* probs, const void* dout, void* dqkv,
                              const int* lengths, int N, int T, int H, float scale, void* stream);
+/* Training-mode scaled-dot-product attention with separate query and key / value sources (Lq <= 64, Lk <= 64, d_k = 64,
+ * head h at columns h*64): Q rows (b*Lq + i)*ldq, K / V rows (b*Lk + j)*ldk|ldv (enc16); mask = causal (key j > query
+ * i) and / or key lengths klens[b] (NULL = all Lk); drop = dropout factor mask/(1-p) fp32 [H*N, Lq, Lk] applied to the
+ * probabilities, or NULL; probs fp32 [H*N, Lq, Lk] (index h*N + b; written by fwd, read by bwd).  fwd: out enc16 rows
+ * (b*Lq + i)*ldo.  bwd: dout bf16 rows with pitch lddo -> dq (pitch lddq), dk / dv (rows (b*Lk + j)*lddk|lddv), bf16,
+ * every output written (dk / dv may be the two halves of one [N*Lk, 2*H*64] buffer, dq / dk / dv the thirds of one
+ * [N*T, 3*H*64] buffer).  (The encoder's packed self-attention stays on sblk_attention_train_*: same values, faster
+ * on its shape.)
+ * replaces: ScaledDotProductAttention.forward + autograd in DecoderLayer, attention.py:72-83 */
+int sblk_xattention_train_fwd(const void* q, const void* k, const void* v, const float* drop, float* probs, void* out,
+                              const int* klens, int ldq, int ldk, int ldv, int ldo, int N, int Lq, int Lk, int H,
+                              int causal, float scale, void* stream);
+int sblk_xattention_train_bwd(const void* q, const void* k, const void* v, const float* drop, const float* probs,
+                              const void* dout, void* dq, void* dk, void* dv, const int* klens, int ldq, int ldk,
+                              int ldv, int lddo, int lddq, int lddk, int lddv, int N, int Lq, int Lk, int H, int causal,
+                              float scale, void* stream);
 
 /* ---- SBL bidirectional decoder glue (SURVEY.md 8f.1) ----------------------------------------------------------------
  * The decoder's projections, FFNs and residual + LayerNorms run on the encoder entry points above (sblk_gemm_fwd,
@@ -397,6 +413,16 @@ int sblk_embed_pe_fwd(const void* tokens_i64, int ld_tokens, const float* emb, c
  * replaces: decoder.py:336-346,358-362 */
 int sblk_bidir_mix_fwd(const float* l2r, const float* r2l, float* l2r_out, float* r2l_out, void* l2r_16, void* r2l_16,
                        int N, int L, int D, void* stream);
+/* Training path: backward of sblk_bidir_mix_fwd, fp32 [N, L, D], from the gradients g_l2r / g_r2l of its outputs:
+ * d_l2r = g_l2r + flip_L(g_r2l); d_r2l = g_r2l + (flip_L(g_l2r) + g_r2l) (autograd's order through the aliased loops,
+ * bit for bit).  16-byte aligned, no aliasing. */
+int sblk_bidir_mix_bwd(const float* g_l2r, const float* g_r2l, float* d_l2r, float* d_r2l, int N, int L, int D,
+                       void* stream);
+/* Training path: backward of sblk_embed_pe_fwd's embedding term.  demb fp32 [vocab, D] = scale * sum of dx fp32 [rows, D]
+ * over the rows whose token id (same layout and clamping as sblk_embed_pe_fwd) is v; overwritten, rows no token
+ * selects are zero.  Deterministic: fixed summation order, no atomics.  16-byte aligned dx / demb, D % 4 == 0. */
+int sblk_embed_bwd(const void* tokens_i64, int ld_tokens, const float* dx, float* demb, int rows, int L, int D,
+                   int vocab, float scale, void* stream);
 
 /* ---- one-shot all-gather of the per-GPU outputs over NVLink / NVSwitch peer memory (one process per GPU) ----------
  * replaces: nn.DataParallel's gather of the replicas' outputs, SBL/train.py:114-115.

@@ -99,9 +99,13 @@ SIGNATURES = {
     "sblk_ln_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _f, _vp]),
     "sblk_attention_train_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _vp]),
     "sblk_attention_train_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _vp]),
+    "sblk_xattention_train_fwd": (_i, [_vp] * 7 + [_i] * 9 + [_f, _vp]),
+    "sblk_xattention_train_bwd": (_i, [_vp] * 10 + [_i] * 12 + [_f, _vp]),
     "sblk_xattention_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _vp]),
     "sblk_embed_pe_fwd": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _f, _vp]),
     "sblk_bidir_mix_fwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    "sblk_bidir_mix_bwd": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    "sblk_embed_bwd": (_i, [_vp, _i, _vp, _vp, _i, _i, _i, _i, _f, _vp]),
     "sblk_encoder_stack_workspace_bytes": (_ll, [_i, _i, _i]),
     "sblk_encoder_stack_fwd": (_i, [ctypes.POINTER(EncoderStackArgs), _vp]),
 }

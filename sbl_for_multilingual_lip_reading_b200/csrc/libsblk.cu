@@ -142,6 +142,8 @@ int ensure_init(int* num_sms_out) {
     if ((rc = set_smem(sblk::attention_kernel<16>, 100 * 1024))) return rc;
     if ((rc = set_smem(sblk::attn_train_kernel<false>, 104 * 1024))) return rc;
     if ((rc = set_smem(sblk::attn_train_kernel<true>, 104 * 1024))) return rc;
+    if ((rc = set_smem(sblk::xattn_train_kernel<false>, 104 * 1024))) return rc;
+    if ((rc = set_smem(sblk::xattn_train_kernel<true>, 104 * 1024))) return rc;
     if ((rc = set_smem(sblk::xattention_kernel, 100 * 1024))) return rc;
     st.ready = true;
   }
@@ -1529,6 +1531,53 @@ int sblk_attention_train_bwd(const void* qkv, const float* drop, const float* pr
   return attn_train_impl(true, qkv, drop, const_cast<float*>(probs), nullptr, dout, dqkv, lengths, N, T, H, scale, stream);
 }
 
+static int xattn_train_impl(bool bwd, const char* name, sblk::XAttnTrainParams& p, void* stream) {
+  int sms, rc;
+  if ((rc = ensure_init(&sms))) return rc;
+  if (!p.q || !p.k || !p.v || !p.probs || (!bwd && !p.out) || (bwd && (!p.dout || !p.dq || !p.dk || !p.dv)))
+    return fail(-1, "%s: null pointer", name);
+  if (p.N <= 0 || p.H <= 0 || p.Lq <= 0 || p.Lq > 64 || p.Lk <= 0 || p.Lk > 64)
+    return fail(-1, "%s: bad shape N=%d H=%d Lq=%d Lk=%d (training attention: Lq <= 64, Lk <= 64)", name, p.N, p.H, p.Lq, p.Lk);
+  const int hd = p.H * 64;
+  if (p.ldq < hd || p.ldk < hd || p.ldv < hd || (!bwd && p.ldo < hd) ||
+      (bwd && (p.lddo < hd || p.lddq < hd || p.lddk < hd || p.lddv < hd)))
+    return fail(-1, "%s: row pitches must cover H*64 features", name);
+  p.causal = p.causal ? 1 : 0;
+  p.fp16 = SBLK_ENC_FP16 ? 1 : 0;
+  const size_t Lq = p.Lq, Lk = p.Lk;
+  const size_t fl = (Lq + 2 * Lk) * 65 + Lq * (Lk + 1) + (bwd ? Lq * 65 + Lq * (Lk + 1) : 0);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  if (bwd)
+    return launch(sblk::xattn_train_kernel<true>, dim3(p.N * p.H), dim3(256), fl * sizeof(float), s, false,
+                  "xattn_train_kernel<bwd>", p);
+  return launch(sblk::xattn_train_kernel<false>, dim3(p.N * p.H), dim3(256), fl * sizeof(float), s, false,
+                "xattn_train_kernel<fwd>", p);
+}
+
+int sblk_xattention_train_fwd(const void* q, const void* k, const void* v, const float* drop, float* probs, void* out,
+                              const int* klens, int ldq, int ldk, int ldv, int ldo, int N, int Lq, int Lk, int H,
+                              int causal, float scale, void* stream) {
+  sblk::XAttnTrainParams p = {};
+  p.q = static_cast<const uint16_t*>(q); p.k = static_cast<const uint16_t*>(k); p.v = static_cast<const uint16_t*>(v);
+  p.drop = drop; p.probs = probs; p.out = static_cast<uint16_t*>(out); p.klens = klens;
+  p.ldq = ldq; p.ldk = ldk; p.ldv = ldv; p.ldo = ldo;
+  p.N = N; p.Lq = Lq; p.Lk = Lk; p.H = H; p.causal = causal; p.scale = scale;
+  return xattn_train_impl(false, "sblk_xattention_train_fwd", p, stream);
+}
+
+int sblk_xattention_train_bwd(const void* q, const void* k, const void* v, const float* drop, const float* probs,
+                              const void* dout, void* dq, void* dk, void* dv, const int* klens, int ldq, int ldk,
+                              int ldv, int lddo, int lddq, int lddk, int lddv, int N, int Lq, int Lk, int H, int causal,
+                              float scale, void* stream) {
+  sblk::XAttnTrainParams p = {};
+  p.q = static_cast<const uint16_t*>(q); p.k = static_cast<const uint16_t*>(k); p.v = static_cast<const uint16_t*>(v);
+  p.drop = drop; p.probs = const_cast<float*>(probs); p.dout = static_cast<const uint16_t*>(dout);
+  p.dq = static_cast<uint16_t*>(dq); p.dk = static_cast<uint16_t*>(dk); p.dv = static_cast<uint16_t*>(dv);
+  p.klens = klens; p.ldq = ldq; p.ldk = ldk; p.ldv = ldv; p.lddo = lddo; p.lddq = lddq; p.lddk = lddk; p.lddv = lddv;
+  p.N = N; p.Lq = Lq; p.Lk = Lk; p.H = H; p.causal = causal; p.scale = scale;
+  return xattn_train_impl(true, "sblk_xattention_train_bwd", p, stream);
+}
+
 
 // =====================================================================================================================
 // SBL bidirectional decoder glue (row f.1): see include/sblk.h "decoder" section, sblk_decoder.cuh
@@ -1577,6 +1626,34 @@ int sblk_bidir_mix_fwd(const float* l2r, const float* r2l, float* l2r_out, float
   return launch(sblk::bidir_mix_kernel, dim3(elementwise_grid(static_cast<long long>(N) * L * (D / 4), 256, sms)), dim3(256), 0,
                 static_cast<cudaStream_t>(stream), false, "bidir_mix_kernel", l2r, r2l, l2r_out, r2l_out,
                 static_cast<uint16_t*>(l2r_16), static_cast<uint16_t*>(r2l_16), N, L, D, SBLK_ENC_FP16 ? 1 : 0);
+}
+
+int sblk_bidir_mix_bwd(const float* g_l2r, const float* g_r2l, float* d_l2r, float* d_r2l, int N, int L, int D,
+                       void* stream) {
+  int sms, rc;
+  if ((rc = ensure_init(&sms))) return rc;
+  if (!g_l2r || !g_r2l || !d_l2r || !d_r2l) return fail(-1, "sblk_bidir_mix_bwd: null pointer");
+  if (N <= 0 || L <= 0 || D <= 0 || D % 4 != 0) return fail(-1, "sblk_bidir_mix_bwd: bad shape N=%d L=%d D=%d", N, L, D);
+  if (g_l2r == d_l2r || g_l2r == d_r2l || g_r2l == d_l2r || g_r2l == d_r2l || d_l2r == d_r2l)
+    return fail(-1, "sblk_bidir_mix_bwd: outputs must not alias inputs or each other");
+  if (!aligned16(g_l2r) || !aligned16(g_r2l) || !aligned16(d_l2r) || !aligned16(d_r2l))
+    return fail(-1, "sblk_bidir_mix_bwd: pointers must be 16-byte aligned");
+  return launch(sblk::bidir_mix_bwd_kernel, dim3(elementwise_grid(static_cast<long long>(N) * L * (D / 4), 256, sms)),
+                dim3(256), 0, static_cast<cudaStream_t>(stream), false, "bidir_mix_bwd_kernel", g_l2r, g_r2l, d_l2r, d_r2l,
+                N, L, D);
+}
+
+int sblk_embed_bwd(const void* tokens_i64, int ld_tokens, const float* dx, float* demb, int rows, int L, int D,
+                   int vocab, float scale, void* stream) {
+  int sms, rc;
+  if ((rc = ensure_init(&sms))) return rc;
+  if (!tokens_i64 || !dx || !demb) return fail(-1, "sblk_embed_bwd: null pointer");
+  if (rows <= 0 || L <= 0 || rows % L != 0 || D <= 0 || D % 4 != 0 || vocab <= 0 || ld_tokens < L)
+    return fail(-1, "sblk_embed_bwd: bad shape rows=%d L=%d D=%d vocab=%d ld_tokens=%d", rows, L, D, vocab, ld_tokens);
+  if (!aligned16(dx) || !aligned16(demb)) return fail(-1, "sblk_embed_bwd: pointers must be 16-byte aligned");
+  return launch(sblk::embed_bwd_kernel, dim3(vocab, (D / 4 + 31) / 32), dim3(256), 0, static_cast<cudaStream_t>(stream),
+                false, "embed_bwd_kernel", static_cast<const long long*>(tokens_i64), ld_tokens, dx, demb, rows, L, D, vocab,
+                scale);
 }
 
 }  // extern "C"

@@ -2,7 +2,9 @@
 //   * general multi-head attention for short sequences with separate Q and K/V sources (decoder self-attention with or
 //     without the subsequent mask, decoder-encoder attention over cached encoder keys / values),
 //   * token embedding + positional encoding,
-//   * the synchronous bidirectional mixing of the two directions' hidden states.
+//   * the synchronous bidirectional mixing of the two directions' hidden states,
+//   * for the training path: the backward of the mixing and of the embedding (the attention's training forward /
+//     backward is xattn_train_kernel in sblk_train.cuh, shared with the encoder).
 // Reference: SBL/transformer/decoder.py:301-385 (recognize_beam), :79-191 (forward), DecoderLayer :388-408,
 //            attention.py:32-83, module.py:8-32, utils.py:116-124 (get_subsequent_mask).
 // Every projection / FFN GEMM and every residual + LayerNorm of the decoder runs on the encoder's tcgen05 kernels
@@ -154,6 +156,82 @@ bidir_mix_kernel(const float* __restrict__ l2r, const float* __restrict__ r2l, f
     w.x = fp16 ? pack_f16x2(ro.x, ro.y) : pack_bf16x2(ro.x, ro.y);
     w.y = fp16 ? pack_f16x2(ro.z, ro.w) : pack_bf16x2(ro.z, ro.w);
     reinterpret_cast<uint2*>(r2l_16)[i] = w;
+  }
+}
+
+// ----------------------------------------------------------------------------------------------------------------
+// Training-path backward kernels of the decoder glue.
+// ----------------------------------------------------------------------------------------------------------------
+// Backward of bidir_mix_kernel, fp32, given the gradients g_a / g_b of l2r' / r2l':
+//   d_l2r[n, i] = g_a[n, i] + g_b[n, L-1-i]
+//   d_r2l[n, i] = g_b[n, i] + (g_a[n, L-1-i] + g_b[n, i])
+// The second line is the order in which autograd through the aliased loops adds the two paths into r2l (the direct one
+// and the one through l2r'[L-1-i]); g_a + 2 g_b would round differently.  __fadd_rn: no contraction, bit-exact.
+__global__ void __launch_bounds__(256)
+bidir_mix_bwd_kernel(const float* __restrict__ ga, const float* __restrict__ gb, float* __restrict__ d_l2r,
+                     float* __restrict__ d_r2l, int N, int L, int D) {
+  const int d4 = D / 4;
+  const long long total = static_cast<long long>(N) * L * d4;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int c = static_cast<int>(i % d4);
+    const long long row = i / d4;
+    const int pos = static_cast<int>(row % L);
+    const long long n = row / L;
+    const long long mirror = (n * L + (L - 1 - pos)) * d4 + c;
+    const float4 a = __ldg(reinterpret_cast<const float4*>(ga) + i);
+    const float4 b = __ldg(reinterpret_cast<const float4*>(gb) + i);
+    const float4 am = __ldg(reinterpret_cast<const float4*>(ga) + mirror);
+    const float4 bm = __ldg(reinterpret_cast<const float4*>(gb) + mirror);
+    reinterpret_cast<float4*>(d_l2r)[i] = make_float4(__fadd_rn(a.x, bm.x), __fadd_rn(a.y, bm.y), __fadd_rn(a.z, bm.z),
+                                                      __fadd_rn(a.w, bm.w));
+    reinterpret_cast<float4*>(d_r2l)[i] = make_float4(
+        __fadd_rn(b.x, __fadd_rn(am.x, b.x)), __fadd_rn(b.y, __fadd_rn(am.y, b.y)),
+        __fadd_rn(b.z, __fadd_rn(am.z, b.z)), __fadd_rn(b.w, __fadd_rn(am.w, b.w)));
+  }
+}
+
+// Embedding backward: demb[v, :] = scale * sum of dx[r, :] over the rows r whose (clamped, as in embed_pe_kernel) token
+// id is v, rows in the token layout of embed_pe_kernel.  Deterministic without atomics: CTA (v, 128-column slice); warp
+// s adds the rows r = s, s + 8, ... in order (lane = 4 columns), the 8 warp sums are then added in warp order.  Every
+// CTA scans the token ids (staged 1024 at a time in shared memory) and reads only its own rows of dx.
+constexpr int kEmbedBwdIds = 1024;
+__global__ void __launch_bounds__(256)
+embed_bwd_kernel(const long long* __restrict__ tok, int ld_tok, const float* __restrict__ dx, float* __restrict__ demb,
+                 int rows, int L, int D, int vocab, float scale) {
+  __shared__ int ids[kEmbedBwdIds];
+  __shared__ float4 part[8][32];
+  const int v = blockIdx.x;
+  const int lane = threadIdx.x & 31, slice = threadIdx.x >> 5;
+  const int d4 = D / 4;
+  const int c4 = blockIdx.y * 32 + lane;
+  float4 acc = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+  for (int r0 = 0; r0 < rows; r0 += kEmbedBwdIds) {
+    const int nr = min(kEmbedBwdIds, rows - r0);
+    for (int i = threadIdx.x; i < nr; i += blockDim.x) {
+      const int r = r0 + i;
+      long long t = __ldg(tok + static_cast<long long>(r / L) * ld_tok + (r % L));
+      t = t < 0 ? 0 : (t >= vocab ? vocab - 1 : t);
+      ids[i] = static_cast<int>(t);
+    }
+    __syncthreads();
+    if (c4 < d4) {
+      for (int i = slice; i < nr; i += 8) {
+        if (ids[i] != v) continue;
+        const float4 g = __ldg(reinterpret_cast<const float4*>(dx) + static_cast<long long>(r0 + i) * d4 + c4);
+        acc.x += g.x; acc.y += g.y; acc.z += g.z; acc.w += g.w;
+      }
+    }
+    __syncthreads();
+  }
+  part[slice][lane] = acc;
+  __syncthreads();
+  if (slice == 0 && c4 < d4) {
+    float4 s = part[0][lane];
+#pragma unroll
+    for (int k = 1; k < 8; ++k) { s.x += part[k][lane].x; s.y += part[k][lane].y; s.z += part[k][lane].z; s.w += part[k][lane].w; }
+    reinterpret_cast<float4*>(demb)[static_cast<long long>(v) * d4 + c4] =
+        make_float4(s.x * scale, s.y * scale, s.z * scale, s.w * scale);
   }
 }
 

@@ -933,4 +933,148 @@ attn_train_kernel(const AttnTrainParams p) {
   }
 }
 
+// ----------------------------------------------------------------------------------------------------------------
+// Scaled-dot-product attention, TRAINING forward + backward for short sequences (Lq, Lk <= 64, d_k = 64), with separate
+// query and key / value sources and an optional causal mask: the decoder's self-attention over the prefix (Lq = Lk = L,
+// causal in its first layer) and its decoder-encoder attention (Lq = L, Lk = t_enc).  One CTA per (clip, head), fp32 math in shared memory.  The encoder
+// keeps attn_train_kernel above: this kernel computes the same values on its shape (bit for bit) but measured 0.8 %
+// slower there (DESIGN.md §9).
+// attention.py:72-83 with the dropout on the probabilities made explicit: `drop` = mask / (1 - p) drawn by the caller
+// ([H*N, Lq, Lk] fp32, or nullptr).
+//   forward : P = softmax(Q K^T * scale, keys j >= klens[b] and (causal) j > i masked) ; O = (P * drop) V
+//             -> O enc16, P fp32 (saved)
+//   backward: dV = (P*drop)^T dO ; dPd = dO V^T ; dP = dPd * drop ; dS = P * (dP - rowsum(dP * P)) * scale ;
+//             dQ = dS K ; dK = dS^T Q                                                  -> dQ, dK, dV bf16
+// Q rows at q + (b*Lq + i)*ldq + h*64, K / V rows at k|v + (b*Lk + j)*ldk|ldv + h*64 (enc16); O / dO / dQ rows with the
+// query pitches ldo / lddo / lddq, dK / dV rows with lddk / lddv.  probs / drop index (h*N + b) like the reference.
+// ----------------------------------------------------------------------------------------------------------------
+struct XAttnTrainParams {
+  const uint16_t* q;     // enc16
+  const uint16_t* k;
+  const uint16_t* v;
+  const float* drop;     // or nullptr
+  float* probs;          // forward: written; backward: read
+  uint16_t* out;         // forward: O enc16
+  const uint16_t* dout;  // backward: dO bf16
+  uint16_t* dq;          // backward: bf16
+  uint16_t* dk;
+  uint16_t* dv;
+  const int* klens;      // [N] valid keys or nullptr
+  int ldq, ldk, ldv, ldo, lddo, lddq, lddk, lddv;
+  int N, Lq, Lk, H, causal;
+  float scale;
+  int fp16;              // q / k / v / out storage is IEEE fp16 (else bf16)
+};
+
+template <bool BWD>
+__global__ void __launch_bounds__(256)
+xattn_train_kernel(const XAttnTrainParams p) {
+  extern __shared__ float sm[];
+  const int Lq = p.Lq, Lk = p.Lk, D = 64;
+  const int b = blockIdx.x / p.H, h = blockIdx.x - b * p.H;
+  float* sQ = sm;                        // [Lq][65]
+  float* sK = sQ + Lq * 65;              // [Lk][65]
+  float* sV = sK + Lk * 65;              // [Lk][65]
+  float* sP = sV + Lk * 65;              // [Lq][Lk+1]
+  float* sG = sP + Lq * (Lk + 1);        // BWD: dO [Lq][65]
+  float* sS = sG + (BWD ? Lq * 65 : 0);  // BWD: dS [Lq][Lk+1]
+  const int klen = (p.klens != nullptr) ? min(max(__ldg(p.klens + b), 0), Lk) : Lk;
+  for (int i = threadIdx.x; i < Lq * D; i += blockDim.x) {
+    const int t = i >> 6, d = i & 63;
+    const size_t row = static_cast<size_t>(b) * Lq + t;
+    sQ[t * 65 + d] = ld16(p.q + row * p.ldq + h * D + d, p.fp16);
+    if (BWD) sG[t * 65 + d] = ld16(p.dout + row * p.lddo + h * D + d, 0);
+  }
+  for (int i = threadIdx.x; i < Lk * D; i += blockDim.x) {
+    const int t = i >> 6, d = i & 63;
+    const size_t row = static_cast<size_t>(b) * Lk + t;
+    sK[t * 65 + d] = ld16(p.k + row * p.ldk + h * D + d, p.fp16);
+    sV[t * 65 + d] = ld16(p.v + row * p.ldv + h * D + d, p.fp16);
+  }
+  float* probs = p.probs + (static_cast<size_t>(h) * p.N + b) * Lq * Lk;
+  const float* drop = p.drop != nullptr ? p.drop + (static_cast<size_t>(h) * p.N + b) * Lq * Lk : nullptr;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+  __syncthreads();
+  if (!BWD) {
+    // S = Q K^T * scale, masked; one warp per query row: softmax with shuffles
+    for (int qi = warp; qi < Lq; qi += nw) {
+      float sc[2] = {-INFINITY, -INFINITY};
+#pragma unroll
+      for (int e = 0; e < 2; ++e) {
+        const int kj = lane + 32 * e;
+        if (kj < klen && !(p.causal && kj > qi)) {
+          float a = 0.0f;
+          for (int d = 0; d < D; ++d) a += sQ[qi * 65 + d] * sK[kj * 65 + d];
+          sc[e] = a * p.scale;
+        }
+      }
+      float mx = fmaxf(sc[0], sc[1]);
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+      float e0 = __expf(sc[0] - mx), e1 = __expf(sc[1] - mx);   // all-masked row: NaN like the reference softmax
+      float sum = e0 + e1;
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+      const float inv = 1.0f / sum;
+      if (lane < Lk) { sP[qi * (Lk + 1) + lane] = e0 * inv; probs[qi * Lk + lane] = e0 * inv; }
+      if (lane + 32 < Lk) { sP[qi * (Lk + 1) + lane + 32] = e1 * inv; probs[qi * Lk + lane + 32] = e1 * inv; }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < Lq * D; i += blockDim.x) {
+      const int t = i >> 6, d = i & 63;
+      float a = 0.0f;
+      for (int j = 0; j < Lk; ++j) {
+        float pj = sP[t * (Lk + 1) + j];
+        if (drop != nullptr) pj *= __ldg(drop + t * Lk + j);
+        a += pj * sV[j * 65 + d];
+      }
+      const uint32_t w = p.fp16 ? pack_f16x2(a, 0.0f) : pack_bf16x2(a, 0.0f);
+      p.out[(static_cast<size_t>(b) * Lq + t) * p.ldo + h * D + d] = static_cast<uint16_t>(w & 0xFFFFu);
+    }
+  } else {
+    for (int i = threadIdx.x; i < Lq * Lk; i += blockDim.x) sP[(i / Lk) * (Lk + 1) + (i % Lk)] = __ldg(probs + i);
+    __syncthreads();
+    // dP = (dO V^T) * drop ; row statistics ; dS
+    for (int qi = warp; qi < Lq; qi += nw) {
+      float dp[2] = {0.0f, 0.0f}, pv[2] = {0.0f, 0.0f};
+#pragma unroll
+      for (int e = 0; e < 2; ++e) {
+        const int kj = lane + 32 * e;
+        if (kj < Lk) {
+          float a = 0.0f;
+          for (int d = 0; d < D; ++d) a += sG[qi * 65 + d] * sV[kj * 65 + d];
+          if (drop != nullptr) a *= __ldg(drop + qi * Lk + kj);
+          dp[e] = a;
+          pv[e] = sP[qi * (Lk + 1) + kj];
+        }
+      }
+      float dot = dp[0] * pv[0] + dp[1] * pv[1];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
+      if (lane < Lk) sS[qi * (Lk + 1) + lane] = pv[0] * (dp[0] - dot) * p.scale;
+      if (lane + 32 < Lk) sS[qi * (Lk + 1) + lane + 32] = pv[1] * (dp[1] - dot) * p.scale;
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < Lq * D; i += blockDim.x) {   // dQ[t] = sum_j dS[t][j] K[j]
+      const int t = i >> 6, d = i & 63;
+      float aq = 0.0f;
+      for (int j = 0; j < Lk; ++j) aq += sS[t * (Lk + 1) + j] * sK[j * 65 + d];
+      p.dq[(static_cast<size_t>(b) * Lq + t) * p.lddq + h * D + d] = static_cast<uint16_t>(pack_bf16x2(aq, 0.0f) & 0xFFFFu);
+    }
+    for (int i = threadIdx.x; i < Lk * D; i += blockDim.x) {   // dK[t] = sum_j dS[j][t] Q[j], dV[t] = sum_j (P*drop)[j][t] dO[j]
+      const int t = i >> 6, d = i & 63;
+      float ak = 0.0f, av = 0.0f;
+      for (int j = 0; j < Lq; ++j) {
+        ak += sS[j * (Lk + 1) + t] * sQ[j * 65 + d];
+        float pj = sP[j * (Lk + 1) + t];
+        if (drop != nullptr) pj *= __ldg(drop + j * Lk + t);
+        av += pj * sG[j * 65 + d];
+      }
+      const size_t row = static_cast<size_t>(b) * Lk + t;
+      p.dk[row * p.lddk + h * D + d] = static_cast<uint16_t>(pack_bf16x2(ak, 0.0f) & 0xFFFFu);
+      p.dv[row * p.lddv + h * D + d] = static_cast<uint16_t>(pack_bf16x2(av, 0.0f) & 0xFFFFu);
+    }
+  }
+}
+
 }  // namespace sblk

@@ -18,8 +18,10 @@ as they call the reference class.  Submodules are parameter holders; the arithme
   The encoder-side K / V projections of all 12 decoder layers are computed ONCE per call (the reference recomputes them
   at each of the 16 steps).  Operands are enc16 (fp16) with fp32 accumulation, LayerNorm, softmax and residual streams.
 
-Evaluation only: the training-mode decoder (backward through 16 x 2 x 6 re-run layers) is the reference's; in
-`model.train()` this class raises and `dropin.patch_reference(..., decoder=False)` keeps the reference decoder.
+Training: in `model.train()`, `forward` runs the same 16 steps as autograd Functions over libsblk forward and backward
+kernels (training.decoder_forward_train, DESIGN.md §9): the logits reach every decoder parameter and the encoder
+outputs.  It reads the live parameters (no packed cache), so an optimizer step is seen by the next call.  Greedy
+decoding (`recognize_beam`) stays an evaluation feature.
 """
 from __future__ import annotations
 
@@ -139,16 +141,18 @@ class Decoder(nn.Module):
         self._packed = None
         self._plans = {}
 
-    def _check(self, enc):
-        if self.training:
-            raise RuntimeError("Decoder (libsblk): evaluation only (greedy decode / teacher-forced forward); training the "
-                               "decoder uses the reference class — dropin.patch_reference(ref_dir, decoder=False)")
+    def _check(self, enc, train_forward=False):
+        if self.training and not train_forward:
+            raise RuntimeError("Decoder (libsblk): greedy decoding (recognize_beam) is an evaluation feature; call "
+                               "model.eval() first (in training mode only forward is available)")
         if self.d_model != 512 or self.d_k != 64 or self.d_v != 64 or self.n_head != 8 or self.d_word_vec != 512:
             raise RuntimeError("Decoder (libsblk): only d_model = d_word_vec = 512, 8 heads of 64 are implemented")
         if not enc.is_cuda:
             raise RuntimeError("Decoder (libsblk) runs on a B200 CUDA device only; no CPU fallback exists")
-        if enc.dim() != 3 or enc.size(2) != 512 or enc.size(1) > 128:
-            raise RuntimeError(f"Decoder (libsblk): encoder outputs must be [N, T <= 128, 512], got {tuple(enc.shape)}")
+        t_max = 64 if train_forward else 128      # the training attention kernel holds <= 64 keys
+        if enc.dim() != 3 or enc.size(2) != 512 or enc.size(1) > t_max:
+            raise RuntimeError(f"Decoder (libsblk): encoder outputs must be [N, T <= {t_max}, 512]"
+                               f"{' in training' if train_forward else ''}, got {tuple(enc.shape)}")
 
     def _pack_layer(self, lyr):
         a, c, f = lyr.slf_attn, lyr.enc_attn, lyr.pos_ffn
@@ -366,7 +370,13 @@ class Decoder(nn.Module):
     def forward(self, padded_input_l2r, padded_input_r2l, encoder_outputs, encoder_input_lengths, return_attns=False):
         """Sampled teacher forcing, reference decoder.py:79-191: 16 steps, each feeding either the model's own argmax or
         the gold token (`random.random() > 0.5`, the reference's coin) -> (logits_l2r [N,16,58], gold_l2r, logits_r2l,
-        gold_r2l)."""
+        gold_r2l).  In training mode the logits are autograd-connected (training.decoder_forward_train)."""
+        if self.training:
+            if return_attns:
+                raise RuntimeError("Decoder (libsblk): return_attns is not implemented in training mode")
+            self._check(encoder_outputs, train_forward=True)
+            from .training import decoder_forward_train
+            return decoder_forward_train(self, padded_input_l2r, padded_input_r2l, encoder_outputs)
         ys_in_pad_l2r, ys_out_pad_l2r = self.preprocess(padded_input_l2r)
         ys_in_pad_r2l, ys_out_pad_r2l = self.preprocess(padded_input_r2l)
         dev = encoder_outputs.device

@@ -31,13 +31,14 @@ _PATCHED = {
 }
 
 
-# opt-in (evaluation only): the SBL bidirectional decoder, greedy decode + teacher-forced forward on libsblk (decoder.py);
-# training keeps the reference decoder
+# opt-in: the SBL bidirectional decoder on libsblk (decoder.py): greedy decode and teacher-forced forward, and in
+# model.train() the training forward + backward, so train.py runs on it too
 _PATCHED_DECODER = {"transformer.decoder": {"Decoder": _dec.Decoder, "DecoderLayer": _dec.DecoderLayer}}
 
 
 def patch_reference(ref_dir, decoder=False):
-    """Rebind the hot-path names inside the reference package found at `ref_dir` (decoder=True: the SBL decoder too).
+    """Rebind the hot-path names inside the reference package found at `ref_dir` (decoder=True: the SBL decoder too,
+    for evaluation and for `train.py`'s training steps).
     Returns ({module name: module}, {(<module>, <attr>): original}) so the patch can be undone."""
     if ref_dir not in sys.path:
         sys.path.insert(0, ref_dir)

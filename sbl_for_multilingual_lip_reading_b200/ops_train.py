@@ -256,6 +256,64 @@ def ln_bwd(dy, z, gamma, lengths=None, T=1, eps=1e-5, want_f32=True, want_bf16=T
     return dz32, dz16, dgb[0], dgb[1]
 
 
+def _rows(t, name, rows, cols):
+    """t: a 2-D CUDA tensor view with unit column stride, >= rows rows and >= cols columns -> its row pitch."""
+    if t.dim() != 2 or t.stride(1) != 1 or t.shape[0] < rows or t.shape[1] < cols:
+        raise RuntimeError(f"{name}: expected a [>= {rows}, >= {cols}] row-major view, got {tuple(t.shape)} "
+                           f"strides {t.stride()}")
+    return t.stride(0)
+
+
+def xattention_train_fwd(q, k, v, n, lq, lk, h, causal=False, drop=None, klens=None, scale=0.125):
+    """Training attention with separate sources (include/sblk.h: sblk_xattention_train_fwd).  q [n*lq, >= h*64], k / v
+    [n*lk, >= h*64]: enc16 row-major views (column slices of one buffer allowed); drop fp32 [h*n, lq, lk] or None;
+    klens int32 [n] or None -> (out enc16 [n*lq, h*64], probs fp32 [h*n, lq, lk])."""
+    e16 = enc16_dtype()
+    for t_, nm in ((q, "q"), (k, "k"), (v, "v")):
+        if not t_.is_cuda or t_.dtype != e16:
+            raise RuntimeError(f"{nm}: expected a CUDA {e16} tensor (no CPU fallback exists)")
+    _req(drop, F32, "drop"); _req(klens, torch.int32, "klens")
+    ldq = _rows(q, "q", n * lq, h * 64)
+    ldk, ldv = _rows(k, "k", n * lk, h * 64), _rows(v, "v", n * lk, h * 64)
+    if drop is not None and tuple(drop.shape) != (h * n, lq, lk):
+        raise RuntimeError(f"xattention_train_fwd: drop shape {tuple(drop.shape)} != {(h * n, lq, lk)}")
+    probs = torch.empty((h * n, lq, lk), dtype=F32, device=q.device)
+    out = torch.empty((n * lq, h * 64), dtype=e16, device=q.device)
+    _call("sblk_xattention_train_fwd", f"xattention train fwd Lq={lq} Lk={lk}", 4 * n * h * lq * lk * 64,
+          2 * (n * lq + 2 * n * lk + n * lq) * h * 64 + 4 * probs.numel(), _p(q), _p(k), _p(v), _p(drop), _p(probs),
+          _p(out), _p(klens), ldq, ldk, ldv, h * 64, n, lq, lk, h, 1 if causal else 0, float(scale), _stream())
+    return out, probs
+
+
+def xattention_train_bwd(q, k, v, probs, dout, n, lq, lk, h, causal=False, drop=None, klens=None, scale=0.125,
+                         dq=None, dk=None, dv=None):
+    """Backward of xattention_train_fwd: dout bf16 [n*lq, h*64] -> (dq bf16, dk bf16, dv bf16).  The outputs are
+    allocated [n*lq | n*lk, h*64] unless row-major views to write into are given (e.g. the thirds of one dqkv buffer)."""
+    e16 = enc16_dtype()
+    for t_, nm in ((q, "q"), (k, "k"), (v, "v")):
+        if not t_.is_cuda or t_.dtype != e16:
+            raise RuntimeError(f"{nm}: expected a CUDA {e16} tensor (no CPU fallback exists)")
+    _req(probs, F32, "probs"); _req(dout, BF16, "dout"); _req(drop, F32, "drop"); _req(klens, torch.int32, "klens")
+    if tuple(probs.shape) != (h * n, lq, lk) or (drop is not None and tuple(drop.shape) != (h * n, lq, lk)):
+        raise RuntimeError(f"xattention_train_bwd: probs / drop must be [{h * n}, {lq}, {lk}]")
+    ldq = _rows(q, "q", n * lq, h * 64)
+    ldk, ldv = _rows(k, "k", n * lk, h * 64), _rows(v, "v", n * lk, h * 64)
+    lddo = _rows(dout, "dout", n * lq, h * 64)
+    grads = []
+    for g_, rows, nm in ((dq, n * lq, "dq"), (dk, n * lk, "dk"), (dv, n * lk, "dv")):
+        if g_ is None:
+            g_ = torch.empty((rows, h * 64), dtype=BF16, device=q.device)
+        elif not g_.is_cuda or g_.dtype != BF16:
+            raise RuntimeError(f"{nm}: expected a CUDA bfloat16 tensor")
+        grads.append((g_, _rows(g_, nm, rows, h * 64)))
+    (dq, lddq), (dk, lddk), (dv, lddv) = grads
+    _call("sblk_xattention_train_bwd", f"xattention train bwd Lq={lq} Lk={lk}", 8 * n * h * lq * lk * 64,
+          2 * (2 * n * lq + 2 * n * lk) * h * 64 + 4 * probs.numel(), _p(q), _p(k), _p(v), _p(drop), _p(probs),
+          _p(dout), _p(dq), _p(dk), _p(dv), _p(klens), ldq, ldk, ldv, lddo, lddq, lddk, lddv, n, lq, lk, h,
+          1 if causal else 0, float(scale), _stream())
+    return dq, dk, dv
+
+
 def attention_train_fwd(qkv, n, t, h, drop=None, lengths=None, scale=0.125):
     e16 = enc16_dtype()
     _req(qkv, e16, "qkv"); _req(drop, F32, "drop"); _req(lengths, torch.int32, "lengths")
@@ -274,3 +332,32 @@ def attention_train_bwd(qkv, probs, dout, n, t, h, drop=None, lengths=None, scal
     _call("sblk_attention_train_bwd", "attention train bwd", 8 * n * h * t * t * 64, 2 * qkv.numel(), _p(qkv), _p(drop),
           _p(probs), _p(dout), _p(dqkv), _p(lengths), n, t, h, float(scale), _stream())
     return dqkv
+
+
+def bidir_mix_bwd(g_l2r, g_r2l, n, L):
+    """Backward of the bidirectional mixing (include/sblk.h: sblk_bidir_mix_bwd): fp32 [n*L, D] x2 -> (d_l2r, d_r2l)."""
+    _req(g_l2r, F32, "g_l2r"); _req(g_r2l, F32, "g_r2l")
+    if g_l2r.shape != g_r2l.shape or g_l2r.dim() != 2 or g_l2r.shape[0] != n * L:
+        raise RuntimeError(f"bidir_mix_bwd: gradients must both be [{n * L}, D], got {tuple(g_l2r.shape)} / "
+                           f"{tuple(g_r2l.shape)}")
+    d = g_l2r.shape[1]
+    d_l2r, d_r2l = torch.empty_like(g_l2r), torch.empty_like(g_r2l)
+    _call("sblk_bidir_mix_bwd", "bidir_mix bwd", 3 * g_l2r.numel(), 16 * g_l2r.numel(), _p(g_l2r), _p(g_r2l), _p(d_l2r),
+          _p(d_r2l), n, L, d, _stream())
+    return d_l2r, d_r2l
+
+
+def embed_bwd(tokens, L, dx, vocab, scale=1.0):
+    """Embedding gradient (include/sblk.h: sblk_embed_bwd): tokens int64 [n, >= L] (any row pitch, unit column stride),
+    dx fp32 [n*L, D] -> fp32 [vocab, D]."""
+    if not tokens.is_cuda or tokens.dtype != torch.int64 or tokens.dim() != 2 or tokens.stride(1) != 1:
+        raise RuntimeError("embed_bwd: tokens must be a CUDA int64 [n, >= L] tensor with unit column stride")
+    _req(dx, F32, "dx")
+    n = tokens.shape[0]
+    if tokens.shape[1] < L or dx.dim() != 2 or dx.shape[0] != n * L:
+        raise RuntimeError(f"embed_bwd: tokens {tuple(tokens.shape)} / dx {tuple(dx.shape)} do not match L={L}")
+    d = dx.shape[1]
+    demb = torch.empty((int(vocab), d), dtype=F32, device=dx.device)
+    _call("sblk_embed_bwd", "embed bwd", dx.numel(), 4 * (dx.numel() + demb.numel()), _p(tokens), tokens.stride(0),
+          _p(dx), _p(demb), n * L, L, d, int(vocab), float(scale), _stream())
+    return demb

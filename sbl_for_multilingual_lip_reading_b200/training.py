@@ -14,6 +14,8 @@ of BASELINE configs[3]).
             zero-stuffed gradient); wgrad = split-K tcgen05 GEMM dY^T x im2col^T; BN / ReLU / pool derivative kernels
   encoder : per layer  QKV GEMM -> training attention (dropout on the probabilities) -> fc GEMM -> dropout -> +residual
             -> LayerNorm -> w_1 GEMM + ReLU -> w_2 GEMM -> dropout -> +residual -> LayerNorm, and the mirror-image backward
+  decoder : 16 steps x 2 directions x n_layers of the same blocks plus the decoder-encoder attention over K | V projected
+            once per call, embedding, bidirectional mixing and output projection Functions (decoder_forward_train)
 
 Precision: bf16 conv operands / activations / gradients, enc16 encoder activations, fp32 accumulation, statistics,
 LayerNorm / softmax math, residual-stream gradients and parameter gradients.  Dropout masks are drawn with
@@ -22,6 +24,8 @@ F.dropout calls, so a seeded reference run draws the same masks; the mask multip
 on the path (plus fp32 gradient additions where two branches meet).
 """
 from __future__ import annotations
+
+import random
 
 import torch
 import torch.nn.functional as F
@@ -261,9 +265,9 @@ def frontend_forward_train(fe, x):
 # ------------------------------------------------------------------------------------------------------------------
 # encoder Functions
 # ------------------------------------------------------------------------------------------------------------------
-def _lin_bwd(dy16, dy32, x16, w):
+def _lin_bwd(dy16, dy32, x16, w, bias=True):
     """Linear backward: dy16 bf16 [M,out] (GEMM operand), dy32 fp32 or None (bias gradient source), x16 saved enc16
-    input [M,in], w fp32 [out,in]  ->  (dW fp32 [out,in], db fp32 [out])."""
+    input [M,in], w fp32 [out,in]  ->  (dW fp32 [out,in], db fp32 [out] | None when bias=False)."""
     m, n_out = dy16.shape
     kb = -(-m // 64)
     splits = 1
@@ -276,6 +280,8 @@ def _lin_bwd(dy16, dy32, x16, w):
     x_t = ot.transpose16(x16, ld_out=ld, to_bf16=True)
     _, parts = ot.gemm_fmt(dy_t, x_t, out_f32=True, splits=splits)
     dw = parts.sum(0) if splits > 1 else parts
+    if not bias:
+        return dw, None
     db = ot.colreduce(2, dy32)[0].clone() if dy32 is not None else ot.colreduce(4, dy16)[0].clone()
     return dw, db
 
@@ -285,6 +291,89 @@ def _lin_dgrad(dy16, w, out_f32=True):
     wt = ops.cast_bf16(w.detach().t().contiguous())                   # [in, out] = the K-major B operand
     o16, o32 = ot.gemm_fmt(dy16, wt, out16=not out_f32, out_f32=out_f32)
     return o32 if out_f32 else o16
+
+
+def _e16(w):
+    return ops.cast_enc16(w.detach().contiguous())
+
+
+# Blocks shared by the encoder and decoder layers: every block ends in  out = LayerNorm(dropout(y) + x)  with the fp32
+# pre-normalisation sum z saved for the backward.
+def _drop_res_ln(y, d, x, g, be, lengths, t, eps, want16=True):
+    """-> (out fp32, out enc16 | None, z fp32) of LayerNorm(y * d + x) (d None: no dropout)."""
+    if d is not None:
+        y = y * d
+    z = y + x
+    out, out16 = ops.add_layernorm(z, g.detach(), be.detach(), lengths=lengths, T=t, eps=eps, want_bf16=want16)
+    return out, out16, z
+
+
+def _ln_drop_bwd(dout, z, g, d, lengths, t, eps):
+    """Backward of _drop_res_ln -> (dz fp32 = the residual's gradient, dy fp32, dy bf16, dgamma, dbeta)."""
+    dz32, dz16, dg, dbe = ot.ln_bwd(dout, z, g.detach(), lengths=lengths, T=t, eps=eps)
+    if d is None:
+        return dz32, dz32, dz16, dg, dbe
+    dy32 = dz32 * d
+    return dz32, dy32, ops.cast_bf16(dy32), dg, dbe
+
+
+def _ffn_fwd(x, x16, w1, b1, w2, b2, g, be, d, lengths, t, eps, want16):
+    """PositionwiseFeedForward (module.py:47-52) -> (out fp32, out enc16 | None, saved (h16, z))."""
+    h16, _ = ops.gemm(x16, _e16(w1), bias=b1.detach(), relu=True, out_bf16=True)
+    _, y = ops.gemm(h16, _e16(w2), bias=b2.detach(), out_f32=True)
+    out, out16, z = _drop_res_ln(y, d, x, g, be, lengths, t, eps, want16)
+    return out, out16, (h16, z)
+
+
+def _ffn_bwd(dout, x16, saved, w1, w2, g, d, lengths, t, eps):
+    """-> (dx fp32, dw1, db1, dw2, db2, dgamma, dbeta)."""
+    h16, z = saved
+    dz32, dy32, dy16, dg, dbe = _ln_drop_bwd(dout, z, g, d, lengths, t, eps)
+    dw2, db2 = _lin_bwd(dy16, dy32, h16, w2)
+    dh = _lin_dgrad(dy16, w2, out_f32=False)
+    ot.relu_bwd_(dh, h16)
+    dw1, db1 = _lin_bwd(dh, None, x16, w1)
+    return dz32 + _lin_dgrad(dh, w1), dw1, db1, dw2, db2, dg, dbe
+
+
+def _self_attn_fwd(x, x16, wq, bq, wk, bk, wv, bv, wfc, bfc, g, be, d_attn, d_fc, lengths, n, t, h, scale, eps,
+                   causal=None):
+    """MultiHeadAttention as self-attention (attention.py:32-60) on [n*t, 512] rows -> (out fp32, out enc16,
+    saved (qkv16, probs, att16, z)).  causal None: the encoder's packed kernel pair (sblk_attention_train_*);
+    True / False: the separate-source pair (sblk_xattention_train_*) with / without the subsequent mask."""
+    hd = wq.shape[0]
+    wqkv = ops.cast_enc16(torch.cat([wq.detach(), wk.detach(), wv.detach()], 0).contiguous())
+    bqkv = torch.cat([bq.detach(), bk.detach(), bv.detach()]).contiguous()
+    qkv16, _ = ops.gemm(x16, wqkv, bias=bqkv, out_bf16=True)
+    if causal is None:
+        att16, probs = ot.attention_train_fwd(qkv16, n, t, h, drop=d_attn, lengths=lengths, scale=scale)
+    else:
+        att16, probs = ot.xattention_train_fwd(qkv16[:, :hd], qkv16[:, hd:2 * hd], qkv16[:, 2 * hd:], n, t, t, h,
+                                               causal=causal, drop=d_attn, klens=lengths, scale=scale)
+    _, y = ops.gemm(att16, _e16(wfc), bias=bfc.detach(), out_f32=True)
+    out, out16, z = _drop_res_ln(y, d_fc, x, g, be, lengths, t, eps)
+    return out, out16, (qkv16, probs, att16, z)
+
+
+def _self_attn_bwd(dout, x16, saved, wq, wk, wv, wfc, g, d_attn, d_fc, lengths, n, t, h, scale, eps, causal=None):
+    """-> (dx fp32, dwq, dbq, dwk, dbk, dwv, dbv, dwfc, dbfc, dgamma, dbeta)."""
+    qkv16, probs, att16, z = saved
+    hd = wq.shape[0]
+    dz32, dy32, dy16, dg, dbe = _ln_drop_bwd(dout, z, g, d_fc, lengths, t, eps)
+    dwfc, dbfc = _lin_bwd(dy16, dy32, att16, wfc)
+    datt = _lin_dgrad(dy16, wfc, out_f32=False)
+    if causal is None:
+        dqkv = ot.attention_train_bwd(qkv16, probs, datt, n, t, h, drop=d_attn, lengths=lengths, scale=scale)
+    else:
+        dqkv = torch.empty((n * t, 3 * hd), dtype=BF16, device=x16.device)
+        ot.xattention_train_bwd(qkv16[:, :hd], qkv16[:, hd:2 * hd], qkv16[:, 2 * hd:], probs, datt, n, t, t, h,
+                                causal=causal, drop=d_attn, klens=lengths, scale=scale, dq=dqkv[:, :hd],
+                                dk=dqkv[:, hd:2 * hd], dv=dqkv[:, 2 * hd:])
+    wqkv = torch.cat([wq.detach(), wk.detach(), wv.detach()], 0)
+    dwqkv, dbqkv = _lin_bwd(dqkv, None, x16, wqkv)
+    dx = dz32 + _lin_dgrad(dqkv, wqkv)
+    return (dx, dwqkv[:hd].contiguous(), dbqkv[:hd].contiguous(), dwqkv[hd:2 * hd].contiguous(),
+            dbqkv[hd:2 * hd].contiguous(), dwqkv[2 * hd:].contiguous(), dbqkv[2 * hd:].contiguous(), dwfc, dbfc, dg, dbe)
 
 
 class EncoderInFn(torch.autograd.Function):
@@ -317,25 +406,12 @@ class EncoderLayerFn(torch.autograd.Function):
     def forward(ctx, x, wq, bq, wk, bk, wv, bv, wfc, bfc, g1, be1, w1, b1, w2, b2, g2, be2, drops, lengths, n, t, h, scale,
                 eps):
         x = x.detach().contiguous()
-        m = n * t
         d_attn, d_fc, d_ffn = drops
         x16 = ops.cast_enc16(x)
-        wqkv = ops.cast_enc16(torch.cat([wq.detach(), wk.detach(), wv.detach()], 0).contiguous())
-        bqkv = torch.cat([bq.detach(), bk.detach(), bv.detach()]).contiguous()
-        qkv16, _ = ops.gemm(x16, wqkv, bias=bqkv, out_bf16=True)
-        att16, probs = ot.attention_train_fwd(qkv16, n, t, h, drop=d_attn, lengths=lengths, scale=scale)
-        _, y1 = ops.gemm(att16, ops.cast_enc16(wfc.detach().contiguous()), bias=bfc.detach(), out_f32=True)
-        if d_fc is not None:
-            y1 = y1 * d_fc
-        z1 = y1 + x
-        x1, x1_16 = ops.add_layernorm(z1, g1.detach(), be1.detach(), lengths=lengths, T=t, eps=eps)
-        h16, _ = ops.gemm(x1_16, ops.cast_enc16(w1.detach().contiguous()), bias=b1.detach(), relu=True, out_bf16=True)
-        _, y2 = ops.gemm(h16, ops.cast_enc16(w2.detach().contiguous()), bias=b2.detach(), out_f32=True)
-        if d_ffn is not None:
-            y2 = y2 * d_ffn
-        z2 = y2 + x1
-        out, _ = ops.add_layernorm(z2, g2.detach(), be2.detach(), lengths=lengths, T=t, eps=eps, want_bf16=False)
-        ctx.save_for_backward(x16, qkv16, probs, att16, z1, x1_16, h16, z2, wq, wk, wv, wfc, w1, w2, g1, g2)
+        x1, x1_16, sa = _self_attn_fwd(x, x16, wq, bq, wk, bk, wv, bv, wfc, bfc, g1, be1, d_attn, d_fc, lengths, n, t, h,
+                                       scale, eps)
+        out, _, ff = _ffn_fwd(x1, x1_16, w1, b1, w2, b2, g2, be2, d_ffn, lengths, t, eps, want16=False)
+        ctx.save_for_backward(x16, *sa, x1_16, *ff, wq, wk, wv, wfc, w1, w2, g1, g2)
         ctx.misc = (drops, lengths, n, t, h, scale, eps)
         return out
 
@@ -343,35 +419,12 @@ class EncoderLayerFn(torch.autograd.Function):
     def backward(ctx, dout):
         x16, qkv16, probs, att16, z1, x1_16, h16, z2, wq, wk, wv, wfc, w1, w2, g1, g2 = ctx.saved_tensors
         (d_attn, d_fc, d_ffn), lengths, n, t, h, scale, eps = ctx.misc
-        # x2 = LN(z2) * keep ; z2 = dropout(w_2 relu(w_1 x1)) + x1
-        dz2_32, dz2_16, dg2, dbe2 = ot.ln_bwd(dout.contiguous().float(), z2, g2.detach(), lengths=lengths, T=t, eps=eps)
-        if d_ffn is not None:
-            dy2_32 = dz2_32 * d_ffn
-            dy2_16 = ops.cast_bf16(dy2_32)
-        else:
-            dy2_32, dy2_16 = dz2_32, dz2_16
-        dw2, db2 = _lin_bwd(dy2_16, dy2_32, h16, w2)
-        dh = _lin_dgrad(dy2_16, w2, out_f32=False)
-        ot.relu_bwd_(dh, h16)
-        dw1, db1 = _lin_bwd(dh, None, x1_16, w1)
-        dx1 = dz2_32 + _lin_dgrad(dh, w1)
-        # x1 = LN(z1) * keep ; z1 = dropout(fc(attention)) + x
-        dz1_32, dz1_16, dg1, dbe1 = ot.ln_bwd(dx1, z1, g1.detach(), lengths=lengths, T=t, eps=eps)
-        if d_fc is not None:
-            dy1_32 = dz1_32 * d_fc
-            dy1_16 = ops.cast_bf16(dy1_32)
-        else:
-            dy1_32, dy1_16 = dz1_32, dz1_16
-        dwfc, dbfc = _lin_bwd(dy1_16, dy1_32, att16, wfc)
-        datt = _lin_dgrad(dy1_16, wfc, out_f32=False)
-        dqkv = ot.attention_train_bwd(qkv16, probs, datt, n, t, h, drop=d_attn, lengths=lengths, scale=scale)
-        wqkv = torch.cat([wq.detach(), wk.detach(), wv.detach()], 0)
-        dwqkv, dbqkv = _lin_bwd(dqkv, None, x16, wqkv)
-        dx = dz1_32 + _lin_dgrad(dqkv, wqkv)
-        hk = wq.shape[0]
-        return (dx, dwqkv[:hk].contiguous(), dbqkv[:hk].contiguous(), dwqkv[hk:2 * hk].contiguous(),
-                dbqkv[hk:2 * hk].contiguous(), dwqkv[2 * hk:].contiguous(), dbqkv[2 * hk:].contiguous(), dwfc, dbfc, dg1,
-                dbe1, dw1, db1, dw2, db2, dg2, dbe2, None, None, None, None, None, None, None)
+        dx1, dw1, db1, dw2, db2, dg2, dbe2 = _ffn_bwd(dout.contiguous().float(), x1_16, (h16, z2), w1, w2, g2, d_ffn,
+                                                      lengths, t, eps)
+        dx, dwq, dbq, dwk, dbk, dwv, dbv, dwfc, dbfc, dg1, dbe1 = _self_attn_bwd(
+            dx1, x16, (qkv16, probs, att16, z1), wq, wk, wv, wfc, g1, d_attn, d_fc, lengths, n, t, h, scale, eps)
+        return (dx, dwq, dbq, dwk, dbk, dwv, dbv, dwfc, dbfc, dg1, dbe1, dw1, db1, dw2, db2, dg2, dbe2, None, None, None,
+                None, None, None, None)
 
 
 def _drop_factor(shape, p, dev, training):
@@ -408,3 +461,211 @@ def encoder_forward_train(enc, padded_input, lens):
                                  f.w_2.weight, f.w_2.bias, f.layer_norm.weight, f.layer_norm.bias, drops, lengths, n, t, h,
                                  1.0 / a.temperature, a.layer_norm.eps)
     return (y.view(n, t, enc.d_model),)
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# decoder Functions (the SBL bidirectional decoder, decoder.py; DESIGN.md §9 "training")
+# ------------------------------------------------------------------------------------------------------------------
+class EncoderKVFn(torch.autograd.Function):
+    """K | V projections of the encoder outputs for one decoder layer's enc_attn, computed once per call and read by all
+    16 steps.  Returns (kv fp32 [n*t, 2*hd], kv enc16): the fp32 tensor carries the gradient (autograd sums the 16
+    steps' contributions in fp32), the enc16 copy is the attention kernel's operand."""
+
+    @staticmethod
+    def forward(ctx, enc, enc16, wk, bk, wv, bv):
+        wkv = torch.cat([wk.detach(), wv.detach()], 0)
+        kv16, kv32 = ops.gemm(enc16, ops.cast_enc16(wkv.contiguous()), bias=torch.cat([bk.detach(), bv.detach()]),
+                              out_bf16=True, out_f32=True)
+        ctx.mark_non_differentiable(kv16)
+        ctx.save_for_backward(enc16, wk, wv)
+        return kv32, kv16
+
+    @staticmethod
+    def backward(ctx, dkv, _):
+        enc16, wk, wv = ctx.saved_tensors
+        hd = wk.shape[0]
+        wkv = torch.cat([wk.detach(), wv.detach()], 0)
+        dkv = dkv.contiguous()
+        dkv16 = ops.cast_bf16(dkv)
+        dw, db = _lin_bwd(dkv16, dkv, enc16, wkv)
+        denc = _lin_dgrad(dkv16, wkv) if ctx.needs_input_grad[0] else None
+        return denc, None, dw[:hd].contiguous(), db[:hd].contiguous(), dw[hd:].contiguous(), db[hd:].contiguous()
+
+
+class DecoderEmbedFn(torch.autograd.Function):
+    """tgt_word_emb(ys[:, :L]) * scale + positional encoding (decoder.py:323-327) -> (x fp32 [n*L, 512], x enc16)."""
+
+    @staticmethod
+    def forward(ctx, emb, ys, L, pe, scale):
+        n = ys.shape[0]
+        e = emb.detach().float().contiguous()
+        x32 = torch.empty((n * L, e.shape[1]), dtype=F32, device=e.device)
+        x16 = torch.empty((n * L, e.shape[1]), dtype=ops.enc16_dtype(), device=e.device)
+        ops._call("sblk_embed_pe_fwd", "embed_pe", 0, 6 * x32.numel(), ys.data_ptr(), ys.stride(0), e.data_ptr(),
+                  pe.data_ptr(), x32.data_ptr(), x16.data_ptr(), n * L, L, e.shape[1], e.shape[0], float(scale),
+                  ops._stream())
+        ctx.mark_non_differentiable(x16)
+        # the token buffer itself, not a copy: the decode loop only writes columns >= L after this step
+        ctx.ys, ctx.L, ctx.vocab, ctx.scale = ys, L, e.shape[0], scale
+        return x32, x16
+
+    @staticmethod
+    def backward(ctx, dx, _):
+        return ot.embed_bwd(ctx.ys, ctx.L, dx.contiguous(), ctx.vocab, ctx.scale), None, None, None, None
+
+
+class BidirMixFn(torch.autograd.Function):
+    """The synchronous bidirectional mixing (decoder.py:336-346,358-362) -> (l2r' fp32, r2l' fp32, l2r' enc16,
+    r2l' enc16)."""
+
+    @staticmethod
+    def forward(ctx, l2r, r2l, n, L):
+        a32, b32 = torch.empty_like(l2r), torch.empty_like(r2l)
+        a16 = torch.empty(l2r.shape, dtype=ops.enc16_dtype(), device=l2r.device)
+        b16 = torch.empty_like(a16)
+        ops._call("sblk_bidir_mix_fwd", "bidir_mix", 3 * l2r.numel(), 20 * l2r.numel(), l2r.data_ptr(), r2l.data_ptr(),
+                  a32.data_ptr(), b32.data_ptr(), a16.data_ptr(), b16.data_ptr(), n, L, l2r.shape[1], ops._stream())
+        ctx.mark_non_differentiable(a16, b16)
+        ctx.n, ctx.L = n, L
+        return a32, b32, a16, b16
+
+    @staticmethod
+    def backward(ctx, ga, gb, _a, _b):
+        d_l2r, d_r2l = ot.bidir_mix_bwd(ga.contiguous(), gb.contiguous(), ctx.n, ctx.L)
+        return d_l2r, d_r2l, None, None
+
+
+class DecoderLayerFn(torch.autograd.Function):
+    """DecoderLayer.forward in training mode (decoder.py:396-408): self-attention over the prefix (subsequent mask when
+    `causal`), attention over the encoder's K | V (kv fp32 / kv16 from EncoderKVFn, no mask), FFN.  x fp32 [n*L, 512],
+    x16 its enc16 copy or None.  drops = (self-attention probabilities, self fc output, enc-attention probabilities,
+    enc fc output, ffn output) factors mask / (1 - p), or None each.  -> (out fp32, out enc16)."""
+
+    @staticmethod
+    def forward(ctx, x, x16, kv, kv16, wq, bq, wk, bk, wv, bv, wfc, bfc, g1, be1, wq2, bq2, wfc2, bfc2, g2, be2, w1, b1,
+                w2, b2, g3, be3, drops, n, L, t_enc, h, causal, scale1, scale2, eps):
+        x = x.detach().contiguous()
+        x16 = ops.cast_enc16(x) if x16 is None else x16
+        hd = wq2.shape[0]
+        d_a1, d_f1, d_a2, d_f2, d_ffn = drops
+        x1, x1_16, sa = _self_attn_fwd(x, x16, wq, bq, wk, bk, wv, bv, wfc, bfc, g1, be1, d_a1, d_f1, None, n, L, h,
+                                       scale1, eps[0], causal=bool(causal))
+        q16, _ = ops.gemm(x1_16, _e16(wq2), bias=bq2.detach(), out_bf16=True)
+        att2, probs2 = ot.xattention_train_fwd(q16, kv16[:, :hd], kv16[:, hd:], n, L, t_enc, h, drop=d_a2,
+                                               scale=scale2)
+        _, y2 = ops.gemm(att2, _e16(wfc2), bias=bfc2.detach(), out_f32=True)
+        x2, x2_16, z2 = _drop_res_ln(y2, d_f2, x1, g2, be2, None, L, eps[1])
+        out, out16, ff = _ffn_fwd(x2, x2_16, w1, b1, w2, b2, g3, be3, d_ffn, None, L, eps[2], want16=True)
+        ctx.mark_non_differentiable(out16)
+        ctx.save_for_backward(x16, *sa, x1_16, q16, kv16, probs2, att2, z2, x2_16, *ff, wq, wk, wv, wfc, wq2, wfc2, w1,
+                              w2, g1, g2, g3)
+        ctx.misc = (drops, n, L, t_enc, h, causal, scale1, scale2, eps)
+        return out, out16
+
+    @staticmethod
+    def backward(ctx, dout, _):
+        (x16, qkv16, probs1, att1, z1, x1_16, q16, kv16, probs2, att2, z2, x2_16, h16, z3, wq, wk, wv, wfc, wq2, wfc2, w1,
+         w2, g1, g2, g3) = ctx.saved_tensors
+        (d_a1, d_f1, d_a2, d_f2, d_ffn), n, L, t_enc, h, causal, scale1, scale2, eps = ctx.misc
+        hd = wq2.shape[0]
+        dx2, dw1, db1, dw2, db2, dg3, dbe3 = _ffn_bwd(dout.contiguous().float(), x2_16, (h16, z3), w1, w2, g3, d_ffn,
+                                                      None, L, eps[2])
+        # x2 = LN(dropout(fc2(attention(q(x1), K, V))) + x1)
+        dz2, dy32, dy16, dg2, dbe2 = _ln_drop_bwd(dx2, z2, g2, d_f2, None, L, eps[1])
+        dwfc2, dbfc2 = _lin_bwd(dy16, dy32, att2, wfc2)
+        datt2 = _lin_dgrad(dy16, wfc2, out_f32=False)
+        dkv = torch.empty((n * t_enc, 2 * hd), dtype=BF16, device=x16.device)
+        dq2, _, _ = ot.xattention_train_bwd(q16, kv16[:, :hd], kv16[:, hd:], probs2, datt2, n, L, t_enc, h, drop=d_a2,
+                                            scale=scale2, dk=dkv[:, :hd], dv=dkv[:, hd:])
+        dwq2, dbq2 = _lin_bwd(dq2, None, x1_16, wq2)
+        dx1 = dz2 + _lin_dgrad(dq2, wq2)
+        dx, dwq, dbq, dwk, dbk, dwv, dbv, dwfc, dbfc, dg1, dbe1 = _self_attn_bwd(
+            dx1, x16, (qkv16, probs1, att1, z1), wq, wk, wv, wfc, g1, d_a1, d_f1, None, n, L, h, scale1, eps[0],
+            causal=bool(causal))
+        return (dx, None, dkv.float(), None, dwq, dbq, dwk, dbk, dwv, dbv, dwfc, dbfc, dg1, dbe1, dwq2, dbq2, dwfc2, dbfc2,
+                dg2, dbe2, dw1, db1, dw2, db2, dg3, dbe3) + (None,) * 9
+
+
+class DecoderProjFn(torch.autograd.Function):
+    """tgt_word_prj(dec_output[:, -1]) (decoder.py:364-365): the last position's enc16 row of every clip times the
+    [vocab, 512] weight, zero-padded to 64 rows like Decoder._get_packed -> logits fp32 [n, vocab]."""
+
+    @staticmethod
+    def forward(ctx, x, x16, w, n, L):
+        vocab, d = w.shape
+        last16 = x16.view(n, L, d)[:, -1].contiguous()
+        wp = torch.zeros((64, d), dtype=F32, device=w.device)
+        wp[:vocab] = w.detach()
+        _, logits = ops.gemm(last16, ops.cast_enc16(wp), out_f32=True)
+        ctx.save_for_backward(last16, wp)
+        ctx.n, ctx.L, ctx.vocab = n, L, vocab
+        return logits[:, :vocab].contiguous()
+
+    @staticmethod
+    def backward(ctx, dlogits):
+        last16, wp = ctx.saved_tensors
+        n, L, vocab = ctx.n, ctx.L, ctx.vocab
+        dl = torch.zeros((n, 64), dtype=F32, device=wp.device)
+        dl[:, :vocab] = dlogits
+        dl16 = ops.cast_bf16(dl)
+        dw, _ = _lin_bwd(dl16, None, last16, wp, bias=False)
+        dx = torch.zeros((n, L, wp.shape[1]), dtype=F32, device=wp.device)
+        dx[:, -1] = _lin_dgrad(dl16, wp)
+        return dx.view(n * L, -1), None, dw[:vocab].contiguous(), None, None
+
+
+def decoder_forward_train(dec, padded_input_l2r, padded_input_r2l, encoder_outputs):
+    """Decoder.forward in training mode (reference decoder.py:79-191) -> (logits_l2r [N,16,vocab], gold_l2r,
+    logits_r2l, gold_r2l), the logits autograd-connected to every decoder parameter and to `encoder_outputs`.
+
+    16 steps; step i recomputes the whole prefix of length L = i + 1 in both directions (subsequent mask in the first
+    layer only, the mixing after every layer) and feeds, per the reference's coin `random.random() > 0.5`, the step's
+    own argmax (a constant for autograd) or the gold token.  Dropout factors are drawn with _drop_factor in this order
+    (DESIGN.md §9): per step, the embedding's of l2r then r2l; then per layer, l2r then r2l, each as (self-attention
+    probabilities [H*N, L, L], self fc output [N*L, 512], enc-attention probabilities [H*N, L, t_enc], enc fc output,
+    ffn output); the embedding's are [N*L, 512]."""
+    ys_out = {}
+    _, ys_out["l2r"] = dec.preprocess(padded_input_l2r)
+    _, ys_out["r2l"] = dec.preprocess(padded_input_r2l)
+    n, t_enc, dm = encoder_outputs.shape
+    dev = encoder_outputs.device
+    h = dec.n_head
+    p = float(dec.dropout.p)
+    enc = encoder_outputs.float().contiguous().view(n * t_enc, dm)
+    enc16 = ops.cast_enc16(enc.detach())
+    layers = {"l2r": [dec.layer_first_l2r] + list(dec.layer_stack_l2r),
+              "r2l": [dec.layer_first_r2l] + list(dec.layer_stack_r2l)}
+    kv = {d: [EncoderKVFn.apply(enc, enc16, l_.enc_attn.w_ks.weight, l_.enc_attn.w_ks.bias, l_.enc_attn.w_vs.weight,
+                                l_.enc_attn.w_vs.bias) for l_ in layers[d]] for d in ("l2r", "r2l")}
+    prj = {"l2r": dec.tgt_word_prj_l2r.weight, "r2l": dec.tgt_word_prj_r2l.weight}
+    pe = dec.positional_encoding.pe[0]
+    ys = {d: torch.full((n, dec.maxlen + 1), dec.sos_id, dtype=torch.long, device=dev) for d in ("l2r", "r2l")}
+    logits = {"l2r": [], "r2l": []}
+    for i in range(dec.maxlen):
+        L = i + 1
+        x = {}
+        for d in ("l2r", "r2l"):
+            x32, x16 = DecoderEmbedFn.apply(dec.tgt_word_emb.weight, ys[d], L, pe, float(dec.x_logit_scale))
+            f = _drop_factor((n * L, dm), p, dev, True)
+            x[d] = (x32, x16) if f is None else (x32 * f, None)
+        for li in range(dec.n_layers):
+            for d in ("l2r", "r2l"):
+                lyr = layers[d][li]
+                a, c, ff = lyr.slf_attn, lyr.enc_attn, lyr.pos_ffn
+                drops = tuple(_drop_factor(s_, p, dev, True) for s_ in ((h * n, L, L), (n * L, dm), (h * n, L, t_enc),
+                                                                         (n * L, dm), (n * L, dm)))
+                x[d] = DecoderLayerFn.apply(
+                    x[d][0], x[d][1], kv[d][li][0], kv[d][li][1], a.w_qs.weight, a.w_qs.bias, a.w_ks.weight,
+                    a.w_ks.bias, a.w_vs.weight, a.w_vs.bias, a.fc.weight, a.fc.bias, a.layer_norm.weight,
+                    a.layer_norm.bias, c.w_qs.weight, c.w_qs.bias, c.fc.weight, c.fc.bias, c.layer_norm.weight,
+                    c.layer_norm.bias, ff.w_1.weight, ff.w_1.bias, ff.w_2.weight, ff.w_2.bias, ff.layer_norm.weight,
+                    ff.layer_norm.bias, drops, n, L, t_enc, h, li == 0, 1.0 / a.temperature, 1.0 / c.temperature,
+                    (a.layer_norm.eps, c.layer_norm.eps, ff.layer_norm.eps))
+            a32, b32, a16, b16 = BidirMixFn.apply(x["l2r"][0], x["r2l"][0], n, L)
+            x = {"l2r": (a32, a16), "r2l": (b32, b16)}
+        step = {d: DecoderProjFn.apply(x[d][0], x[d][1], prj[d], n, L) for d in ("l2r", "r2l")}
+        is_teacher = random.random() > 0.5          # decoder.py:176 (the flag's name is the reference's)
+        for d in ("l2r", "r2l"):
+            logits[d].append(step[d])
+            ys[d][:, i + 1] = step[d].detach().argmax(-1) if is_teacher else ys_out[d][:, i].to(dev)
+    return torch.stack(logits["l2r"], 1), ys_out["l2r"], torch.stack(logits["r2l"], 1), ys_out["r2l"]
